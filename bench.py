@@ -74,6 +74,23 @@ def xstar(n):
     return ((i * np.uint64(2654435761) + np.uint64(40503)) % np.uint64(2 ** 32)).astype(np.float64) / 2.0 ** 31 - 1.0
 
 
+DUMP_MAX_ENTRIES = 1 << 21   # solution entries --dump-outputs writes: 16 MB of values + 16 MB of indices
+
+
+def dump_outputs(out_dir, x, it, hist):
+    """--dump-outputs: what a caller of the timed solve receives from its last step, as float64 .npy files -- the solution
+    (x.npy at the global indices x_index.npy: all of it, or a fixed seeded sample of DUMP_MAX_ENTRIES entries when larger),
+    the residual history (||r_k||, k = 0 .. iters) and the iteration count -- so that two builds can be compared output
+    for output on identical inputs."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(x)
+    idx = np.arange(n) if n <= DUMP_MAX_ENTRIES else np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_ENTRIES, replace=False))
+    np.save(os.path.join(out_dir, "x.npy"), np.asarray(x, np.float64)[idx])
+    np.save(os.path.join(out_dir, "x_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "residual_history.npy"), np.asarray(hist, np.float64))
+    np.save(os.path.join(out_dir, "iters.npy"), np.array([it], np.float64))
+
+
 def config_of(workload, wl, nparts, iters, levels):
     """Identical key set (and, by the asserted parity, identical values) in both arms."""
     return dict(workload=workload, description=wl["desc"], parts=list(PARTS[nparts]), iters=int(iters), levels=int(levels),
@@ -154,13 +171,13 @@ def cpu_solve_timed(c, nparts, b_parts, reps, threads=None):
     from parallel_amg_b200 import _lib as L
     L.set_num_threads(threads or os.cpu_count() or 1)   # launchers export OMP_NUM_THREADS=1; the oracle shares the process's OpenMP runtime
     co = c_oracle.COracle.from_product_context(c, nparts)
-    times, it, hist = [], 0, None
+    times, it, hist, x = [], 0, None, None
     for _ in range(reps):
         t0 = time.perf_counter()
         x, it, hist = co.pcg(b_parts, RTOL, MAXITER, True)
         times.append(time.perf_counter() - t0)
     co.close()
-    return times, it, hist
+    return times, it, hist, x
 
 
 def other_krylov_drivers(c, nparts, b_parts, own_all, b):
@@ -371,6 +388,8 @@ def measure(workload, args, rank, world, local_rank, steps, warmup, headline):
     true_rel = float(np.linalg.norm(b - c.host_matvec_global(xg)) / np.linalg.norm(b)) if have_A else 0.0
     assert true_rel <= 2e-8, f"true residual {true_rel}"
     sol_err = float(np.abs(xg - xs_true).max())
+    if args.dump_outputs and headline and rank == 0:
+        dump_outputs(args.dump_outputs, xg, it, hist)
 
     if args.trace and headline:
         write_trace(c, mine[0], args.trace + f".rank{rank}.txt")
@@ -436,7 +455,7 @@ def measure(workload, args, rank, world, local_rank, steps, warmup, headline):
                 own_all = [c.index_maps(0, p)[0] for p in range(nparts)]
                 reps = args.cpu_reps if headline else 1
                 cores = max(1, (os.cpu_count() or 1) - (world - 1))   # the sleeping ranks still own a helper thread each
-                times, it_cpu, hist_cpu = cpu_solve_timed(c, nparts, [b[o] for o in own_all], reps, threads=cores)
+                times, it_cpu, hist_cpu, _ = cpu_solve_timed(c, nparts, [b[o] for o in own_all], reps, threads=cores)
                 cpu = dict(value=n / min(times), unit="DOF/s", cores=cores, kind="port",
                            sample=f"{reps} whole solve(s) ({it_cpu} iterations each) of the same workload on the same {nparts}-part hierarchy, best one; "
                                   f"C/OpenMP oracle port on {cores} host threads (no reference code exists)",
@@ -491,8 +510,14 @@ def run_reference(args, wl, rank, world):
     c.setup(c.default_options(**wl.get("opts", {})))
     n, nnz = c.global_size()
     b = c.host_matvec_global(xstar(n))
-    b_parts = [b[c.index_maps(0, p)[0]] for p in range(nparts)]
-    times, it, hist = cpu_solve_timed(c, nparts, b_parts, args.warmup + args.steps)
+    own = [c.index_maps(0, p)[0] for p in range(nparts)]
+    b_parts = [b[o] for o in own]
+    times, it, hist, x = cpu_solve_timed(c, nparts, b_parts, args.warmup + args.steps)
+    if args.dump_outputs:
+        xg = np.zeros(n)
+        for o, xp in zip(own, x):
+            xg[o] = xp
+        dump_outputs(args.dump_outputs, xg, it, hist)
     timed = times[args.warmup:]
     total = float(sum(timed))
     cores = os.cpu_count()
@@ -524,9 +549,14 @@ def main():
     ap.add_argument("--smoother", default="jacobi")
     ap.add_argument("--replicate-setup", action="store_true", help="N > 1: every rank runs the host setup itself (default: rank 0 builds, the others load it from shared memory)")
     ap.add_argument("--trace", default=None, help="write a per-kernel timeline of one solve (device globaltimer) to this file prefix")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the solution (sampled above 2M entries), residual history and iteration count of the last timed solve "
+                         "as float64 .npy files into DIR")
     args = ap.parse_args()
     if args.gpus not in PARTS:
         raise SystemExit("--gpus must be 1, 2, 4 or 8")
+    if args.steps < 1:
+        raise SystemExit("--steps must be at least 1")
     wl = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

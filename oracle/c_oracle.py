@@ -5,6 +5,7 @@ Built with plain gcc into oracle/_build/ (git-ignored, travels to the GPU box)."
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
 import os
 import subprocess
 
@@ -14,16 +15,26 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = os.path.join(HERE, "pamg_oracle.c")
 OUT_DIR = os.path.join(HERE, "_build")
 LIB = os.path.join(OUT_DIR, "libpamg_oracle.so")
+STAMP = os.path.join(OUT_DIR, "libpamg_oracle.stamp")
 FLAGS = ["-O3", "-march=x86-64-v3", "-fopenmp", "-fPIC", "-shared", "-ffp-contract=off", "-std=c11"]
 
 
+def _digest():
+    with open(SRC, "rb") as fh:
+        return hashlib.sha256(fh.read() + " ".join(FLAGS).encode()).hexdigest()
+
+
 def build(force=False):
-    os.makedirs(OUT_DIR, exist_ok=True)
-    if not force and os.path.exists(LIB) and os.path.getmtime(LIB) >= os.path.getmtime(SRC):
+    # Rebuild on a change of the source or flags, not of mtimes: a copied tree keeps a valid library and may be read-only.
+    dig = _digest()
+    if not force and os.path.exists(LIB) and os.path.exists(STAMP) and open(STAMP).read().strip() == dig:
         return LIB
+    os.makedirs(OUT_DIR, exist_ok=True)
     r = subprocess.run(["gcc"] + FLAGS + [SRC, "-o", LIB, "-lm"], capture_output=True, text=True)
     if r.returncode:
         raise RuntimeError("gcc failed:\n" + r.stderr)
+    with open(STAMP, "w") as fh:
+        fh.write(dig)
     return LIB
 
 
