@@ -49,8 +49,13 @@ enum { PAMG_CYCLE_V = 0, PAMG_CYCLE_W = 1 };
  * A SELL block (2 rows per thread) with at most 255 distinct values -- stencil matrices, their prolongators -- is stored
  * VALUE-INDEXED: int32 column + one byte into a dictionary of the original doubles (two bytes up to 4095 values), four
  * interleaved rows per lane in slices of 128 rows: 5 (6) instead of 12 bytes per entry, bit-identical products and sums
- * (pamg_stats.value_indexed, pamg_layout_sell_values; env PAMG_VALUE_INDEX=0 keeps fp64 values). */
-enum { PAMG_FORMAT_AUTO = 0, PAMG_FORMAT_CSR = 1, PAMG_FORMAT_STREAM = 2, PAMG_FORMAT_SELL = 3 };
+ * (pamg_stats.value_indexed, pamg_layout_sell_values; env PAMG_VALUE_INDEX=0 keeps fp64 values).
+ * Under AUTO an A block of at least 200000 rows whose rows hold their entries at row + off[j] for at most 32 fixed offsets
+ * (stencil matrices; strictly ascending columns, ndiag x rows <= 1.25 nnz, <= 254 distinct non-zero values) is stored with
+ * IMPLIED COLUMNS: one index byte per (row, offset) slot and no column (pamg_stats.value_indexed bit 64, pamg_layout_sell_diag;
+ * pamg_stats.format still reads SELL).  SELL_DIAG takes that layout for every qualifying A block at any size and handles all
+ * other blocks as SELL; an explicit SELL never takes it. */
+enum { PAMG_FORMAT_AUTO = 0, PAMG_FORMAT_CSR = 1, PAMG_FORMAT_STREAM = 2, PAMG_FORMAT_SELL = 3, PAMG_FORMAT_SELL_DIAG = 4 };
 /* blocks of the split (own/ghost) storage of a level, PSparseMatrix own_own_values /
  * own_ghost_values (SURVEY.md App. A "PSparseMatrix") */
 enum { PAMG_A_OO = 0, PAMG_A_OG = 1, PAMG_P_OO = 2, PAMG_P_OG = 3, PAMG_R_OO = 4, PAMG_R_OG = 5 };
@@ -107,7 +112,8 @@ typedef struct {
   int32_t fused_halo;     /* 1 when the halo roles run inside the consuming kernels */
   int32_t tail_level;     /* first level of the replicated coarse tail (n_levels - 1: coarsest only) */
   int32_t value_indexed[16]; /* per level, bit mask 1 A / 2 P / 4 R: the SELL block stores one byte per entry into a dictionary of its
-                             <= 256 distinct fp64 values instead of the values (same products, same order, same bits) */
+                             <= 256 distinct fp64 values instead of the values (same products, same order, same bits); 8 / 16 / 32:
+                             two index bytes (wide dictionary); 64: A is stored with implied columns (pamg_layout_sell_diag) */
 } pamg_stats;
 
 void pamg_default_options(pamg_options* o);
@@ -211,6 +217,13 @@ int pamg_layout_sell(pamg_ctx* c, int32_t level, int32_t part, int32_t which, in
  * stores such blocks as int32 column + index byte(s) per entry (kernels.cuh k_spmv_sell_vi4); env PAMG_VALUE_INDEX=0 keeps fp64 values. */
 int pamg_layout_sell_values(pamg_ctx* c, int32_t level, int32_t part, int32_t which, int32_t rows_per_slice, int32_t sigma,
                             int32_t* indexed, int64_t* stored, double* dict, uint8_t* vidx);
+/* SELL with implied columns of the same block (which = PAMG_A_OO): *ndiag = 0 when the block does not qualify (see
+ * PAMG_FORMAT_SELL_DIAG).  Else off[*ndiag] (<= 32, ascending column offsets), dict[256] as pamg_layout_sell_values, and
+ * idx[*stored] with *stored = ceil(rows / 128) x ndiag x 128 bytes: slice sl, offset j, byte 4 lane + k (k < 4) at
+ * (sl ndiag + j) 128 + 4 lane + k holds the dictionary index of the entry (row, row + off[j]) for row = 128 sl + 32 k + lane (a full
+ * slice) or 128 sl + 4 lane + k (the partial last slice); 255 = no such entry. */
+int pamg_layout_sell_diag(pamg_ctx* c, int32_t level, int32_t part, int32_t which, int32_t* ndiag, int32_t* off, int64_t* stored,
+                          double* dict, uint8_t* idx);
 int pamg_layout_stream(pamg_ctx* c, int32_t level, int32_t part, int32_t which, int32_t max_rows, int32_t max_entries,
                        int64_t* n_blocks, int32_t* first_row, int32_t* first_entry);
 int pamg_layout_boundary(pamg_ctx* c, int32_t level, int32_t part, int32_t which, int64_t* n_rows, int64_t* n_entries,

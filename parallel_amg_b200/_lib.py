@@ -12,7 +12,7 @@ LIB_PATH = os.path.join(HERE, "libpamg.so")
 
 OK, ERR_ARG, ERR_CUDA, ERR_NOGPU, ERR_COMM, ERR_NOTCONV, ERR_ALLOC = 0, -1, -2, -3, -4, -5, -6
 SMOOTHER_JACOBI, SMOOTHER_L1JACOBI, SMOOTHER_CHEBYSHEV = 0, 1, 2
-FORMAT_AUTO, FORMAT_CSR, FORMAT_STREAM, FORMAT_SELL = 0, 1, 2, 3
+FORMAT_AUTO, FORMAT_CSR, FORMAT_STREAM, FORMAT_SELL, FORMAT_SELL_DIAG = 0, 1, 2, 3, 4
 CYCLE_V, CYCLE_W = 0, 1
 A_OO, A_OG, P_OO, P_OG, R_OO, R_OG = range(6)
 BLOCK_NAMES = ("A_oo", "A_og", "P_oo", "P_og", "R_oo", "R_og")
@@ -83,6 +83,7 @@ PROTOTYPES = {
     "pamg_hierarchy_end": [_ctx],
     "pamg_layout_sell": [_ctx, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _i64p, _i64p, _i32p, _i32p, _i32p, _f64p, _i32p],
     "pamg_layout_sell_values": [_ctx, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _i32p, _i64p, _f64p, _P(C.c_uint8)],
+    "pamg_layout_sell_diag": [_ctx, C.c_int32, C.c_int32, C.c_int32, _i32p, _i32p, _i64p, _f64p, _P(C.c_uint8)],
     "pamg_layout_stream": [_ctx, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _i64p, _i32p, _i32p],
     "pamg_layout_boundary": [_ctx, C.c_int32, C.c_int32, C.c_int32, _i64p, _i64p, _i32p, _i32p, _i32p, _i32p, _i32p, _f64p,
                              _P(C.c_uint8)],
@@ -383,6 +384,17 @@ class Context:
         self._ck(self.lib.pamg_layout_sell_values(self._h, level, part, which, rows_per_slice, sigma, C.byref(ix), C.byref(st),
                                                   _ptr(d, C.c_double), _ptr(v, C.c_uint8)))
         return d, (v if ix.value == 1 else v.view("<u2"))
+
+    def layout_sell_diag(self, level, part, which=A_OO):
+        """SELL with implied columns: dict(off, dict[256], idx[stored] uint8; 255 = no entry), or None when the block does not qualify."""
+        nd, st = C.c_int32(), C.c_int64()
+        self._ck(self.lib.pamg_layout_sell_diag(self._h, level, part, which, C.byref(nd), None, C.byref(st), None, None))
+        if not nd.value:
+            return None
+        off, d, idx = np.zeros(nd.value, np.int32), np.zeros(256), np.zeros(st.value, np.uint8)
+        self._ck(self.lib.pamg_layout_sell_diag(self._h, level, part, which, C.byref(nd), _ptr(off, C.c_int32), C.byref(st),
+                                                _ptr(d, C.c_double), _ptr(idx, C.c_uint8)))
+        return dict(off=off, dict=d, idx=idx)
 
     def layout_stream(self, level, part, which, max_rows=1024, max_entries=3069):
         nb = C.c_int64()

@@ -366,6 +366,26 @@ int pamg_layout_sell_values(pamg_ctx* c, int32_t level, int32_t part, int32_t wh
   });
 }
 
+int pamg_layout_sell_diag(pamg_ctx* c, int32_t level, int32_t part, int32_t which, int32_t* ndiag, int32_t* off, int64_t* stored,
+                          double* dict, uint8_t* idx) {
+  return guard(c, [&] {
+    const PartLevel& pl = part_level(c, level, part);
+    need(pl.full, "this part was loaded as metadata only (pamg_hierarchy_load keep_part)");
+    need(which == PAMG_A_OO || which == PAMG_P_OO || which == PAMG_R_OO, "SELL applies to own-own blocks");
+    need(ndiag && stored, "bad arguments");
+    DiagHost dh;
+    *ndiag = 0;
+    *stored = 0;
+    if (which != PAMG_A_OO || !diag_layout(pl.blk[which], dh, idx != nullptr)) return PAMG_OK;  // the upload takes it for A only
+    *ndiag = (int32_t)dh.off.size();
+    *stored = dh.nslices * (int64_t)dh.off.size() * 128;
+    if (off) std::memcpy(off, dh.off.data(), dh.off.size() * sizeof(int32_t));
+    if (dict) std::memcpy(dict, dh.dict.data(), 256 * sizeof(double));
+    if (idx) std::memcpy(idx, dh.idx.data(), dh.idx.size());
+    return PAMG_OK;
+  });
+}
+
 int pamg_layout_stream(pamg_ctx* c, int32_t level, int32_t part, int32_t which, int32_t max_rows, int32_t max_entries,
                        int64_t* n_blocks, int32_t* first_row, int32_t* first_entry) {
   return guard(c, [&] {

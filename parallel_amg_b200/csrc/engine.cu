@@ -27,6 +27,8 @@
 
 namespace pamg {
 
+static_assert(DIAG_MAX_OFFSETS == SELL_DIAG_MAX && DIAG_ABSENT == SELL_DIAG_ABSENT, "formats.hpp and kernels.cuh disagree on the diagonal layout");
+
 #define CK(call)                                                                                      \
   do {                                                                                                \
     cudaError_t e_ = (call);                                                                          \
@@ -92,6 +94,12 @@ struct DevCsr {
   bool sell_vi4 = false;
   int vi4_ib = 1;   // bytes per index of the 128-row layout: 1 (<= 255 distinct values) or 2 (wide: <= VI_WIDE_MAX - 1)
   int ndict = 256;  // dictionary entries uploaded
+  // SELL with implied columns (stencil A blocks, kernels.cuh k_spmv_sell_diag): only these arrays (and sl_dict) are uploaded
+  DBuf<uint32_t> dg_idx;
+  DBuf<int32_t> dg_off;
+  int ndiag = 0;
+  bool sell_diag = false;
+  SellDiagView diagview() const { return SellDiagView{dg_idx.p, sl_dict.p, dg_off.p, nrows, nslices4, ndiag}; }
   SellViView vi4view() const { return SellViView{v4_off.p, v4_col.p, v4_idx.p, sl_dict.p, nullptr, nrows, nslices4, ndict}; }
   SellViView viview() const { return SellViView{sl_off.p, sl_col.p, sl_vidx.p, sl_dict.p, sell_perm ? sl_perm.p : nullptr, nrows, nslices, 256}; }
   CsrView view() const { return CsrView{ptr.p, col.p, val.p, listed ? rows.p : nullptr, nrows}; }
@@ -206,6 +214,7 @@ void build_csr(const LocalCsr& m, bool compress, DevCsr& d, int lanes_override, 
   d.sell_rpt = 0;
   d.sell_vi = false;
   d.sell_vi4 = false;
+  d.sell_diag = false;
   d.short_rows = false;
   if (!m.ptr.empty()) {
     int64_t mx = 0;
@@ -245,10 +254,35 @@ void build_csr(const LocalCsr& m, bool compress, DevCsr& d, int lanes_override, 
     if (which == PAMG_A_OO || which == PAMG_P_OO) auto_sell = nr >= SELL_AUTO_MIN_ROWS_A;
     if (which == PAMG_R_OO) auto_sell = nr >= SELL_AUTO_MIN_ROWS_R;
   }
-  if (!compress && nr > 0 && (fmt == PAMG_FORMAT_SELL || auto_sell)) {
+  const bool sell_req = fmt == PAMG_FORMAT_SELL || fmt == PAMG_FORMAT_SELL_DIAG;
+  if (!compress && nr > 0 && (sell_req || auto_sell)) {
     const int rpt = (o.sell_rows_per_thread == 1 || o.sell_rows_per_thread == 2) ? o.sell_rows_per_thread
                     : (rpt_override == 1 && d.short_rows)                             ? 1
                                                                                       : 2;
+    // stencil A blocks: implied columns, one index byte per slot (0.117 instead of 0.585 GB per pass over A0 at 256^3); only under AUTO and
+    // SELL_DIAG (an explicit SELL keeps the column-stored layouts), and like every value-indexed layout not with PAMG_VALUE_INDEX=0
+    const char* ve = getenv("PAMG_VALUE_INDEX");
+    DiagHost dh;
+    if (which == PAMG_A_OO && fmt != PAMG_FORMAT_SELL && rpt == 2 && !(ve && atoi(ve) == 0) && diag_layout(m, dh, true)) {
+      d.sl_dict.upload(dh.dict);
+      d.ndict = (int)dh.dict.size();
+      d.dg_off.upload(dh.off);
+      std::vector<uint32_t> words(dh.idx.size() / 4);
+      std::memcpy(words.data(), dh.idx.data(), dh.idx.size());
+      d.dg_idx.upload(words);
+      d.ndiag = (int)dh.off.size();
+      d.nslices4 = (int)dh.nslices;
+      d.nslices = 0;
+      d.sell_diag = true;
+      d.sell_rpt = 2;
+      d.sell_perm = false;
+      d.sell_sigma = 1;
+      d.sell_fill = (double)d.ndiag * (double)nr / (double)d.nnz;
+      d.ptr.alloc(1);
+      d.col.alloc(16);
+      d.val.alloc(16);
+      return;
+    }
     const int C = 32 * rpt;
     SellHost sh;
     int sigma = o.sell_sigma > 0 ? o.sell_sigma : 1;
@@ -278,7 +312,7 @@ void build_csr(const LocalCsr& m, bool compress, DevCsr& d, int lanes_override, 
       if (s2.fill < sh.fill - 0.02) sigma = 64 * C;
       sh.fill = std::min(sh.fill, s2.fill);
     }
-    const bool take = fmt == PAMG_FORMAT_SELL || sh.fill <= std::max(SELL_AUTO_MAX_FILL, sort_fill);
+    const bool take = sell_req || sh.fill <= std::max(SELL_AUTO_MAX_FILL, sort_fill);
     if (take) {
       sell_layout(m, C, sigma, sh, true);
       d.sl_off.upload(sh.off);
@@ -787,6 +821,16 @@ void launch_sell(int mode, bool dot, int rpt, int short_variant, bool prefetch, 
   });
 }
 
+// grid as for the vi4 kernel it replaces (same occupancy): the same resident CTAs, so the fused dots add in the same order
+void launch_sell_diag(int mode, bool dot, const SellDiagView& A, const LaunchArgs& L) {
+  dispatch_mode(mode, dot, [&](auto md, auto dt) {
+    constexpr int MD = decltype(md)::value;
+    constexpr bool DT = decltype(dt)::value;
+    auto k = k_spmv_sell_diag<MD, DT>;
+    k<<<main_grid(L, (const void*)k), BLOCK, 0, L.s>>>(A, L.x, L.a, L.st, L.fh, L.partials, L.rc, L.publish, L.slot);
+  });
+}
+
 void launch_boundary(int mode, bool dot, const LaunchArgs& L) {
   dispatch_mode(mode, dot, [&](auto md, auto dt) {
     k_boundary<decltype(md)::value, decltype(dt)::value><<<L.grid, BLOCK, 0, L.s>>>(L.x, L.a, L.st, L.fh, L.partials, L.rc, L.slot);
@@ -873,7 +917,7 @@ void Engine::enqueue_op(const OpSpec& op, const std::vector<const double*>& xin,
     const double mean_nnz = m.nrows ? (double)m.nnz / m.nrows : 0.0;
     // PAMG_UNIFIED bit mask: 1 = A with short rows, 2 = A with long rows, 4 = P, 8 = R
     const int uni_bit = op.which == PAMG_P_OO ? 4 : op.which == PAMG_R_OO ? 8 : (mean_nnz <= 12.0 ? 1 : 2);
-    const bool try_unified = fused && (I.unified & uni_bit) && m.sell_rpt && (fh.n_pack > 0 || fh.n_bnd > 0);
+    const bool try_unified = fused && (I.unified & uni_bit) && m.sell_rpt && !m.sell_diag && (fh.n_pack > 0 || fh.n_bnd > 0);
     // PAMG_SELL_PF bit mask: 1 = P, 2 = A with long rows, 4 = R (these then run persistent, which the prefetch needs)
     const int pf_bit = op.which == PAMG_P_OO ? 1 : op.which == PAMG_R_OO ? 4 : (mean_nnz > 12.0 ? 2 : 0);
     const bool prefetch = I.persistent && m.sell_rpt == 2 && (I.sell_pf & pf_bit) && !op.dot && !try_unified;
@@ -894,8 +938,10 @@ void Engine::enqueue_op(const OpSpec& op, const std::vector<const double*>& xin,
     SellViView viv{};
     const bool use_vi4 = m.sell_vi4 && I.vi_variant == 3 && !try_unified;
     if (m.sell_vi || use_vi4) viv = use_vi4 ? m.vi4view() : m.viview();
-    if (use_vi4) L.grid = std::max((m.nslices4 + BLOCK / 32 - 1) / (BLOCK / 32), 1);
-    if (m.sell_rpt)
+    if (use_vi4 || m.sell_diag) L.grid = std::max((m.nslices4 + BLOCK / 32 - 1) / (BLOCK / 32), 1);
+    if (m.sell_diag)
+      launch_sell_diag(op.mode, op.dot, m.diagview(), L);
+    else if (m.sell_rpt)
       launch_sell(op.mode, op.dot, m.sell_rpt, (op.which == PAMG_P_OO && m.short_rows) ? I.p_kernel : 0, prefetch, m.slview(), L,
                   try_unified, I.unified_mode, &was_unified, (m.sell_vi || use_vi4) ? &viv : nullptr,
                   use_vi4 ? (m.vi4_ib == 2 ? 4 : 3) + (I.vi_ahead && L.bounded ? 2 : 0) : (I.vi_variant == 3 ? 0 : I.vi_variant), I.vi_occ);  // blocks without the 128-row layout (sorted rows): two rows per lane
@@ -906,7 +952,7 @@ void Engine::enqueue_op(const OpSpec& op, const std::vector<const double*>& xin,
     if (I.naming) {
       static const char* MODES[] = {"mul", "resid", "jacobi", "add", "restrict", "cheb"};
       static const char* OPS[] = {"A", "P", "R"};
-      I.names.push_back(std::string(m.sell_rpt ? ((m.sell_vi || use_vi4) && !was_unified ? (use_vi4 && m.vi4_ib == 2 ? "sell-vi16 " : "sell-vi ") : "sell ") : m.stream ? "stream " : "csr ") + MODES[op.mode] + (op.dot ? "+dot " : " ") +
+      I.names.push_back(std::string(m.sell_diag ? "sell-diag " : m.sell_rpt ? ((m.sell_vi || use_vi4) && !was_unified ? (use_vi4 && m.vi4_ib == 2 ? "sell-vi16 " : "sell-vi ") : "sell ") : m.stream ? "stream " : "csr ") + MODES[op.mode] + (op.dot ? "+dot " : " ") +
                         OPS[wsel] + std::to_string(l) + (I.tail_mode ? " tail" : "") + (fh.n_pack ? " +pack" : "") +
                         (fh.n_bnd ? " +bnd" : "") + (was_unified ? " uni" : ""));
       I.naming = false;
@@ -1073,7 +1119,7 @@ Engine::Engine(Hierarchy* h, int nlocal, const int32_t* local_parts, const int32
       if (re && atoi(re) != 0)  // off by default: measured a net loss at 256^3 (profiles/r02_kernel_sweep.md)
         for (int l = 1; l < I.L; ++l) {
           const PartLevel& pl = h->levels[l].parts[part];
-          const bool sell = o.spmv_format == PAMG_FORMAT_SELL || (o.spmv_format == PAMG_FORMAT_AUTO && pl.n_own >= SELL_AUTO_MIN_ROWS_A);
+          const bool sell = o.spmv_format == PAMG_FORMAT_SELL || o.spmv_format == PAMG_FORMAT_SELL_DIAG || (o.spmv_format == PAMG_FORMAT_AUTO && pl.n_own >= SELL_AUTO_MIN_ROWS_A);
           if (sell) plan_renumbering(pl, &h->levels[l - 1].parts[part], 64, window, pd.renum[l]);
         }
     }
@@ -1103,7 +1149,7 @@ Engine::Engine(Hierarchy* h, int nlocal, const int32_t* local_parts, const int32
         build_csr(oo, false, ld.blk[b], lanes, o.spmv_format, o, b, b == PAMG_P_OO && I.p_kernel == 2 ? 1 : 0);
         build_bnd(oo, og, ld.bnd[b / 2]);
         max_blocks = std::max(max_blocks, ld.blk[b].nblocks);
-        max_blocks = std::max(max_blocks, (ld.blk[b].nslices + BLOCK / 32 - 1) / (BLOCK / 32));
+        max_blocks = std::max(max_blocks, (std::max(ld.blk[b].nslices, ld.blk[b].nslices4) + BLOCK / 32 - 1) / (BLOCK / 32));
       }
       // smoother weights (device numbering)
       std::vector<double> w(pl.n_own), dinv(pl.n_own);
@@ -2729,10 +2775,11 @@ void Engine::get_stats(pamg_stats* s) {
     s->value_indexed[l] = 0;
     if (have) {
       const LevelDev& ld = *I.P(0).lev[l];
-      auto vi_of = [](const DevCsr& m) { return m.sell_vi || m.sell_vi4; };
+      auto vi_of = [](const DevCsr& m) { return m.sell_vi || m.sell_vi4 || m.sell_diag; };
       auto wide_of = [](const DevCsr& m) { return m.sell_vi4 && m.vi4_ib == 2; };
       s->value_indexed[l] = (vi_of(ld.blk[PAMG_A_OO]) ? 1 : 0) | (vi_of(ld.blk[PAMG_P_OO]) ? 2 : 0) | (vi_of(ld.blk[PAMG_R_OO]) ? 4 : 0) |
-                            (wide_of(ld.blk[PAMG_A_OO]) ? 8 : 0) | (wide_of(ld.blk[PAMG_P_OO]) ? 16 : 0) | (wide_of(ld.blk[PAMG_R_OO]) ? 32 : 0);
+                            (wide_of(ld.blk[PAMG_A_OO]) ? 8 : 0) | (wide_of(ld.blk[PAMG_P_OO]) ? 16 : 0) | (wide_of(ld.blk[PAMG_R_OO]) ? 32 : 0) |
+                            (ld.blk[PAMG_A_OO].sell_diag ? 64 : 0);
     }
   }
 }

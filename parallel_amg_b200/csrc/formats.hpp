@@ -168,6 +168,95 @@ inline void sell_layout(const LocalCsr& m, int C, int sigma, SellHost& out, bool
   }
 }
 
+// ---- SELL with implied columns ("diagonal" layout, kernels.cuh k_spmv_sell_diag) -----------------------------
+// Stencil operators hold every row's entries at columns row + off[j] for a few fixed offsets.  Slot j of every row then stands
+// for column row + off[j], so a slot stores its one value-index byte and no column.  Slices of 128 rows; inside a slice
+// ndiag groups of 128 bytes, one per offset (diagonal-major), each with the four-rows-per-lane interleave of the 128-row
+// value-indexed layout: byte 4 lane + k is row base + 32 k + lane of a full slice, row base + 4 lane + k of the partial last
+// slice.  Code DIAG_ABSENT marks a slot without an entry (rows at the domain boundary, tail rows of the last slice).
+// A block qualifies when every row's columns are strictly ascending (then ascending offset = stored order, so the kernel adds
+// the products in CSR order), it has at most DIAG_MAX_OFFSETS distinct offsets, ndiag * nrows <= DIAG_MAX_FILL * nnz, and at
+// most DIAG_MAX_VALUES distinct non-zero values (value_dictionary's dictionary and order; code 255 stays free).
+constexpr int DIAG_MAX_OFFSETS = 32;
+constexpr double DIAG_MAX_FILL = 1.25;
+constexpr int DIAG_MAX_VALUES = 254;
+constexpr uint8_t DIAG_ABSENT = 255;
+
+struct DiagHost {
+  std::vector<int32_t> off;  // [ndiag] ascending; empty when the block does not qualify
+  std::vector<double> dict;  // [256] (value_dictionary)
+  std::vector<uint8_t> idx;  // [nslices * ndiag * 128]
+  int64_t nslices = 0;
+};
+
+// Returns false (out.off empty) when m does not qualify; fill_arrays = false stops after the checks.
+inline bool diag_layout(const LocalCsr& m, DiagHost& out, bool fill_arrays) {
+  out = DiagHost();
+  const int64_t nr = m.nrows, nnz = m.nnz();
+  if (nr <= 0 || m.ncols != nr || m.ptr.empty() || nnz == 0 || nr > INT32_MAX / 2) return false;
+  std::vector<int64_t> all;
+  bool refused = false;
+#pragma omp parallel
+  {
+    std::vector<int64_t> mine;  // sorted, at most DIAG_MAX_OFFSETS + 1 entries
+#pragma omp for schedule(static)
+    for (int64_t i = 0; i < nr; ++i) {
+      bool stop;
+#pragma omp atomic read
+      stop = refused;
+      if (stop) continue;
+      bool ok = true;
+      for (int64_t k = m.ptr[i]; k < m.ptr[i + 1] && ok; ++k) {
+        if (k > m.ptr[i] && m.col[k] <= m.col[k - 1]) ok = false;
+        const int64_t o = (int64_t)m.col[k] - i;
+        auto it = std::lower_bound(mine.begin(), mine.end(), o);
+        if (it == mine.end() || *it != o) {
+          mine.insert(it, o);
+          if ((int)mine.size() > DIAG_MAX_OFFSETS) ok = false;
+        }
+      }
+      if (!ok) {
+#pragma omp atomic write
+        refused = true;
+      }
+    }
+#pragma omp critical
+    all.insert(all.end(), mine.begin(), mine.end());
+  }
+  if (refused) return false;
+  std::sort(all.begin(), all.end());
+  all.erase(std::unique(all.begin(), all.end()), all.end());
+  const int nd = (int)all.size();
+  if (nd > DIAG_MAX_OFFSETS || (double)nd * (double)nr > DIAG_MAX_FILL * (double)nnz) return false;
+  if (!value_dictionary(m, out.dict, DIAG_MAX_VALUES)) return false;
+  out.off.assign(all.begin(), all.end());
+  out.nslices = (nr + 127) / 128;
+  if (!fill_arrays) return true;
+  std::vector<uint64_t> key(1, 0);  // dictionary bit patterns behind dict[0] = +0.0
+  for (int i = 1; i < (int)out.dict.size(); ++i) {
+    uint64_t b;
+    std::memcpy(&b, &out.dict[i], sizeof(b));
+    if (b == 0) break;
+    key.push_back(b);
+  }
+  out.idx.assign((size_t)out.nslices * nd * 128, DIAG_ABSENT);
+#pragma omp parallel for schedule(static)
+  for (int64_t i = 0; i < nr; ++i) {
+    const int64_t sl = i / 128, q = i % 128;
+    const int64_t pos = (sl + 1) * 128 <= nr ? (q % 32) * 4 + q / 32 : q;
+    int j = 0;
+    for (int64_t k = m.ptr[i]; k < m.ptr[i + 1]; ++k) {
+      const int64_t o = (int64_t)m.col[k] - i;
+      while (out.off[j] != o) ++j;  // both ascending, o is one of the offsets
+      uint64_t b;
+      std::memcpy(&b, &m.val[k], sizeof(b));
+      const uint8_t code = b == 0 ? 0 : (uint8_t)(std::lower_bound(key.begin() + 1, key.end(), b) - key.begin());
+      out.idx[(size_t)(sl * nd + j) * 128 + pos] = code;
+    }
+  }
+  return true;
+}
+
 // ---- CSR-stream row blocks -----------------------------------------------------------------------------
 // Greedy runs of consecutive rows with <= max_rows rows and <= max_entries entries; blk[k] = {first row, first
 // entry}, closed by {nrows, nnz}.  Returns false (blk unusable) when a single row exceeds max_entries.

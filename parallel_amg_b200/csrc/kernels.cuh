@@ -7,7 +7,8 @@
 //   a4 prolong+correct out = x + P e_c
 // so one templated kernel family (three storage formats) covers them.  Operators with few distinct values (the three
 // BASELINE matrices and their prolongators) run the value-indexed SELL kernels (k_spmv_sell_vi4: int32 column + index
-// byte(s) into a dictionary of the original doubles, 5-6 instead of 12 bytes per entry, same bits).
+// byte(s) into a dictionary of the original doubles, 5-6 instead of 12 bytes per entry, same bits); stencil operators store no
+// column at all (k_spmv_sell_diag: one index byte per (row, offset) slot, the column is row + offset).
 //
 // Halo exchange (PartitionedArrays mul!: start consistent!(b); c_own = A_oo b_own; wait;
 // c_own += A_og b_ghost, SURVEY App. A) is FUSED INTO THE SAME KERNEL as three CTA roles:
@@ -1270,6 +1271,62 @@ __device__ __forceinline__ unsigned vi_index(const uint2& v, int k) { return ((k
 __device__ __forceinline__ unsigned vi_bits(unsigned v) { return v; }
 __device__ __forceinline__ unsigned vi_bits(const uint2& v) { return v.x | v.y; }
 
+// The four rows of a lane in the 128-row layouts: r_first + k rstep, k = 0..3 (rstep 32 in a full slice, 1 in the partial last one).
+// Their epilogue operands are requested into L1 before the entry loop ...
+template <int MODE, bool DOT>
+__device__ __forceinline__ void rows4_prefetch(const EpiArgs& a, const FusedHalo& fh, int r_first, int rstep, int nrows) {
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    const int r = r_first + k * rstep;
+    if (r < nrows) {
+      if (fh.skip) asm volatile("prefetch.global.L1 [%0];" ::"l"(fh.skip + r));
+      if (MODE == M_RESID || MODE == M_JACOBI || MODE == M_ADD || MODE == M_CHEB) prefetch_l1(a.in0 + r);
+      if (MODE == M_JACOBI || MODE == M_CHEB || (MODE == M_RESTRICT && a.out2)) prefetch_l1(a.w + r);
+      if (MODE == M_CHEB && a.aux) prefetch_l1(a.aux + r);
+      if (DOT && a.dotv != a.in0) prefetch_l1(a.dotv + r);
+    }
+  }
+}
+
+// ... and the epilogue runs two rows at a time: their operand loads first (L1 hits), then arithmetic and stores.  Returns the lane's dot
+// contribution, added over its rows in order k = 0..3.
+template <int MODE, bool DOT>
+__device__ __forceinline__ double rows4_epilogue(const EpiArgs& a, const FusedHalo& fh, const double (&s)[4], int r_first, int rstep,
+                                                 int nrows) {
+  double contrib = 0.0;
+#pragma unroll
+  for (int h = 0; h < 4; h += 2) {
+    bool live[2];
+    double e_in0[2], e_in1[2], e_w[2], e_aux[2], e_dot[2];
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      const int r = r_first + (h + k) * rstep;
+      live[k] = r < nrows && !(fh.skip && fh.skip[r]);
+      e_in0[k] = e_in1[k] = e_w[k] = e_aux[k] = e_dot[k] = 0.0;
+    }
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      const int r = r_first + (h + k) * rstep;
+      if (live[k]) {
+        if (MODE == M_RESID || MODE == M_JACOBI || MODE == M_ADD || MODE == M_CHEB) e_in0[k] = a.in0[r];
+        if (MODE == M_JACOBI || MODE == M_CHEB) e_in1[k] = a.in1[r];
+        if (MODE == M_JACOBI || MODE == M_CHEB || (MODE == M_RESTRICT && a.out2)) e_w[k] = a.w[r];
+        if (MODE == M_CHEB && a.aux) e_aux[k] = a.aux[r];
+        if (DOT) e_dot[k] = (a.dotv == a.in0 && (MODE == M_JACOBI || MODE == M_RESID)) ? e_in0[k] : a.dotv[r];
+      }
+    }
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      const int r = r_first + (h + k) * rstep;
+      if (live[k]) {
+        const double res = stream_epilogue<MODE>(a, r, s[h + k], e_in0[k], e_in1[k], e_w[k], e_aux[k]);
+        if (DOT) contrib += e_dot[k] * res;
+      }
+    }
+  }
+  return contrib;
+}
+
 // AHEAD = 1: the extents of a warp's NEXT slice are loaded one iteration early and that slice's columns / indices are requested into L2
 // (prefetch.global.L2: no register, no scoreboard), which takes the extents latency off the per-slice chain and turns the column latency
 // from HBM into L2.
@@ -1326,17 +1383,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) k_spmv_sell_vi4(SellViView A, con
     // row of (lane, k): 32 apart in a full slice, adjacent in the partial last one
     const int rstep = full ? 32 : 1;
     const int r_first = full ? base + lane : base + lane * 4;
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      const int r = r_first + k * rstep;
-      if (r < A.nrows) {
-        if (fh.skip) asm volatile("prefetch.global.L1 [%0];" ::"l"(fh.skip + r));
-        if (MODE == M_RESID || MODE == M_JACOBI || MODE == M_ADD || MODE == M_CHEB) prefetch_l1(a.in0 + r);
-        if (MODE == M_JACOBI || MODE == M_CHEB || (MODE == M_RESTRICT && a.out2)) prefetch_l1(a.w + r);
-        if (MODE == M_CHEB && a.aux) prefetch_l1(a.aux + r);
-        if (DOT && a.dotv != a.in0) prefetch_l1(a.dotv + r);
-      }
-    }
+    rows4_prefetch<MODE, DOT>(a, fh, r_first, rstep, A.nrows);
     double s[4] = {0.0, 0.0, 0.0, 0.0};
     const int4* __restrict__ cj = reinterpret_cast<const int4*>(A.col) + (size_t)o0 * 32 + lane;
     using IV = typename std::conditional<IB == 1, unsigned, uint2>::type;
@@ -1383,38 +1430,89 @@ __global__ void __launch_bounds__(BLOCK, MINB) k_spmv_sell_vi4(SellViView A, con
       for (int q = lane; q < wc * 4; q += 32) asm volatile("prefetch.global.L2 [%0];" ::"l"(pc + (size_t)q * 128));
       for (int q = lane; q < wc * IB; q += 32) asm volatile("prefetch.global.L2 [%0];" ::"l"(pi + (size_t)q * 128));
     }
-    // epilogue, two rows at a time: their operand loads first (L1 hits, requested before the entry loop), then arithmetic and stores
-    double contrib = 0.0;
+    const double contrib = rows4_epilogue<MODE, DOT>(a, fh, s, r_first, rstep, A.nrows);
+    if (DOT) s_acc[threadIdx.x] += contrib;
+  }
+  if (DOT) dot_finish(s_acc[threadIdx.x], partials, st, &st->ticket[0], rc, publish, 0, red_slot);
+}
+
+// SELL with implied columns (formats.hpp diag_layout): stencil operators, whose rows hold their entries at row + off[j] for at most
+// SELL_DIAG_MAX fixed offsets.  A slot stores only its index byte (1 byte per slot instead of 5 per entry: at 256^3 the matrix is
+// 0.117 instead of 0.585 GB per pass), and every x address is row + off[j], known before any load: no column -> gather chain, and the
+// 32 lanes of a warp read 32 consecutive doubles per diagonal.  Same slice -> warp -> lane map, same per-row product order
+// (ascending offset = ascending column = stored order) and the same epilogue as k_spmv_sell_vi4, so with the same grid every row result
+// AND the fused dot products are bit-identical to it.  An absent slot leaves the sum untouched (the vi4 kernel's row padding adds
+// +0.0 * x, which cannot change a sum that starts at +0.0 when x is finite).
+constexpr int SELL_DIAG_MAX = 32;
+constexpr unsigned SELL_DIAG_ABSENT = 255u;
+struct SellDiagView {
+  const uint32_t* idx;  // [nslices * ndiag * 32] words: byte k of word (sl * ndiag + j) * 32 + lane = row k of the lane on diagonal j
+  const double* dict;   // [256]
+  const int32_t* off;   // [ndiag] ascending column offsets
+  int32_t nrows, nslices, ndiag;
+};
+
+// U = 2 diagonals per step: no spills at 64 registers (4 CTAs/SM, the vi4 launch's occupancy); U = 3 spills in JACOBI + DOT, U = 4 in
+// five of the eight instantiations.
+template <int MODE, bool DOT, int U = 2, int MINB = 4>
+__global__ void __launch_bounds__(BLOCK, MINB) k_spmv_sell_diag(SellDiagView A, const double* __restrict__ x, EpiArgs a, DevState* st,
+                                                              FusedHalo fh, double* partials, RedCtx rc, int publish, int red_slot) {
+  if (st->done) return;
+  trace_mark(st);
+  const int n_main = (int)gridDim.x - fh.n_pack - fh.n_bnd;
+  const int bid = (int)blockIdx.x - fh.n_pack - (fh.bnd_first ? fh.n_bnd : 0);
+  const int b0 = fh.n_pack + (fh.bnd_first ? 0 : n_main);  // first boundary CTA
+  if ((int)blockIdx.x < fh.n_pack || ((int)blockIdx.x >= b0 && (int)blockIdx.x < b0 + fh.n_bnd)) {  // halo roles
+    double racc = 0.0;
+    if ((int)blockIdx.x < fh.n_pack)
+      pack_role(fh, st, blockIdx.x);
+    else
+      racc = boundary_role<MODE, DOT>(fh, x, a, st, (int)blockIdx.x - b0);
+    if (DOT) dot_finish(racc, partials, st, &st->ticket[0], rc, publish, 0, red_slot);
+    return;
+  }
+  __shared__ double s_dict[256];
+  __shared__ int s_off[SELL_DIAG_MAX];
+  __shared__ double s_acc[DOT ? BLOCK : 1];
+  s_dict[threadIdx.x] = A.dict[threadIdx.x];  // BLOCK == 256
+  if (threadIdx.x < A.ndiag) s_off[threadIdx.x] = A.off[threadIdx.x];
+  if (DOT) s_acc[threadIdx.x] = 0.0;
+  __syncthreads();
+  const int lane = threadIdx.x & 31;
+  const int wpb = BLOCK / 32;
+  const int last = A.nrows - 1;
+  for (int sl = bid * wpb + (threadIdx.x >> 5); sl < A.nslices; sl += n_main * wpb) {
+    const int base = sl * 128;
+    const bool full = base + 128 <= A.nrows;
+    const int rstep = full ? 32 : 1;
+    const int r_first = full ? base + lane : base + lane * 4;
+    rows4_prefetch<MODE, DOT>(a, fh, r_first, rstep, A.nrows);
+    double s[4] = {0.0, 0.0, 0.0, 0.0};
+    const uint32_t* __restrict__ ij = A.idx + (size_t)sl * A.ndiag * 32 + lane;
+#pragma unroll 1
+    for (int j0 = 0; j0 < A.ndiag; j0 += U) {
+      unsigned iv[U];
+      double xv[U][4];
+      // x addresses come from the row and the offset only (clamped into the vector; an absent slot's value is never used)
 #pragma unroll
-    for (int h = 0; h < 4; h += 2) {
-      bool live[2];
-      double e_in0[2], e_in1[2], e_w[2], e_aux[2], e_dot[2];
+      for (int u = 0; u < U; ++u)
+        if (j0 + u < A.ndiag) {
+          iv[u] = __ldcs(ij + (j0 + u) * 32);
+          const int o = s_off[j0 + u];
 #pragma unroll
-      for (int k = 0; k < 2; ++k) {
-        const int r = r_first + (h + k) * rstep;
-        live[k] = r < A.nrows && !(fh.skip && fh.skip[r]);
-        e_in0[k] = e_in1[k] = e_w[k] = e_aux[k] = e_dot[k] = 0.0;
-      }
-#pragma unroll
-      for (int k = 0; k < 2; ++k) {
-        const int r = r_first + (h + k) * rstep;
-        if (live[k]) {
-          if (MODE == M_RESID || MODE == M_JACOBI || MODE == M_ADD || MODE == M_CHEB) e_in0[k] = a.in0[r];
-          if (MODE == M_JACOBI || MODE == M_CHEB) e_in1[k] = a.in1[r];
-          if (MODE == M_JACOBI || MODE == M_CHEB || (MODE == M_RESTRICT && a.out2)) e_w[k] = a.w[r];
-          if (MODE == M_CHEB && a.aux) e_aux[k] = a.aux[r];
-          if (DOT) e_dot[k] = (a.dotv == a.in0 && (MODE == M_JACOBI || MODE == M_RESID)) ? e_in0[k] : a.dotv[r];
+          for (int k = 0; k < 4; ++k) xv[u][k] = x[min(max(r_first + k * rstep + o, 0), last)];
         }
-      }
 #pragma unroll
-      for (int k = 0; k < 2; ++k) {
-        const int r = r_first + (h + k) * rstep;
-        if (live[k]) {
-          const double res = stream_epilogue<MODE>(a, r, s[h + k], e_in0[k], e_in1[k], e_w[k], e_aux[k]);
-          if (DOT) contrib += e_dot[k] * res;
+      for (int u = 0; u < U; ++u)
+        if (j0 + u < A.ndiag) {
+#pragma unroll
+          for (int k = 0; k < 4; ++k) {
+            const unsigned v = vi_index(iv[u], k);
+            if (v != SELL_DIAG_ABSENT) s[k] = __dadd_rn(s[k], __dmul_rn(s_dict[v], xv[u][k]));
+          }
         }
-      }
     }
+    const double contrib = rows4_epilogue<MODE, DOT>(a, fh, s, r_first, rstep, A.nrows);
     if (DOT) s_acc[threadIdx.x] += contrib;
   }
   if (DOT) dot_finish(s_acc[threadIdx.x], partials, st, &st->ticket[0], rc, publish, 0, red_slot);
