@@ -939,6 +939,7 @@ void Engine::enqueue_op(const OpSpec& op, const std::vector<const double*>& xin,
     const bool use_vi4 = m.sell_vi4 && I.vi_variant == 3 && !try_unified;
     if (m.sell_vi || use_vi4) viv = use_vi4 ? m.vi4view() : m.viview();
     if (use_vi4 || m.sell_diag) L.grid = std::max((m.nslices4 + BLOCK / 32 - 1) / (BLOCK / 32), 1);
+    const bool long_rows = I.stream_long && mean_nnz >= 48.0 && !op.dot;  // CSR-stream phase B with 16 lanes per row (no DOT form)
     if (m.sell_diag)
       launch_sell_diag(op.mode, op.dot, m.diagview(), L);
     else if (m.sell_rpt)
@@ -946,13 +947,16 @@ void Engine::enqueue_op(const OpSpec& op, const std::vector<const double*>& xin,
                   try_unified, I.unified_mode, &was_unified, (m.sell_vi || use_vi4) ? &viv : nullptr,
                   use_vi4 ? (m.vi4_ib == 2 ? 4 : 3) + (I.vi_ahead && L.bounded ? 2 : 0) : (I.vi_variant == 3 ? 0 : I.vi_variant), I.vi_occ);  // blocks without the 128-row layout (sorted rows): two rows per lane
     else if (m.stream)
-      launch_stream(op.mode, op.dot, I.stream_long && mean_nnz >= 48.0, m.sview(), L);
+      launch_stream(op.mode, op.dot, long_rows, m.sview(), L);
     else
       launch_csr(op.mode, op.dot, m.lanes, m.view(), L);
     if (I.naming) {
       static const char* MODES[] = {"mul", "resid", "jacobi", "add", "restrict", "cheb"};
       static const char* OPS[] = {"A", "P", "R"};
-      I.names.push_back(std::string(m.sell_diag ? "sell-diag " : m.sell_rpt ? ((m.sell_vi || use_vi4) && !was_unified ? (use_vi4 && m.vi4_ib == 2 ? "sell-vi16 " : "sell-vi ") : "sell ") : m.stream ? "stream " : "csr ") + MODES[op.mode] + (op.dot ? "+dot " : " ") +
+      // the name says which kernel ran: sell-vi = four rows per lane (one-byte indices), sell-vi16 = the same with two-byte
+      // indices, sell-vi2 = two rows per lane (sorted rows), stream-long = CSR-stream with 16 lanes per row in phase B
+      const char* vi_name = use_vi4 ? (m.vi4_ib == 2 ? "sell-vi16 " : "sell-vi ") : "sell-vi2 ";
+      I.names.push_back(std::string(m.sell_diag ? "sell-diag " : m.sell_rpt ? ((m.sell_vi || use_vi4) && !was_unified ? vi_name : "sell ") : m.stream ? (long_rows ? "stream-long " : "stream ") : "csr ") + MODES[op.mode] + (op.dot ? "+dot " : " ") +
                         OPS[wsel] + std::to_string(l) + (I.tail_mode ? " tail" : "") + (fh.n_pack ? " +pack" : "") +
                         (fh.n_bnd ? " +bnd" : "") + (was_unified ? " uni" : ""));
       I.naming = false;
