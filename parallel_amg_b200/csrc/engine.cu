@@ -378,90 +378,6 @@ void build_csr(const LocalCsr& m, bool compress, DevCsr& d, int lanes_override, 
   }
 }
 
-// ---- upload-time renumbering of the own rows of a coarse level -------------------------------------------------------
-// SELL stores max-row-length entries for every row of a 64-row slice.  On the coarse levels of smoothed aggregation the row
-// lengths of A vary with the position of the aggregate (256^3, level 1: 8 .. 47 entries, mean 31), so consecutive rows pad
-// each other: 1.16x stored entries, and the level-1 sweeps were traffic-bound at 0.80 of the roofline (ncu r01).  A run-time
-// row permutation inside the kernel costs more than it saves (scattered epilogue accesses), so the own rows of a level >= 1
-// are RENUMBERED once at upload: sorted by row length inside windows of a few thousand rows, the same permutation applied to
-// A's rows and columns, P_{l-1}'s columns, R_{l-1}'s rows, P_l's rows, R_l's columns, the smoother weights, the halo send
-// lists and the tail gather map.  Entry order inside a row is kept, so every row sum adds the same products in the same
-// order: results are unchanged bit for bit; only the (internal) position of a row in the device vectors moves.  Host
-// vectors of such a level are permuted in upload_vec / download_vec.  Level 0 is never renumbered (PCG vectors, b and x).
-struct Renumbering {
-  std::vector<int32_t> old_of_new, new_of_old;  // empty: identity
-  bool active() const { return !old_of_new.empty(); }
-};
-
-double sell_fill_of(const std::vector<int32_t>& len, const std::vector<int32_t>* order, int C) {
-  const int64_t n = (int64_t)len.size();
-  int64_t stored = 0, nnz = 0;
-  for (int64_t s0 = 0; s0 < n; s0 += C) {
-    int32_t w = 0;
-    for (int64_t k = s0; k < std::min<int64_t>(n, s0 + C); ++k) {
-      const int32_t v = len[order ? (*order)[k] : k];
-      w = std::max(w, v);
-      nnz += v;
-    }
-    stored += (int64_t)w * C;
-  }
-  return nnz ? (double)stored / (double)nnz : 1.0;
-}
-
-// key: A's row length first, then R_{l-1}'s and P_l's (their rows are this level's rows too), so that one permutation
-// serves the three operators as far as their lengths correlate
-void plan_renumbering(const PartLevel& pl, const PartLevel* finer, int C, int window, Renumbering& rn) {
-  rn = Renumbering();
-  const int64_t n = pl.n_own;
-  const LocalCsr& A = pl.blk[PAMG_A_OO];
-  if (A.ptr.empty() || n < 4 * C) return;
-  std::vector<int32_t> lenA(n), order(n);
-  std::vector<int64_t> key(n);
-  for (int64_t i = 0; i < n; ++i) {
-    lenA[i] = (int32_t)(A.ptr[i + 1] - A.ptr[i]);
-    int64_t lr = 0, lp = 0;
-    if (finer && !finer->blk[PAMG_R_OO].ptr.empty()) lr = finer->blk[PAMG_R_OO].ptr[i + 1] - finer->blk[PAMG_R_OO].ptr[i];
-    if (!pl.blk[PAMG_P_OO].ptr.empty()) lp = pl.blk[PAMG_P_OO].ptr[i + 1] - pl.blk[PAMG_P_OO].ptr[i];
-    key[i] = ((int64_t)lenA[i] << 24) | (std::min<int64_t>(lr, 4095) << 12) | std::min<int64_t>(lp, 4095);
-    order[i] = (int32_t)i;
-  }
-  const double fill0 = sell_fill_of(lenA, nullptr, C);
-  if (fill0 <= 1.03) return;
-  for (int64_t w0 = 0; w0 < n; w0 += window)
-    std::stable_sort(order.begin() + w0, order.begin() + std::min<int64_t>(n, w0 + window),
-                     [&](int32_t a, int32_t b) { return key[a] > key[b]; });
-  if (sell_fill_of(lenA, &order, C) > fill0 - 0.02) return;
-  rn.old_of_new = order;
-  rn.new_of_old.resize(n);
-  for (int64_t k = 0; k < n; ++k) rn.new_of_old[order[k]] = (int32_t)k;
-}
-
-// rows of m in the order `rows.old_of_new`, own columns relabelled through `cols.new_of_old`; entry order inside a row kept
-LocalCsr renumbered_block(const LocalCsr& m, const Renumbering* rows, const Renumbering* cols) {
-  if (m.ptr.empty()) return m;
-  const bool pr = rows && rows->active(), pc = cols && cols->active();
-  LocalCsr out;
-  out.nrows = m.nrows;
-  out.ncols = m.ncols;
-  out.ptr.assign(m.nrows + 1, 0);
-  for (int64_t k = 0; k < m.nrows; ++k) {
-    const int64_t i = pr ? rows->old_of_new[k] : k;
-    out.ptr[k + 1] = out.ptr[k] + (m.ptr[i + 1] - m.ptr[i]);
-  }
-  out.col.resize(m.col.size());
-  out.val.resize(m.val.size());
-#pragma omp parallel for schedule(static)
-  for (int64_t k = 0; k < m.nrows; ++k) {
-    const int64_t i = pr ? rows->old_of_new[k] : k;
-    int64_t q = out.ptr[k];
-    for (int64_t e = m.ptr[i]; e < m.ptr[i + 1]; ++e, ++q) {
-      out.col[q] = pc ? cols->new_of_old[m.col[e]] : m.col[e];
-      out.val[q] = m.val[e];
-    }
-  }
-  return out;
-}
-
 // byte offsets inside a part's peer-visible arena; computable by every process for every part
 struct ArenaLayout {
   std::vector<size_t> ghost, flags, asm_stage, asm_flags;
@@ -552,9 +468,6 @@ struct PartDev {
   int gm_restart = 0;
   bool gm_precond = false;
   DBuf<unsigned long long> trace;
-  std::vector<Renumbering> renum;  // per level: device numbering of the own rows (identity on level 0)
-  DBuf<TailOp> tail_ops;           // phases of the fused replicated tail (k_tail_fused), empty: multi-launch tail
-  int n_tail_ops = 0;
   int hist_cap = 0;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
 };
@@ -577,15 +490,8 @@ struct Engine::Impl {
   int bnd_first = -1;       // block ids of a fused launch: 1 [pack | boundary | main], 0 [pack | main | boundary], -1 by size
   bool persistent = true;   // SELL / CSR-stream main roles run as one resident wave (env PAMG_PERSISTENT=0: one CTA per work item)
   bool fused_halo = false;  // every local part has a GPU of its own: halo roles run inside the consuming kernel
-  bool alone = false;       // every local part has a GPU of its own (a kernel may wait for its peers)
-  bool fused_tail = false;  // replicated tail as ONE persistent kernel (env PAMG_FUSED_TAIL=1; measured slower than one launch per operation)
-  int tail_ctas = 2 * 148;  // its grid (env PAMG_TAIL_CTAS), capped by the occupancy limit: all CTAs must be resident
-  std::vector<std::vector<TailOp>>* tail_rec = nullptr;  // != nullptr: enqueue_* record tail phases instead of launching
-  int unified = 0;          // fused persistent SELL launches without role CTAs: bit mask over operator classes (env PAMG_UNIFIED;
-                            // 1 A short rows, 2 A long rows, 4 P, 8 R).  Off: measured +67 us per iteration on 8 GPUs (profiles/r02)
   bool fold_check = false;  // the convergence check runs inside k_update_xr / k_pcg_init (every local part alone on its GPU)
   bool stream_long = true;  // CSR-stream blocks with long rows use 16 lanes per row in phase B (env PAMG_STREAM_LONG=0: one thread per row)
-  int unified_mode = 1;     // 1: every CTA packs + boundary own/ghost split; 2 ("lite", env PAMG_UNIFIED_MODE): pack CTAs + boundary role behind the slices
   int sell_pf = 0;          // persistent SELL launches with an L2 prefetch two slices ahead: bit mask 1 P, 2 long-row A, 4 R (env PAMG_SELL_PF)
   int vi_occ = 2;           // one-byte value-indexed kernel, persistent launches (short rows): 2 = U = 2 at 64 registers / 4 CTAs per SM (shipped:
                             // 256^3 solve 33.7 -> 31.4 ms, SpMV 0.163 -> 0.144 ms), 0 = U = 4 at 80 registers / 3 CTAs, 1 = U = 4 squeezed into 64
@@ -760,15 +666,12 @@ void launch_stream(int mode, bool dot, bool long_rows, StreamView A, const Launc
 
 // short_variant (operators whose rows have at most 8 entries, i.e. the prolongators; M_ADD only): 0 = the A kernel,
 // 1 = <RPT 2, U 2, 5 CTAs/SM>, 2 = <RPT 1, U 4, 6 CTAs/SM> (needs the C = 32 layout).
-// try_unified: fused launch of one part per GPU -- run without role CTAs when every CTA's share of the boundary rows fits
-// (kernels.cuh "Unified CTA roles"); *was_unified reports the decision.
-void launch_sell(int mode, bool dot, int rpt, int short_variant, bool prefetch, SellView A, LaunchArgs L, bool try_unified,
-                 int unified_mode, bool* was_unified, const SellViView* vi = nullptr, int vi_variant = 0, int vi_occ = 0) {
+void launch_sell(int mode, bool dot, int rpt, int short_variant, bool prefetch, SellView A, const LaunchArgs& L,
+                 const SellViView* vi = nullptr, int vi_variant = 0, int vi_occ = 0) {
   dispatch_mode(mode, dot, [&](auto md, auto dt) {
     constexpr int MD = decltype(md)::value;
     constexpr bool DT = decltype(dt)::value;
-    if (vi && rpt == 2 && !try_unified) {  // value-indexed operator: its own kernel (the experimental variants below do not apply)
-      *was_unified = false;
+    if (vi && rpt == 2) {  // value-indexed operator: its own kernel (the experimental variants below do not apply)
       using KernVi = void (*)(SellViView, const double*, EpiArgs, DevState*, FusedHalo, double*, RedCtx, int, int);
       KernVi kv = vi_variant == 5 && vi_occ == 1 ? (KernVi)k_spmv_sell_vi4<MD, DT, 1, 4, 4, 1>   // 64 registers (spills), 4 CTAs/SM
                   : vi_variant == 5 && vi_occ == 2 ? (KernVi)k_spmv_sell_vi4<MD, DT, 1, 2, 4, 1> // U = 2, 64 registers, 4 CTAs/SM
@@ -792,32 +695,7 @@ void launch_sell(int mode, bool dot, int rpt, int short_variant, bool prefetch, 
     if constexpr (!DT) {  // L2 prefetch of the slice two iterations ahead (persistent launches of the latency-bound operators)
       if (prefetch && rpt == 2 && short_variant == 0) k = (Kern)k_spmv_sell<2, MD, false, 4, 3, 2>;
     }
-    int grid = 0;
-    *was_unified = false;
-    if (try_unified && rpt == 2 && unified_mode == 2) {  // "lite": pack CTAs + work CTAs that finish with the boundary role
-      k = (Kern)k_spmv_sell_uni<MD, DT>;
-      const int n_work = std::max(1, std::min(L.grid, std::min(resident_ctas((const void*)k), RED_GRID)));
-      L.fh.unified = 2;
-      if (L.fh.n_bnd > 0) L.fh.n_bnd = n_work;
-      grid = L.fh.n_pack + n_work;
-      *was_unified = true;
-    } else if (try_unified && rpt == 2) {
-      k = (Kern)k_spmv_sell_uni<MD, DT>;
-      const int n_work = std::max(1, std::min(L.grid, std::min(resident_ctas((const void*)k), RED_GRID)));
-      const int share = (L.fh.B.n + n_work - 1) / n_work;
-      if (share > BLOCK) {  // too many boundary rows for one resident wave: role CTAs
-        k = (Kern)k_spmv_sell<2, MD, DT>;
-      } else {
-        L.fh.unified = 1;
-        L.fh.bnd_share = std::max(share, 1);
-        if (L.fh.n_pack > 0) L.fh.n_pack = n_work;
-        if (L.fh.n_bnd > 0) L.fh.n_bnd = n_work;
-        grid = n_work;
-        *was_unified = true;
-      }
-    }
-    if (!grid) grid = main_grid(L, (const void*)k);
-    k<<<grid, BLOCK, 0, L.s>>>(A, L.x, L.a, L.st, L.fh, L.partials, L.rc, L.publish, L.slot);
+    k<<<main_grid(L, (const void*)k), BLOCK, 0, L.s>>>(A, L.x, L.a, L.st, L.fh, L.partials, L.rc, L.publish, L.slot);
   });
 }
 
@@ -842,8 +720,6 @@ void launch_boundary(int mode, bool dot, const LaunchArgs& L) {
 // One SpMV-family operation over all local parts: consistent!(xin) + own rows of the operator.
 // which: PAMG_A_OO / PAMG_P_OO / PAMG_R_OO (the matching *_OG is implied).
 // row_level: level whose LevelDev holds the blocks; halo_level: level of the column partition.
-struct TailRecordAbort {};  // an operation of the tail has no phase form (format, smoother): keep the multi-launch tail
-
 struct OpSpec {
   int row_level, which, halo_level, mode;
   bool dot = false;
@@ -865,20 +741,6 @@ void Engine::enqueue_op(const OpSpec& op, const std::vector<const double*>& xin,
   const bool exchange = need && !op.coarse_ghosts_local;
   const bool fused = I.fused_halo;
   const int wsel = op.which / 2;  // 0 A, 1 P, 2 R
-  if (I.tail_rec) {  // recording the phases of the fused tail kernel: merged levels, CSR-stream blocks, no halo, no dot
-    for (size_t i = 0; i < I.parts.size(); ++i) {
-      const DevCsr& m = I.LV(i, l).blk[op.which];
-      if (!I.tail_mode || !m.stream || op.dot) throw TailRecordAbort();
-      TailOp t{};
-      t.kind = T_STREAM;
-      t.mode = op.mode;
-      t.A = m.sview();
-      t.x = xin[i];
-      t.a = epi[i];
-      (*I.tail_rec)[i].push_back(t);
-    }
-    return;
-  }
 
   auto halo_args = [&](PartDev& pd, bool with_pack, bool with_bnd) {
     LevelDev& ld = I.LV(pd, l);
@@ -915,14 +777,11 @@ void Engine::enqueue_op(const OpSpec& op, const std::vector<const double*>& xin,
     // B200 (256^3): SELL Jacobi sweep 0.316 ms persistent vs 0.344 ms with one CTA per 8 slices.
     // Long rows (level >= 1, 30+ entries per row) lose 10 % that way: they keep one CTA per 8 slices.
     const double mean_nnz = m.nrows ? (double)m.nnz / m.nrows : 0.0;
-    // PAMG_UNIFIED bit mask: 1 = A with short rows, 2 = A with long rows, 4 = P, 8 = R
-    const int uni_bit = op.which == PAMG_P_OO ? 4 : op.which == PAMG_R_OO ? 8 : (mean_nnz <= 12.0 ? 1 : 2);
-    const bool try_unified = fused && (I.unified & uni_bit) && m.sell_rpt && !m.sell_diag && (fh.n_pack > 0 || fh.n_bnd > 0);
     // PAMG_SELL_PF bit mask: 1 = P, 2 = A with long rows, 4 = R (these then run persistent, which the prefetch needs)
     const int pf_bit = op.which == PAMG_P_OO ? 1 : op.which == PAMG_R_OO ? 4 : (mean_nnz > 12.0 ? 2 : 0);
-    const bool prefetch = I.persistent && m.sell_rpt == 2 && (I.sell_pf & pf_bit) && !op.dot && !try_unified;
-    const bool vi4_here = m.sell_vi4 && I.vi_variant == 3 && !try_unified;
-    const bool bounded = I.persistent && m.sell_rpt && (mean_nnz <= 12.0 || try_unified || prefetch || (vi4_here && I.vi_persist_long));
+    const bool prefetch = I.persistent && m.sell_rpt == 2 && (I.sell_pf & pf_bit) && !op.dot;
+    const bool use_vi4 = m.sell_vi4 && I.vi_variant == 3;
+    const bool bounded = I.persistent && m.sell_rpt && (mean_nnz <= 12.0 || prefetch || (use_vi4 && I.vi_persist_long));
     LaunchArgs L{0, bounded || op.dot, pd.stream, xin[i], epi[i], pd.st.p, fh, pd.partials.p, pd.rc, publish, op.slot};
     L.fh.v = xin[i];
     int n_main;
@@ -934,9 +793,7 @@ void Engine::enqueue_op(const OpSpec& op, const std::vector<const double*>& xin,
       n_main = I.grid_for(m.nrows, (BLOCK / m.lanes) * 4);
     }
     L.grid = std::max(n_main, 1);
-    bool was_unified = false;
     SellViView viv{};
-    const bool use_vi4 = m.sell_vi4 && I.vi_variant == 3 && !try_unified;
     if (m.sell_vi || use_vi4) viv = use_vi4 ? m.vi4view() : m.viview();
     if (use_vi4 || m.sell_diag) L.grid = std::max((m.nslices4 + BLOCK / 32 - 1) / (BLOCK / 32), 1);
     const bool long_rows = I.stream_long && mean_nnz >= 48.0 && !op.dot;  // CSR-stream phase B with 16 lanes per row (no DOT form)
@@ -944,7 +801,7 @@ void Engine::enqueue_op(const OpSpec& op, const std::vector<const double*>& xin,
       launch_sell_diag(op.mode, op.dot, m.diagview(), L);
     else if (m.sell_rpt)
       launch_sell(op.mode, op.dot, m.sell_rpt, (op.which == PAMG_P_OO && m.short_rows) ? I.p_kernel : 0, prefetch, m.slview(), L,
-                  try_unified, I.unified_mode, &was_unified, (m.sell_vi || use_vi4) ? &viv : nullptr,
+                  (m.sell_vi || use_vi4) ? &viv : nullptr,
                   use_vi4 ? (m.vi4_ib == 2 ? 4 : 3) + (I.vi_ahead && L.bounded ? 2 : 0) : (I.vi_variant == 3 ? 0 : I.vi_variant), I.vi_occ);  // blocks without the 128-row layout (sorted rows): two rows per lane
     else if (m.stream)
       launch_stream(op.mode, op.dot, long_rows, m.sview(), L);
@@ -956,9 +813,9 @@ void Engine::enqueue_op(const OpSpec& op, const std::vector<const double*>& xin,
       // the name says which kernel ran: sell-vi = four rows per lane (one-byte indices), sell-vi16 = the same with two-byte
       // indices, sell-vi2 = two rows per lane (sorted rows), stream-long = CSR-stream with 16 lanes per row in phase B
       const char* vi_name = use_vi4 ? (m.vi4_ib == 2 ? "sell-vi16 " : "sell-vi ") : "sell-vi2 ";
-      I.names.push_back(std::string(m.sell_diag ? "sell-diag " : m.sell_rpt ? ((m.sell_vi || use_vi4) && !was_unified ? vi_name : "sell ") : m.stream ? (long_rows ? "stream-long " : "stream ") : "csr ") + MODES[op.mode] + (op.dot ? "+dot " : " ") +
+      I.names.push_back(std::string(m.sell_diag ? "sell-diag " : m.sell_rpt ? ((m.sell_vi || use_vi4) ? vi_name : "sell ") : m.stream ? (long_rows ? "stream-long " : "stream ") : "csr ") + MODES[op.mode] + (op.dot ? "+dot " : " ") +
                         OPS[wsel] + std::to_string(l) + (I.tail_mode ? " tail" : "") + (fh.n_pack ? " +pack" : "") +
-                        (fh.n_bnd ? " +bnd" : "") + (was_unified ? " uni" : ""));
+                        (fh.n_bnd ? " +bnd" : ""));
       I.naming = false;
       I.note_launch();
       I.naming = true;
@@ -1114,61 +971,33 @@ Engine::Engine(Hierarchy* h, int nlocal, const int32_t* local_parts, const int32
     pd.scratch4.alloc(RED_W);
     int max_blocks = Impl::MAX_GRID;
 
-    // device numbering of the own rows of the levels >= 1 that will run in SELL (see "upload-time renumbering" above)
-    pd.renum.assign(I.L, Renumbering());
-    {
-      const char* re = getenv("PAMG_RENUMBER");
-      const char* we = getenv("PAMG_RENUMBER_WINDOW");
-      const int window = we ? std::max(64, atoi(we)) : 4096;
-      if (re && atoi(re) != 0)  // off by default: measured a net loss at 256^3 (profiles/r02_kernel_sweep.md)
-        for (int l = 1; l < I.L; ++l) {
-          const PartLevel& pl = h->levels[l].parts[part];
-          const bool sell = o.spmv_format == PAMG_FORMAT_SELL || o.spmv_format == PAMG_FORMAT_SELL_DIAG || (o.spmv_format == PAMG_FORMAT_AUTO && pl.n_own >= SELL_AUTO_MIN_ROWS_A);
-          if (sell) plan_renumbering(pl, &h->levels[l - 1].parts[part], 64, window, pd.renum[l]);
-        }
-    }
-
     for (int l = 0; l < I.L; ++l) {
       const PartLevel& pl = h->levels[l].parts[part];
       pd.lev.emplace_back(new LevelDev);
       LevelDev& ld = *pd.lev.back();
       ld.n_own = pl.n_own;
       ld.n_ghost = pl.n_ghost;
-      const Renumbering& rn = pd.renum[l];
-      const Renumbering* rnc = l + 1 < I.L ? &pd.renum[l + 1] : nullptr;  // numbering of the next coarser level
       for (int b = 0; b < 6; b += 2) {
         int lanes = 0;
         if (b == PAMG_A_OO && o.lanes_per_row > 0) lanes = o.lanes_per_row;
-        // row / own-column numbering of this block: A (l, l), P (l, l+1), R (l+1, l); ghost columns are staging slots
-        const Renumbering* rows = b == PAMG_R_OO ? rnc : &rn;
-        const Renumbering* cols = b == PAMG_P_OO ? rnc : &rn;
-        const bool moved = (rows && rows->active()) || (cols && cols->active());
-        LocalCsr t_oo, t_og;
-        if (moved) {
-          t_oo = renumbered_block(pl.blk[b], rows, cols);
-          t_og = renumbered_block(pl.blk[b + 1], rows, nullptr);
-        }
-        const LocalCsr& oo = moved ? t_oo : pl.blk[b];
-        const LocalCsr& og = moved ? t_og : pl.blk[b + 1];
-        build_csr(oo, false, ld.blk[b], lanes, o.spmv_format, o, b, b == PAMG_P_OO && I.p_kernel == 2 ? 1 : 0);
-        build_bnd(oo, og, ld.bnd[b / 2]);
+        build_csr(pl.blk[b], false, ld.blk[b], lanes, o.spmv_format, o, b, b == PAMG_P_OO && I.p_kernel == 2 ? 1 : 0);
+        build_bnd(pl.blk[b], pl.blk[b + 1], ld.bnd[b / 2]);
         max_blocks = std::max(max_blocks, ld.blk[b].nblocks);
         max_blocks = std::max(max_blocks, (std::max(ld.blk[b].nslices, ld.blk[b].nslices4) + BLOCK / 32 - 1) / (BLOCK / 32));
       }
-      // smoother weights (device numbering)
+      // smoother weights
       std::vector<double> w(pl.n_own), dinv(pl.n_own);
       const double rho = h->levels[l].rho;
       const double lmax = o.cheb_hi_frac * rho, lmin = o.cheb_lo_frac * rho;
       const double theta = 0.5 * (lmax + lmin);
-      for (int64_t kn = 0; kn < pl.n_own; ++kn) {
-        const int64_t k = rn.active() ? rn.old_of_new[kn] : kn;
-        dinv[kn] = 1.0 / pl.diag[k];
+      for (int64_t k = 0; k < pl.n_own; ++k) {
+        dinv[k] = 1.0 / pl.diag[k];
         if (o.smoother == PAMG_SMOOTHER_L1JACOBI)
-          w[kn] = 1.0 / pl.diag_l1[k];
+          w[k] = 1.0 / pl.diag_l1[k];
         else if (o.smoother == PAMG_SMOOTHER_CHEBYSHEV)
-          w[kn] = (1.0 / theta) / pl.diag[k];
+          w[k] = (1.0 / theta) / pl.diag[k];
         else
-          w[kn] = o.omega_jacobi / pl.diag[k];
+          w[k] = o.omega_jacobi / pl.diag[k];
       }
       ld.w.upload(w);
       ld.dinv.upload(dinv);
@@ -1180,13 +1009,7 @@ Engine::Engine(Hierarchy* h, int nlocal, const int32_t* local_parts, const int32
         ld.d.alloc(pl.n_own);
         ld.d2.alloc(pl.n_own);
       }
-      if (rn.active()) {  // the halo pack gathers from device vectors
-        std::vector<int32_t> si(pl.send_idx.size());
-        for (size_t k = 0; k < si.size(); ++k) si[k] = rn.new_of_old[pl.send_idx[k]];
-        ld.send_idx.upload(si);
-      } else {
-        ld.send_idx.upload(pl.send_idx);
-      }
+      ld.send_idx.upload(pl.send_idx);
       ld.n_send = (int)pl.send_idx.size();
       ld.n_send_nbrs = (int)pl.send.size();
       ld.n_recv_nbrs = (int)pl.recv.size();
@@ -1196,7 +1019,7 @@ Engine::Engine(Hierarchy* h, int nlocal, const int32_t* local_parts, const int32
       ld.hr.n_nbrs = ld.n_recv_nbrs;
       // assemble! gather plan: for every own row that some neighbour holds as a ghost, the staging
       // positions that contribute to it (ascending neighbour part, ascending slot).  It works on the caller's
-      // local vector (io_local), i.e. in the ORIGINAL numbering.
+      // local vector (io_local).
       {
         std::vector<std::vector<int32_t>> contrib(pl.n_own);
         for (size_t k = 0; k < pl.send_idx.size(); ++k) contrib[pl.send_idx[k]].push_back((int32_t)k);
@@ -1246,13 +1069,7 @@ Engine::Engine(Hierarchy* h, int nlocal, const int32_t* local_parts, const int32
       }
     const PartLevel& pc = h->levels[I.tail_level].parts[part];
     pd.inv.upload(h->coarse_inv);
-    {
-      const Renumbering& rt = pd.renum[I.tail_level];
-      std::vector<int64_t> og(pc.own_to_global);
-      if (rt.active())
-        for (size_t k = 0; k < og.size(); ++k) og[k] = pc.own_to_global[rt.old_of_new[k]];
-      pd.own_gid_T.upload(og);
-    }
+    pd.own_gid_T.upload(pc.own_to_global);
     pd.ghost_gid_T.upload(pc.ghost_to_global);
     // PCG vectors on level 0
     const int64_t n0 = h->levels[0].parts[part].n_own;
@@ -1292,13 +1109,8 @@ Engine::Engine(Hierarchy* h, int nlocal, const int32_t* local_parts, const int32
       throw CommError("halo plan: a part's send-neighbour set differs from its receive-neighbour set (structurally non-symmetric "
                       "operator); the peer-memory exchange protocol needs symmetric neighbour sets on multi-GPU layouts");
     if (const char* pe = getenv("PAMG_PERSISTENT")) I.persistent = atoi(pe) != 0;
-    if (const char* ue = getenv("PAMG_UNIFIED")) I.unified = atoi(ue);
-    if (const char* ue = getenv("PAMG_UNIFIED_MODE")) I.unified_mode = atoi(ue) == 2 ? 2 : 1;
-    if (const char* te = getenv("PAMG_FUSED_TAIL")) I.fused_tail = atoi(te) != 0;
     if (const char* le = getenv("PAMG_STREAM_LONG")) I.stream_long = atoi(le) != 0;
     if (const char* pe2 = getenv("PAMG_SELL_PF")) I.sell_pf = atoi(pe2);
-    if (const char* te = getenv("PAMG_TAIL_CTAS")) I.tail_ctas = std::max(1, atoi(te));
-    I.alone = alone;
     {
       const char* fe = getenv("PAMG_FOLD_CHECK");
       I.fold_check = alone && (!fe || atoi(fe) != 0);
@@ -1308,42 +1120,10 @@ Engine::Engine(Hierarchy* h, int nlocal, const int32_t* local_parts, const int32
     const bool want = env ? atoi(env) != 0 : o.fuse_halo != 0;
     I.fused_halo = want && alone && symmetric;
   }
-  build_tail_programs();
   if (nlocal == I.nparts) connect();
 }
 
 Engine::~Engine() { delete impl; }
-
-// The replicated tail as a list of phases for k_tail_fused: the V-cycle schedule of the merged levels is RECORDED by
-// running the ordinary enqueue code with Impl::tail_rec set, so the phase list follows nu_pre / nu_post / smoother /
-// buffer plan exactly as the multi-launch tail does.
-void Engine::build_tail_programs() {
-  Impl& I = *impl;
-  for (auto& up : I.parts) up->n_tail_ops = 0;
-  if (!I.fused_tail || I.tail_level >= I.L - 1 || I.h->opts.cycle != PAMG_CYCLE_V) return;
-  std::vector<std::vector<TailOp>> rec(I.parts.size());
-  I.tail_rec = &rec;
-  I.tail_mode = true;
-  bool ok = true;
-  try {
-    enqueue_vcycle(I.tail_level, false, true);
-  } catch (const TailRecordAbort&) {
-    ok = false;
-  } catch (...) {
-    I.tail_mode = false;
-    I.tail_rec = nullptr;
-    throw;
-  }
-  I.tail_mode = false;
-  I.tail_rec = nullptr;
-  if (!ok) return;
-  for (size_t i = 0; i < I.parts.size(); ++i) {
-    PartDev& pd = I.P(i);
-    I.set_dev(pd);
-    pd.tail_ops.upload(rec[i]);
-    pd.n_tail_ops = (int)rec[i].size();
-  }
-}
 
 // decide, per level, which buffer receives the zero-guess first sweep so that the V-cycle result
 // always ends in LevelDev::x whatever nu_pre / nu_post / Chebyshev degree are
@@ -1502,33 +1282,15 @@ void Engine::upload_vec(int level, const double* const* host, int which_buf) {
     PartDev& pd = *up;
     I.set_dev(pd);
     if (!host[pd.part]) throw std::runtime_error("null vector pointer for a local part");
-    const Renumbering& rn = pd.renum[level];
-    if (rn.active()) {  // host vectors are in the partition's numbering, device vectors of this level in the renumbered one
-      const int64_t n = pd.lev[level]->n_own;
-      std::vector<double> tmp(n);
-      for (int64_t k = 0; k < n; ++k) tmp[k] = host[pd.part][rn.old_of_new[k]];
-      CK(cudaMemcpyAsync(vec(pd, level, which_buf), tmp.data(), n * sizeof(double), cudaMemcpyHostToDevice, pd.stream));
-      CK(cudaStreamSynchronize(pd.stream));  // tmp goes out of scope
-      continue;
-    }
     CK(cudaMemcpyAsync(vec(pd, level, which_buf), host[pd.part], pd.lev[level]->n_own * sizeof(double), cudaMemcpyHostToDevice,
                        pd.stream));
   }
 }
 
-// device vector `src` of `level` (own length) -> host array in the partition's numbering; synchronous for renumbered levels
+// device vector `src` of `level` (own length) -> host array (asynchronous on the part's stream)
 void Engine::download_own(PartDev& pd, int level, const double* src, double* host) {
-  const Renumbering& rn = pd.renum[level];
-  const int64_t n = pd.lev[level]->n_own;
   impl->set_dev(pd);
-  if (!rn.active()) {
-    CK(cudaMemcpyAsync(host, src, n * sizeof(double), cudaMemcpyDeviceToHost, pd.stream));
-    return;
-  }
-  std::vector<double> tmp(n);
-  CK(cudaMemcpyAsync(tmp.data(), src, n * sizeof(double), cudaMemcpyDeviceToHost, pd.stream));
-  CK(cudaStreamSynchronize(pd.stream));
-  for (int64_t k = 0; k < n; ++k) host[rn.old_of_new[k]] = tmp[k];
+  CK(cudaMemcpyAsync(host, src, pd.lev[level]->n_own * sizeof(double), cudaMemcpyDeviceToHost, pd.stream));
 }
 
 void Engine::download_vec(int level, double* const* host, int which_buf) {
@@ -1687,55 +1449,13 @@ void Engine::enqueue_tail(bool zero_guess) {
     CK(cudaGetLastError());
     return;
   }
-  bool fused_tail = l < I.L - 1;
-  for (auto& up : I.parts) fused_tail = fused_tail && up->n_tail_ops > 0;
-  const bool fold_gather = fused_tail && I.alone;  // the all-gather is phase 0 of the fused kernel
-  if (!fold_gather)
-    for (auto& up : I.parts) {
-      PartDev& pd = *up;
-      LevelDev& ld = *pd.lev[l];
-      I.set_dev(pd);
-      k_coarse_gather<<<I.grid_for(ld.n_own, BLOCK), BLOCK, 0, pd.stream>>>(ld.b.p, pd.own_gid_T.p, (int)ld.n_own, pd.coarse_pubs.p,
-                                                                           I.nparts, pd.st.p);
-      I.note_launch("k_coarse_gather");
-    }
-  if (fused_tail) {
-    for (auto& up : I.parts) {
-      PartDev& pd = *up;
-      LevelDev& ld = *pd.lev[l];
-      LevelDev& tl = *pd.tlev[l];
-      I.set_dev(pd);
-      TailIO io{};
-      io.g0 = (const double*)(pd.arena + pd.lay.coarse);
-      io.g1 = io.g0 + n;
-      io.flags = (const uint32_t*)(pd.arena + pd.lay.coarse_flags);
-      io.pubs = pd.coarse_pubs.p;
-      io.b_own = ld.b.p;
-      io.own_gid = pd.own_gid_T.p;
-      io.ghost_gid = pd.ghost_gid_T.p;
-      io.nparts = I.nparts;
-      io.n_own = (int32_t)ld.n_own;
-      io.n_ghost = (int32_t)ld.n_ghost;
-      io.n = n;
-      io.b_full = tl.b.p;
-      io.xstart = tl.xstart;
-      io.w = o.nu_pre > 0 ? tl.w.p : nullptr;
-      io.x_full = tl.x.p;
-      io.x_own = ld.x.p;
-      io.xg = (double*)ld.hr.ghost[0];
-      io.inv = pd.inv.p;
-      io.do_gather = fold_gather ? 1 : 0;
-      const int grid = std::max(1, std::min(I.tail_ctas, resident_ctas((const void*)k_tail_fused)));
-      // cooperative launch: the grid barrier needs every CTA resident, and the runtime refuses the launch otherwise
-      const TailOp* ops_arg = pd.tail_ops.p;
-      int n_ops_arg = pd.n_tail_ops;
-      DevState* st_arg = pd.st.p;
-      void* args[] = {(void*)&ops_arg, (void*)&n_ops_arg, (void*)&io, (void*)&st_arg};
-      CK(cudaLaunchCooperativeKernel((const void*)k_tail_fused, dim3(grid), dim3(BLOCK), args, 0, pd.stream));
-      I.note_launch(fold_gather ? "k_tail_fused (gather + tail V-cycle + scatter)" : "k_tail_fused (tail V-cycle + scatter)");
-    }
-    CK(cudaGetLastError());
-    return;
+  for (auto& up : I.parts) {
+    PartDev& pd = *up;
+    LevelDev& ld = *pd.lev[l];
+    I.set_dev(pd);
+    k_coarse_gather<<<I.grid_for(ld.n_own, BLOCK), BLOCK, 0, pd.stream>>>(ld.b.p, pd.own_gid_T.p, (int)ld.n_own, pd.coarse_pubs.p,
+                                                                         I.nparts, pd.st.p);
+    I.note_launch("k_coarse_gather");
   }
   if (l == I.L - 1) {
     for (auto& up : I.parts) {
@@ -1794,18 +1514,6 @@ void Engine::enqueue_vcycle(int l, bool dot_rz, bool zero_guess) {
     return;
   }
   if (I.tail_mode && l == I.L - 1) {  // coarsest level of the replicated tail: x = A_L^-1 b, whole vector
-    if (I.tail_rec) {
-      for (size_t i = 0; i < np; ++i) {
-        LevelDev& ld = I.LV(i, l);
-        TailOp t{};
-        t.kind = T_DENSE;
-        t.x = ld.b.p;
-        t.a.out = ld.x.p;
-        t.n = (int32_t)ld.n_own;
-        (*I.tail_rec)[i].push_back(t);
-      }
-      return;
-    }
     for (auto& up : I.parts) {
       PartDev& pd = *up;
       LevelDev& ld = I.LV(pd, l);
@@ -1854,15 +1562,6 @@ void Engine::enqueue_vcycle(int l, bool dot_rz, bool zero_guess) {
       for (size_t i = 0; i < np; ++i) {
         PartDev& pd = I.P(i);
         LevelDev& lc = I.LV(pd, l + 1);
-        if (I.tail_rec) {
-          TailOp t{};
-          t.kind = T_SCALE;
-          t.x = lc.b.p;
-          t.a.out = lc.xstart;
-          t.n = (int32_t)lc.n_own;
-          (*I.tail_rec)[i].push_back(t);
-          continue;
-        }
         I.set_dev(pd);
         k_scale<<<I.grid_for(lc.n_own, BLOCK * 4), BLOCK, 0, pd.stream>>>(lc.b.p, nullptr, lc.xstart, (int)lc.n_own, pd.st.p);
         I.note_launch("k_scale");

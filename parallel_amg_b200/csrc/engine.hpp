@@ -64,7 +64,6 @@ class Engine {
   Impl* impl;
 
   void plan_buffers();
-  void build_tail_programs();
   void require_connected();
   void sync_all();
   void upload_vec(int level, const double* const* host, int which_buf);

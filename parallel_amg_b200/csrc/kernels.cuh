@@ -71,7 +71,6 @@ struct DevState {
   uint32_t pack_done[MAX_LEVELS];  // fused launches: epoch whose pack role has finished
   uint32_t asm_epoch[MAX_LEVELS];
   uint32_t ticket[8];
-  uint32_t bar_count, bar_gen;  // grid barrier of the fused tail kernel (all its CTAs are resident)
   int32_t done;
   int32_t iters;
   int32_t error;
@@ -131,10 +130,6 @@ struct FusedHalo {
   int32_t fixed_parity;     // >= 0: ghost values are already in staging[parity], no wait (coarsest level)
   int32_t fused;            // 1: roles inside one launch (boundary role advances the epoch)
   int32_t bnd_first;        // 1: block ids [pack | boundary | main]; 0: [pack | main | boundary]
-  int32_t unified;          // 1 (SELL, fused, persistent): no role CTAs -- EVERY CTA packs a share, does a share of the
-                            // boundary rows and its static share of the slices (n_pack, n_bnd = 0 or gridDim.x); bnd_share =
-                            // boundary rows per CTA (<= BLOCK)
-  int32_t bnd_share;
   int32_t n_send, n_nbrs;   // pack role
   const double* v;
   const int32_t* send_idx;
@@ -573,98 +568,6 @@ struct StreamView {
 // variants with a fused dot product, which run RED_GRID CTAs that stride over the row blocks: a
 // gpu-scope fence per CTA (needed by the last-block reduction) invalidates the SM's L1, so it must
 // not happen once per row block (ncu r01: +45 % time with 65536 fencing CTAs).
-// One row block `bk` of the CSR-stream family as a device function, for the fused tail kernel (k_tail_fused).  It restates
-// the loop body of k_spmv_stream below statement by statement (same products, same summation order: identical bits); the
-// kernel keeps its own inline copy because routing it through this function changed ptxas' register allocation (more
-// spills in three instantiations).  prod = the CTA's product buffer.  CS: the matrix entries are read once
-// (evict-first); the fused tail kernel reads them with the default policy so that the second pass of a V-cycle over a
-// tail matrix hits L2.  `more`: another row block follows in this CTA (prod is reused).
-template <int MODE, bool DOT, bool CS>
-__device__ __forceinline__ void stream_row_block(const StreamView& A, const double* x, const EpiArgs& a, const uint8_t* skip, int bk,
-                                                 double* prod, double& acc, bool more) {
-  const int t = threadIdx.x;
-  const int2 b0 = A.blk[bk], b1 = A.blk[bk + 1];
-  const int r0 = b0.x, nr = b1.x - b0.x;
-  const int ea = b0.y & ~3;              // 4-entry aligned start: 16 B (col) / 32 B (val) aligned
-  const int n4 = (b1.y - ea + 3) >> 2;   // 4-entry groups to stream (<= S_STEPS * BLOCK by construction)
-  // prefetch row extents and the first chunk's epilogue operands; their latency overlaps phase A
-  int pb = 0, pe = 0;
-  unsigned char sk = 0;
-  double e_in0 = 0.0, e_in1 = 0.0, e_w = 0.0, e_aux = 0.0, e_dot = 0.0;
-  if (t < nr) {
-    const int row = r0 + t;
-    pb = A.ptr[row] - ea;
-    pe = A.ptr[row + 1] - ea;
-    if (skip) sk = skip[row];
-    if (MODE == M_RESID || MODE == M_JACOBI || MODE == M_ADD || MODE == M_CHEB) e_in0 = a.in0[row];
-    if (MODE == M_JACOBI || MODE == M_CHEB) e_in1 = a.in1[row];
-    if (MODE == M_JACOBI || MODE == M_CHEB || (MODE == M_RESTRICT && a.out2)) e_w = a.w[row];
-    if (MODE == M_CHEB && a.aux) e_aux = a.aux[row];
-    if (DOT) e_dot = a.dotv[row];
-  }
-  // phase A: stream entries [ea, ea + 4 n4).  Entries outside the block's own range belong to the
-  // neighbouring blocks (or the zero padding): valid data, their products are simply never read.
-  const int4* __restrict__ col4 = reinterpret_cast<const int4*>(A.col + ea);
-  const double2* __restrict__ val2 = reinterpret_cast<const double2*>(A.val + ea);
-  int4 c[S_STEPS];
-  double2 v0[S_STEPS], v1[S_STEPS];
-#pragma unroll
-  for (int j = 0; j < S_STEPS; ++j) {
-    const int g = t + j * BLOCK;
-    if (g < n4) {
-      if (CS) {
-        c[j] = __ldcs(col4 + g);
-        v0[j] = __ldcs(val2 + 2 * g);
-        v1[j] = __ldcs(val2 + 2 * g + 1);
-      } else {
-        c[j] = col4[g];
-        v0[j] = val2[2 * g];
-        v1[j] = val2[2 * g + 1];
-      }
-    }
-  }
-#pragma unroll
-  for (int j = 0; j < S_STEPS; ++j) {
-    const int g = t + j * BLOCK;
-    if (g < n4) {
-      const double x0 = x[c[j].x], x1 = x[c[j].y], x2 = x[c[j].z], x3 = x[c[j].w];
-      double2 p0, p1;
-      p0.x = v0[j].x * x0;
-      p0.y = v0[j].y * x1;
-      p1.x = v1[j].x * x2;
-      p1.y = v1[j].y * x3;
-      reinterpret_cast<double2*>(prod)[2 * g] = p0;
-      reinterpret_cast<double2*>(prod)[2 * g + 1] = p1;
-    }
-  }
-  __syncthreads();
-  // phase B: thread t owns rows t, t + BLOCK, ...; products summed in column order
-#pragma unroll
-  for (int q = 0; q < S_CHUNKS; ++q) {
-    const int rr = t + q * BLOCK;
-    if (rr < nr) {
-      const int row = r0 + rr;
-      if (q > 0) {  // extents / operands of the later chunks (short-row matrices only) are fetched here
-        pb = A.ptr[row] - ea;
-        pe = A.ptr[row + 1] - ea;
-        if (skip) sk = skip[row];
-        if (MODE == M_RESID || MODE == M_JACOBI || MODE == M_ADD || MODE == M_CHEB) e_in0 = a.in0[row];
-        if (MODE == M_JACOBI || MODE == M_CHEB) e_in1 = a.in1[row];
-        if (MODE == M_JACOBI || MODE == M_CHEB || (MODE == M_RESTRICT && a.out2)) e_w = a.w[row];
-        if (MODE == M_CHEB && a.aux) e_aux = a.aux[row];
-        if (DOT) e_dot = a.dotv[row];
-      }
-      double s = 0.0;
-      for (int k = pb; k < pe; ++k) s += prod[k];
-      if (!sk) {
-        const double res = stream_epilogue<MODE>(a, row, s, e_in0, e_in1, e_w, e_aux);
-        if (DOT) acc += e_dot * res;
-      }
-    }
-  }
-  if (more) __syncthreads();  // prod is reused by the next row block
-}
-
 // LONG (rows of >= 48 entries on average: the restriction operators of the coarse levels, 240 entries per row at 256^3, and
 // the Galerkin matrices of the tail): a row block then holds a dozen rows, and one thread per row leaves 244 of 256 threads
 // idle through a 240-step dependent add chain (restrict R1: 68 us for 146 MB).  Phase B there gives every row S_LB lanes:
@@ -835,80 +738,6 @@ __device__ __forceinline__ double sv_get(const double& v, int) { return v; }
 __device__ __forceinline__ double sv_get(const double2& v, int k) { return k ? v.y : v.x; }
 __device__ __forceinline__ int sv_get(const int32_t& v, int) { return v; }
 __device__ __forceinline__ int sv_get(const int2& v, int k) { return k ? v.y : v.x; }
-
-// Unified CTA roles (fused launches of a persistent SELL kernel, one part per GPU).  With separate role CTAs the
-// boundary CTAs either hold resident-CTA slots while they spin (dispatched first) or only start once the persistent main
-// wave retires (dispatched last: the boundary rows are then appended to the kernel instead of hidden behind it).  Here
-// every CTA of the one resident wave
-//   1. packs a share of the halo (owner -> neighbours' staging over NVLink, fence, ticket; the last one raises the flags),
-//   2. computes the own-column sums of its share of the boundary rows and parks them in shared memory,
-//   3. streams its static share of the slices (the halo is in flight meanwhile),
-//   4. waits for the neighbours' flags (long since there), adds the ghost-column sums, applies the epilogue,
-//   5. tickets; the last CTA advances the halo epoch.
-// The row -> CTA assignment is static, so fused dot products stay reproducible bit for bit.
-template <int MODE, bool DOT>
-__device__ __forceinline__ void unified_bnd_own(const FusedHalo& fh, const double* __restrict__ x, double* s_bnd, int w) {
-  const BndView& B = fh.B;
-  const int lanes = B.lanes, lane = threadIdx.x & (lanes - 1), grp = threadIdx.x / lanes, rpb = BLOCK / lanes;
-  for (int j0 = 0; j0 < fh.bnd_share; j0 += rpb) {  // block-uniform trip count (full-mask shuffles inside)
-    const int j = j0 + grp, k = w * fh.bnd_share + j;
-    const bool valid = j < fh.bnd_share && k < B.n;
-    int beg = 0, mid = 0;
-    if (valid) {
-      beg = B.ptr[k];
-      mid = B.mid[k];
-    }
-    double s = row_part<false>(B.col, B.val, beg, mid, lane, lanes, x);
-    for (int o = lanes >> 1; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-    if (valid && lane == 0) s_bnd[j] = s;
-  }
-}
-
-template <int MODE, bool DOT>
-__device__ __forceinline__ double unified_bnd_ghost(const FusedHalo& fh, const EpiArgs& a, DevState* st, const double* s_bnd, int w,
-                                                    int n_work) {
-  __shared__ int s_par;
-  const BndView& B = fh.B;
-  const int lanes = B.lanes, lane = threadIdx.x & (lanes - 1), grp = threadIdx.x / lanes, rpb = BLOCK / lanes;
-  const bool have_rows = w * fh.bnd_share < B.n;
-  if (threadIdx.x == 0) {
-    if (fh.fixed_parity >= 0) {
-      s_par = fh.fixed_parity;
-    } else {
-      const uint32_t e = *(volatile uint32_t*)&st->halo_epoch[fh.level] + 1u;
-      // CTA 0 always consumes the exchange (keeps the epoch protocol in step even without boundary rows)
-      if (have_rows || w == 0) halo_wait(fh.hr, e, st);
-      s_par = (int)(e & 1u);
-    }
-  }
-  __syncthreads();  // also orders the s_bnd stores of step 2 before the loads below
-  const double* g = fh.hr.ghost[s_par];
-  double acc = 0.0;
-  if (have_rows)
-    for (int j0 = 0; j0 < fh.bnd_share; j0 += rpb) {
-      const int j = j0 + grp, k = w * fh.bnd_share + j;
-      const bool valid = j < fh.bnd_share && k < B.n;
-      int mid = 0, end = 0;
-      if (valid) {
-        mid = B.mid[k];
-        end = B.ptr[k + 1];
-      }
-      double sg = row_part<true>(B.col, B.val, mid, end, lane, lanes, g);
-      for (int o = lanes >> 1; o > 0; o >>= 1) sg += __shfl_xor_sync(0xffffffffu, sg, o);
-      if (valid && lane == 0) {
-        const double res = apply_epilogue<MODE, DOT>(a, B.rows[k], s_bnd[j] + sg);  // mul!: own-own sum, then += own-ghost sum
-        if (DOT) acc += res;
-      }
-    }
-  if (fh.fixed_parity < 0 && last_block_n(&st->ticket[4], (uint32_t)n_work)) {
-    if (threadIdx.x == 0) {  // every CTA is through with epoch e: advance once the local pack is out
-      const uint32_t e = *(volatile uint32_t*)&st->halo_epoch[fh.level] + 1u;
-      if (fh.n_pack > 0) spin_until(&st->pack_done[fh.level], e, st);
-      *(volatile uint32_t*)&st->halo_epoch[fh.level] = e;
-    }
-  }
-  return acc;
-}
 
 // U: entries of a row in flight per step; MINB: resident CTAs per SM the register budget must allow.  The defaults are the
 // production kernels (RPT = 2: 4 x 128-bit value loads + 4 x 64-bit column loads per thread and step, 3 CTAs/SM).  The
@@ -1518,99 +1347,6 @@ __global__ void __launch_bounds__(BLOCK, MINB) k_spmv_sell_diag(SellDiagView A, 
   if (DOT) dot_finish(s_acc[threadIdx.x], partials, st, &st->ticket[0], rc, publish, 0, red_slot);
 }
 
-// The unified-role kernel (RPT = 2, U = 4).  A kernel of its own: with the role code inlined into k_spmv_sell, ptxas gave
-// three of the production instantiations 80 instead of 72 registers and a worse load schedule (L0 Jacobi +5 %, P0 2.2x).
-template <int MODE, bool DOT>
-__global__ void __launch_bounds__(BLOCK, 3) k_spmv_sell_uni(SellView A, const double* __restrict__ x, EpiArgs a, DevState* st,
-                                                          FusedHalo fh, double* partials, RedCtx rc, int publish, int red_slot) {
-  if (st->done) return;
-  trace_mark(st);
-  // fh.unified == 1: every CTA packs, does boundary rows (own part before, ghost part behind the slices) and slices.
-  // fh.unified == 2 ("lite"): the first fh.n_pack CTAs are pack CTAs as in k_spmv_sell; the others stream their static
-  // share of the slices and THEN run the whole boundary role over fh.n_bnd = all work CTAs (the flags are there by then).
-  const bool lite = fh.unified == 2;
-  if (lite && (int)blockIdx.x < fh.n_pack) {
-    pack_role(fh, st, blockIdx.x);
-    if (DOT) dot_finish(0.0, partials, st, &st->ticket[0], rc, publish, 0, red_slot);
-    return;
-  }
-  const int n_main = lite ? (int)gridDim.x - fh.n_pack : (int)gridDim.x, bid = lite ? (int)blockIdx.x - fh.n_pack : (int)blockIdx.x;
-  constexpr int RPT = 2, U = 4;
-  using V = typename SellVec<RPT>::V;
-  using I = typename SellVec<RPT>::I;
-  const int lane = threadIdx.x & 31;
-  const int wpb = BLOCK / 32;
-  __shared__ double s_acc[DOT ? BLOCK : 1];  // per-thread running dot (each thread touches only its own slot)
-  __shared__ double s_bnd[BLOCK];            // unified roles: own-column sums of this CTA's boundary rows
-  if (DOT) s_acc[threadIdx.x] = 0.0;
-  if (!lite) {
-    if (fh.n_pack > 0) pack_role(fh, st, bid);
-    if (fh.n_bnd > 0) unified_bnd_own<MODE, DOT>(fh, x, s_bnd, bid);
-  }
-  for (int sl = bid * wpb + (threadIdx.x >> 5); sl < A.nslices; sl += n_main * wpb) {
-    const int o0 = A.slice_off[sl], w = A.slice_off[sl + 1] - o0;
-    const int slot0 = sl * (32 * RPT) + lane * RPT;
-    // Nothing but the row sums stays in registers across the entry loop: the epilogue operands, the skip flags and
-    // (with a permutation) the row ids are prefetched into L1 here and loaded after the loop.
-#pragma unroll
-    for (int k = 0; k < RPT; ++k) {
-      const int slot = slot0 + k;
-      if (slot < A.nrows) {
-        const int r = A.perm ? A.perm[slot] : slot;
-        if (fh.skip) asm volatile("prefetch.global.L1 [%0];" ::"l"(fh.skip + r));
-        if (MODE == M_RESID || MODE == M_JACOBI || MODE == M_ADD || MODE == M_CHEB) prefetch_l1(a.in0 + r);
-        if (MODE == M_JACOBI || MODE == M_CHEB || (MODE == M_RESTRICT && a.out2)) prefetch_l1(a.w + r);
-        if (MODE == M_CHEB && a.aux) prefetch_l1(a.aux + r);
-        if (DOT && a.dotv != a.in0) prefetch_l1(a.dotv + r);
-      }
-    }
-    double s[RPT];
-#pragma unroll
-    for (int k = 0; k < RPT; ++k) s[k] = 0.0;
-    const V* __restrict__ vj = reinterpret_cast<const V*>(A.val) + (size_t)o0 * 32 + lane;
-    const I* __restrict__ cj = reinterpret_cast<const I*>(A.col) + (size_t)o0 * 32 + lane;
-#pragma unroll 1
-    for (int j0 = 0; j0 < w; j0 += U, vj += U * 32, cj += U * 32) {
-      V v[U];
-      I c[U];
-#pragma unroll
-      for (int u = 0; u < U; ++u)
-        if (j0 + u < w) {
-          c[u] = __ldcs(cj + u * 32);
-          v[u] = __ldcs(vj + u * 32);
-        }
-      double xv[U][RPT];
-#pragma unroll
-      for (int u = 0; u < U; ++u)
-        if (j0 + u < w) {
-#pragma unroll
-          for (int k = 0; k < RPT; ++k) xv[u][k] = x[sv_get(c[u], k)];
-        }
-#pragma unroll
-      for (int u = 0; u < U; ++u)
-        if (j0 + u < w) {
-#pragma unroll
-          for (int k = 0; k < RPT; ++k) s[k] = __dadd_rn(s[k], __dmul_rn(sv_get(v[u], k), xv[u][k]));
-        }
-    }
-    double contrib = 0.0;
-#pragma unroll
-    for (int k = 0; k < RPT; ++k) {
-      const int slot = slot0 + k;
-      if (slot < A.nrows) {
-        const int r = A.perm ? A.perm[slot] : slot;
-        if (fh.skip && fh.skip[r]) continue;
-        const double res = apply_epilogue<MODE, false>(a, r, s[k]);
-        if (DOT) contrib += a.dotv[r] * res;  // after the stores: an L1 hit (prefetched above), and it keeps ptxas batching the loop loads
-      }
-    }
-    if (DOT) s_acc[threadIdx.x] += contrib;  // in shared memory: a register live across the entry loop costs its load batching
-  }
-  double bacc = 0.0;
-  if (fh.n_bnd > 0) bacc = lite ? boundary_role<MODE, DOT>(fh, x, a, st, bid) : unified_bnd_ghost<MODE, DOT>(fh, a, st, s_bnd, bid, n_main);
-  if (DOT) dot_finish(s_acc[threadIdx.x] + bacc, partials, st, &st->ticket[0], rc, publish, 0, red_slot);
-}
-
 // ---------------------------------------------------------------------------------------------
 // halo pack: owner -> ghost (consistent!).  Stores into the neighbours' staging, then flags.
 // ---------------------------------------------------------------------------------------------
@@ -1800,145 +1536,6 @@ __global__ void __launch_bounds__(BLOCK) k_tail_out(const double* __restrict__ x
     else
       xg[r - n_own] = xfull[ghost_gid[r - n_own]];
   }
-}
-
-// ---------------------------------------------------------------------------------------------
-// Fused replicated tail: ONE persistent kernel runs gather -> tail_in -> the whole V-cycle of the merged levels ->
-// tail_out, its phases separated by grid barriers instead of kernel boundaries.  On 8 GPUs the tail of the 256^3
-// hierarchy (44k + 2k + 0.4k rows) was 12 launches and 104 us of a 523 us iteration (profiles/r01 trace): every launch
-// pays ~4-6 us of launch latency for ~1 us of work, and the 3 M-entry level ran as 1000 CTAs in two waves.  The row
-// arithmetic is the CSR-stream family's (stream_row_block), so the results equal the multi-launch path bit for bit.
-// All CTAs must be resident at once (grid = at most the occupancy limit, nothing else runs on the stream).
-// ---------------------------------------------------------------------------------------------
-enum TailKind : int { T_GATHER = 0, T_IN = 1, T_STREAM = 2, T_DENSE = 3, T_SCALE = 4, T_OUT = 5 };
-struct TailOp {   // one phase; pointers come from memory, so no load in the kernel may take the non-coherent path
-  int32_t kind, mode;
-  StreamView A;      // T_STREAM
-  const double* x;   // T_STREAM: gather vector | T_DENSE, T_SCALE: b
-  EpiArgs a;         // T_STREAM epilogue | T_DENSE, T_SCALE: a.out (T_SCALE: a.w or nullptr)
-  int32_t n;         // T_DENSE, T_SCALE: length
-};
-struct TailIO {
-  const double *g0, *g1;      // this part's gather buffer, per parity
-  const uint32_t* flags;      // [nparts]
-  const CoarsePub* pubs;      // T_GATHER: where this part's slice goes in every part
-  const double* b_own;        // restricted residual of this part on the entry level
-  const int64_t *own_gid, *ghost_gid;
-  int32_t nparts, n_own, n_ghost, n;  // n: rows of the entry level (all parts)
-  double *b_full, *xstart;    // T_IN outputs (merged entry level)
-  const double* w;            // T_IN: smoother weights of the merged entry level (nullptr: xstart = 0)
-  const double* x_full;       // T_OUT input
-  double *x_own, *xg;         // T_OUT outputs: own slice and ghost staging (parity 0) of the entry level
-  const double* inv;          // dense inverse of the coarsest matrix
-  int32_t do_gather;          // 1: the gather is phase 0 of this kernel (every part alone on its GPU)
-};
-
-__device__ __forceinline__ uint32_t ld_acquire_gpu(const uint32_t* p) {
-  uint32_t v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ uint32_t atom_add_acq_rel_gpu(uint32_t* p, uint32_t v) {
-  uint32_t r;
-  asm volatile("atom.acq_rel.gpu.global.add.u32 %0, [%1], %2;" : "=r"(r) : "l"(p), "r"(v) : "memory");
-  return r;
-}
-__device__ __forceinline__ void st_release_gpu(uint32_t* p, uint32_t v) {
-  asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-// Sense-reversing barrier over all CTAs of the grid; `gen` = the generation every thread read at kernel start.
-// Arrive = one acq_rel atomic (release: cumulative over the CTA's stores ordered before it by bar.sync), wait = acquire
-// loads of the generation word (the acquire also drops this SM's L1 lines of vectors other CTAs have rewritten).
-// sys: the CTA's stores before the barrier must be visible system-wide (peer GPUs), not only device-wide.
-__device__ __forceinline__ void grid_barrier(DevState* st, uint32_t& gen, bool sys) {
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    if (sys) __threadfence_system();
-    const uint32_t t = atom_add_acq_rel_gpu(&st->bar_count, 1u);
-    if (t == gridDim.x - 1) {
-      *(volatile uint32_t*)&st->bar_count = 0;
-      st_release_gpu(&st->bar_gen, gen + 1u);
-    } else {
-      while (ld_acquire_gpu(&st->bar_gen) == gen) {
-      }
-    }
-  }
-  ++gen;
-  __syncthreads();
-}
-
-// not inlined: six inlined copies of the row-block body in one kernel spilled 1 KB per thread
-template <int MODE>
-__device__ __noinline__ void tail_stream_phase(const TailOp& op, double* prod) {
-  double acc = 0.0;
-  for (int bk = blockIdx.x; bk < op.A.nblocks; bk += gridDim.x)
-    stream_row_block<MODE, false, false>(op.A, op.x, op.a, nullptr, bk, prod, acc, bk + (int)gridDim.x < op.A.nblocks);
-}
-
-__global__ void __launch_bounds__(BLOCK, 4) k_tail_fused(const TailOp* __restrict__ ops, int n_ops, TailIO io, DevState* st) {
-  if (st->done) return;
-  trace_mark(st);
-  __shared__ double prod[S_STEPS * 4 * BLOCK];
-  __shared__ TailOp s_op;
-  uint32_t gen = *(volatile uint32_t*)&st->bar_gen;  // cannot change before every CTA has arrived at the first barrier
-  const uint32_t e = *(volatile uint32_t*)&st->coarse_epoch + (io.do_gather ? 1u : 0u);
-  const int par = (int)(e & 1u);
-  const int gtid = blockIdx.x * BLOCK + threadIdx.x, gsz = gridDim.x * BLOCK;
-  if (io.do_gather) {  // all-gather of the entry level's right-hand side: this part's slice into every part
-    for (int d = 0; d < io.nparts; ++d) {
-      double* dst = io.pubs[d].buf[par];
-      for (int i = gtid; i < io.n_own; i += gsz) dst[io.own_gid[i]] = io.b_own[i];
-    }
-    grid_barrier(st, gen, true);
-    if (blockIdx.x == 0 && threadIdx.x < io.nparts) st_release_sys(io.pubs[threadIdx.x].flag, e);
-  }
-  {  // T_IN: wait for every part's slice, copy, zero-guess first smoothing step
-    if (threadIdx.x == 0) spin_until_all(io.flags, io.nparts, e, st);
-    __syncthreads();
-    const double* g = par ? io.g1 : io.g0;
-    for (int i = gtid; i < io.n; i += gsz) {
-      const double v = __ldcv(g + i);
-      io.b_full[i] = v;
-      if (io.xstart) io.xstart[i] = io.w ? io.w[i] * v : 0.0;
-    }
-  }
-  for (int k = 0; k < n_ops; ++k) {
-    grid_barrier(st, gen, false);
-    static_assert(sizeof(TailOp) % 8 == 0, "TailOp is copied in 8-byte words");
-    if (threadIdx.x < sizeof(TailOp) / 8)
-      reinterpret_cast<unsigned long long*>(&s_op)[threadIdx.x] = reinterpret_cast<const unsigned long long*>(ops + k)[threadIdx.x];
-    __syncthreads();
-    const TailOp& op = s_op;
-    if (op.kind == T_STREAM) {
-      switch (op.mode) {
-        case M_RESID: tail_stream_phase<M_RESID>(op, prod); break;
-        case M_RESTRICT: tail_stream_phase<M_RESTRICT>(op, prod); break;
-        case M_ADD: tail_stream_phase<M_ADD>(op, prod); break;
-        case M_JACOBI: tail_stream_phase<M_JACOBI>(op, prod); break;
-        case M_CHEB: tail_stream_phase<M_CHEB>(op, prod); break;
-        default: tail_stream_phase<M_MUL>(op, prod); break;
-      }
-    } else if (op.kind == T_DENSE) {  // x = inv * b, one warp per row (same arithmetic as k_dense)
-      const int lane = threadIdx.x & 31, warp = gtid >> 5, nwarps = gsz >> 5;
-      for (int r = warp; r < op.n; r += nwarps) {
-        const double* row = io.inv + (size_t)r * op.n;
-        double s = 0.0;
-        for (int j = lane; j < op.n; j += 32) s += row[j] * op.x[j];
-        s = group_sum<32>(s);
-        if (lane == 0) op.a.out[r] = s;
-      }
-    } else if (op.kind == T_SCALE) {
-      for (int i = gtid; i < op.n; i += gsz) op.a.out[i] = op.a.w ? op.a.w[i] * op.x[i] : 0.0;
-    }
-  }
-  grid_barrier(st, gen, false);
-  for (int r = gtid; r < io.n_own + io.n_ghost; r += gsz) {  // T_OUT
-    if (r < io.n_own)
-      io.x_own[r] = io.x_full[io.own_gid[r]];
-    else
-      io.xg[r - io.n_own] = io.x_full[io.ghost_gid[r - io.n_own]];
-  }
-  if (io.do_gather && blockIdx.x == 0 && threadIdx.x == 0) st->coarse_epoch = e;  // every CTA read it before the first barrier
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -41,16 +41,11 @@ CONFIGS = {
 }
 # A/B switches of the engine (read at device_init): name -> environment
 ENVS = {
-    "auto-r1": dict(PAMG_P_KERNEL="0", PAMG_RENUMBER="0", PAMG_STREAM_LONG="0"),       # round-1 behaviour
+    "auto-r1": dict(PAMG_P_KERNEL="0", PAMG_STREAM_LONG="0"),       # round-1 behaviour
     "auto-p0": dict(PAMG_P_KERNEL="0"),
     "auto-p2": dict(PAMG_P_KERNEL="2"),
-    "auto-nore": dict(PAMG_RENUMBER="0"),
     "auto-nosort": dict(PAMG_SELL_SORT_FILL="9"),
     "auto-p2-nosort": dict(PAMG_P_KERNEL="2", PAMG_SELL_SORT_FILL="9"),
-    "auto-w16k": dict(PAMG_RENUMBER="1", PAMG_RENUMBER_WINDOW="16384"),
-    "auto-renum": dict(PAMG_RENUMBER="1"),
-    "auto-w512": dict(PAMG_RENUMBER="1", PAMG_RENUMBER_WINDOW="512"),
-    "auto-w1024": dict(PAMG_RENUMBER="1", PAMG_RENUMBER_WINDOW="1024"),
     "auto-p1": dict(PAMG_P_KERNEL="1"),
     "auto-nolong": dict(PAMG_STREAM_LONG="0"),
     "auto-psig256": dict(PAMG_P_SIGMA="256"),
@@ -67,7 +62,6 @@ ENVS = {
     "auto-occ1": dict(PAMG_VI_OCC="1"),            # one-byte value-indexed kernel at 64 registers / 4 CTAs per SM (U = 4, spills)
     "auto-occ2": dict(PAMG_VI_OCC="2"),            # ... U = 2, no spills
     "auto-plong": dict(PAMG_VI_PERSIST_LONG="1"),  # level-1 A (value-indexed, 31 entries per row) as one resident wave + look-ahead
-    "auto-plong-w512": dict(PAMG_VI_PERSIST_LONG="1", PAMG_RENUMBER="1", PAMG_RENUMBER_WINDOW="512"),         # extents one iteration early + L2 prefetch of the next slice
     "auto-vi8only": dict(PAMG_VALUE_INDEX="1"),    # one-byte indices only (no wide dictionaries on the coarse levels)
     "auto-vi0": dict(PAMG_VI_VARIANT="0"),         # two rows per lane
     "auto-vi-sorted": dict(PAMG_SELL_SORT_FILL="1.25"),
@@ -76,8 +70,6 @@ ENVS = {
     "auto-pf3": dict(PAMG_SELL_PF="3"),
     "auto-pf5": dict(PAMG_SELL_PF="5"),
     "auto-pf7": dict(PAMG_SELL_PF="7"),
-    "auto-pf7-w512": dict(PAMG_SELL_PF="7", PAMG_RENUMBER="1", PAMG_RENUMBER_WINDOW="512"),
-    "auto-pf1-w512": dict(PAMG_SELL_PF="1", PAMG_RENUMBER="1", PAMG_RENUMBER_WINDOW="512"),
 }
 for k in ENVS:
     CONFIGS[k] = dict(spmv_format=L.FORMAT_AUTO)
@@ -87,7 +79,7 @@ else:
     CONFIGS = {k: v for k, v in CONFIGS.items() if k not in ENVS}
 res = {}
 for name, kw in CONFIGS.items():
-    for k in ("PAMG_VI_OCC", "PAMG_VI_PERSIST_LONG", "PAMG_VI_AHEAD", "PAMG_VALUE_INDEX", "PAMG_VI_VARIANT", "PAMG_P_KERNEL", "PAMG_RENUMBER", "PAMG_SELL_SORT_FILL", "PAMG_RENUMBER_WINDOW", "PAMG_STREAM_LONG", "PAMG_P_SIGMA", "PAMG_R_SIGMA", "PAMG_SELL_PF"):
+    for k in ("PAMG_VI_OCC", "PAMG_VI_PERSIST_LONG", "PAMG_VI_AHEAD", "PAMG_VALUE_INDEX", "PAMG_VI_VARIANT", "PAMG_P_KERNEL", "PAMG_SELL_SORT_FILL", "PAMG_STREAM_LONG", "PAMG_P_SIGMA", "PAMG_R_SIGMA", "PAMG_SELL_PF"):
         os.environ.pop(k, None)
     os.environ.update(ENVS.get(name, {}))
     c.set_kernel_options(**kw)

@@ -25,19 +25,17 @@ def main():
              ((40, 40, 40), {}, dict(spmv_format=L.FORMAT_SELL), {}), ((24, 20, 16), {}, dict(spmv_format=L.FORMAT_CSR), {}),
              ((40, 40, 40), {"smoother": "l1jacobi"}, dict(spmv_format=L.FORMAT_SELL, sell_sigma=128, sell_rows_per_thread=1), {}),
              ((24, 20, 16), {}, dict(fuse_halo=0), {}),
-             # unified CTA roles (SELL, RPT 2) with distributed coarse levels, two sweeps, Chebyshev; role CTAs for comparison
-             ((40, 40, 40), {"nu_pre": 2, "nu_post": 2}, dict(spmv_format=L.FORMAT_SELL, tail_rows=600), {"PAMG_UNIFIED": "15"}),
-             ((40, 40, 40), {"smoother": "chebyshev", "cheb_degree": 3}, dict(spmv_format=L.FORMAT_SELL, tail_rows=600), {"PAMG_UNIFIED": "15"}),
+             # SELL with distributed coarse levels (two sweeps, Chebyshev degree 3, defaults); l1-Jacobi and sigma 256 with no replicated tail
+             ((40, 40, 40), {"nu_pre": 2, "nu_post": 2}, dict(spmv_format=L.FORMAT_SELL, tail_rows=600), {}),
+             ((40, 40, 40), {"smoother": "chebyshev", "cheb_degree": 3}, dict(spmv_format=L.FORMAT_SELL, tail_rows=600), {}),
              ((40, 40, 40), {}, dict(spmv_format=L.FORMAT_SELL, tail_rows=600), {}),
-             ((40, 40, 40), {"nu_pre": 2, "nu_post": 2}, dict(spmv_format=L.FORMAT_SELL, tail_rows=600), {"PAMG_UNIFIED": "15", "PAMG_UNIFIED_MODE": "2"}),
-             ((48, 40, 36), {"smoother": "l1jacobi"}, dict(spmv_format=L.FORMAT_SELL, tail_rows=0), {"PAMG_UNIFIED": "15", "PAMG_UNIFIED_MODE": "2"}),
-             ((48, 40, 36), {}, dict(spmv_format=L.FORMAT_SELL, sell_sigma=256, tail_rows=0), {"PAMG_UNIFIED": "15"}),
-             # replicated tail: one launch per operation / separate convergence check / renumbered coarse levels
-             ((40, 40, 40), {}, {}, {"PAMG_FUSED_TAIL": "1"}), ((40, 40, 40), {}, {}, {"PAMG_FOLD_CHECK": "0"}),
+             ((48, 40, 36), {"smoother": "l1jacobi"}, dict(spmv_format=L.FORMAT_SELL, tail_rows=0), {}),
+             ((48, 40, 36), {}, dict(spmv_format=L.FORMAT_SELL, sell_sigma=256, tail_rows=0), {}),
+             # separate convergence check / W-cycle with a replicated tail / no pre-smoothing
+             ((40, 40, 40), {}, {}, {"PAMG_FOLD_CHECK": "0"}),
              ((40, 40, 40), {"cycle": "w", "coarse_size": 40}, dict(tail_rows=600), {}),
-             ((40, 40, 40), {"nu_pre": 0, "nu_post": 2}, {}, {}),
-             ((40, 40, 40), {}, dict(spmv_format=L.FORMAT_SELL, tail_rows=600), {"PAMG_RENUMBER": "1", "PAMG_RENUMBER_WINDOW": "256"}))
-    switches = ("PAMG_UNIFIED", "PAMG_UNIFIED_MODE", "PAMG_FUSED_TAIL", "PAMG_FOLD_CHECK", "PAMG_RENUMBER", "PAMG_RENUMBER_WINDOW")
+             ((40, 40, 40), {"nu_pre": 0, "nu_post": 2}, {}, {}))
+    switches = ("PAMG_FOLD_CHECK",)
     for dims, oopts, kopts, env in cases:
         for k in switches:
             os.environ.pop(k, None)

@@ -8,7 +8,7 @@ if [ "$3" != "notests" ]; then
 fi
 $TR --master-port 29601 bench.py --gpus $N --steps 5 --warmup 3 --trace gpurun_out/${TAG}_trace_full > gpurun_out/${TAG}_bench_full.json 2> gpurun_out/${TAG}_bench_full.err; echo "rc=$?" >> gpurun_out/${TAG}_bench_full.err
 P=29602
-for SW in "PAMG_UNIFIED=0" "PAMG_FUSED_TAIL=0" "PAMG_FOLD_CHECK=0" "PAMG_UNIFIED=0 PAMG_FUSED_TAIL=0 PAMG_FOLD_CHECK=0"; do
+for SW in "PAMG_FOLD_CHECK=0"; do
   NAME=$(echo "$SW" | tr ' =' '__')
   env $SW $TR --master-port $P bench.py --gpus $N --steps 5 --warmup 3 --no-cpu-baseline --no-small-parity --secondary none \
       --trace gpurun_out/${TAG}_trace_${NAME} > gpurun_out/${TAG}_bench_${NAME}.json 2> gpurun_out/${TAG}_bench_${NAME}.err; echo "rc=$?" >> gpurun_out/${TAG}_bench_${NAME}.err

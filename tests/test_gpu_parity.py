@@ -184,13 +184,11 @@ def test_pcg_iteration_count_and_history(dims, pp, oopts):
 
 @pytest.mark.parametrize("dims,pp", PROBLEMS[1:])
 @pytest.mark.parametrize("tail_rows", [0, 600, 1 << 20])
-@pytest.mark.parametrize("fused_tail", ["0", "1"], ids=["tail-launches", "tail-one-kernel"])
-def test_coarse_agglomeration_thresholds(dims, pp, tail_rows, fused_tail, monkeypatch):
+def test_coarse_agglomeration_thresholds(dims, pp, tail_rows):
     """Coarse-level agglomeration (levels merged over all parts and run replicated, pamg_options.tail_rows)
     is an execution layout, not a different hierarchy: whatever the threshold, the V-cycle matches the
-    oracle's N-part V-cycle to 1e-12 and PCG takes the same number of iterations.  The tail runs either as one launch
-    per operation (default) or as ONE persistent kernel with grid barriers (PAMG_FUSED_TAIL=1): same row arithmetic."""
-    monkeypatch.setenv("PAMG_FUSED_TAIL", fused_tail)
+    oracle's N-part V-cycle to 1e-12 and PCG takes the same number of iterations.  The tail runs one launch per
+    operation."""
     A, h, c = make(dims, pp, None, tail_rows=tail_rows)
     L_ = len(h["levels"])
     sizes = [h["global"]["levels"][l]["A"].shape[0] for l in range(L_)]
