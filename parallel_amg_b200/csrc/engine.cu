@@ -82,7 +82,6 @@ struct DevCsr {
   int nslices = 0, sell_rpt = 0, sell_sigma = 1;  // sell_rpt != 0 <=> the SELL kernel runs this block
   bool sell_perm = false;
   double sell_fill = 1.0;  // stored entries / nnz
-  bool short_rows = false; // no row has more than 8 entries (prolongators): eligible for the short-row instantiations
   // value-indexed SELL (RPT = 2 only): one byte per stored entry into a dictionary of the <= 256 distinct values
   DBuf<uint8_t> sl_vidx;
   DBuf<double> sl_dict;
@@ -185,7 +184,7 @@ void merged_block(const Hierarchy& h, int l, int which, LocalCsr& out) {
 constexpr double SELL_AUTO_MAX_FILL = 1.25;
 // AUTO per operator (gpurun kernel sweep, profiles/r01_kernel_sweep.md): A -> SELL (0.29 vs 0.36 ms at 256^3);
 // R -> SELL only with enough coarse rows to fill the GPU one thread per row, else CSR-stream (few, long rows);
-// P (1-8 entries per row) -> SELL like A once the short-row kernels run as persistent CTAs (0.228 vs 0.268 ms).
+// P (1-8 entries per row) -> SELL like A once its short rows run as one resident wave of persistent CTAs (0.228 vs 0.268 ms).
 // (one thread per row needs >= ~200k rows to fill 148 SMs: at 44k rows x 68 nnz the SELL sweep takes 63 us, CSR-stream 20 us)
 constexpr int64_t SELL_AUTO_MIN_ROWS_A = 200000, SELL_AUTO_MIN_ROWS_R = 65536;
 
@@ -199,12 +198,7 @@ int pick_lanes(double mean) {
 }
 
 // fmt: PAMG_FORMAT_* requested for this block (own-ghost blocks are always compressed-row CSR)
-// value-indexed kernel when PAMG_VI_VARIANT is not set (Engine::Impl::vi_variant): 3 = four interleaved rows per lane (256^3 solve
-// 34.5 ms; 0 = two rows per lane 39.4 ms; fp64 values 43.1 ms; 1 = <U 8, 2 CTAs/SM> and 2 = software-pipelined: slower than 0)
-constexpr int VI_DEFAULT_VARIANT = 3;
-
-void build_csr(const LocalCsr& m, bool compress, DevCsr& d, int lanes_override, int fmt, const pamg_options& o, int which,
-               int rpt_override = 0) {
+void build_csr(const LocalCsr& m, bool compress, DevCsr& d, int lanes_override, int fmt, const pamg_options& o, int which) {
   const int64_t nr = m.nrows;
   std::vector<int32_t> ptr;
   d.listed = compress;
@@ -215,12 +209,6 @@ void build_csr(const LocalCsr& m, bool compress, DevCsr& d, int lanes_override, 
   d.sell_vi = false;
   d.sell_vi4 = false;
   d.sell_diag = false;
-  d.short_rows = false;
-  if (!m.ptr.empty()) {
-    int64_t mx = 0;
-    for (int64_t i = 0; i < nr; ++i) mx = std::max(mx, m.ptr[i + 1] - m.ptr[i]);
-    d.short_rows = mx <= 8;
-  }
   if (m.ptr.empty()) {  // absent block
     d.nrows = compress ? 0 : (int32_t)nr;
     ptr.assign((compress ? 0 : nr) + 1, 0);
@@ -256,9 +244,7 @@ void build_csr(const LocalCsr& m, bool compress, DevCsr& d, int lanes_override, 
   }
   const bool sell_req = fmt == PAMG_FORMAT_SELL || fmt == PAMG_FORMAT_SELL_DIAG;
   if (!compress && nr > 0 && (sell_req || auto_sell)) {
-    const int rpt = (o.sell_rows_per_thread == 1 || o.sell_rows_per_thread == 2) ? o.sell_rows_per_thread
-                    : (rpt_override == 1 && d.short_rows)                             ? 1
-                                                                                      : 2;
+    const int rpt = (o.sell_rows_per_thread == 1 || o.sell_rows_per_thread == 2) ? o.sell_rows_per_thread : 2;
     // stencil A blocks: implied columns, one index byte per slot (0.117 instead of 0.585 GB per pass over A0 at 256^3); only under AUTO and
     // SELL_DIAG (an explicit SELL keeps the column-stored layouts), and like every value-indexed layout not with PAMG_VALUE_INDEX=0
     const char* ve = getenv("PAMG_VALUE_INDEX");
@@ -286,27 +272,22 @@ void build_csr(const LocalCsr& m, bool compress, DevCsr& d, int lanes_override, 
     const int C = 32 * rpt;
     SellHost sh;
     int sigma = o.sell_sigma > 0 ? o.sell_sigma : 1;
-    int forced_sigma = 0;  // experiments: sorting window of one operator class (rows), overriding the automatic choice
-    if (which == PAMG_P_OO && getenv("PAMG_P_SIGMA")) forced_sigma = atoi(getenv("PAMG_P_SIGMA"));
-    if (which == PAMG_R_OO && getenv("PAMG_R_SIGMA")) forced_sigma = atoi(getenv("PAMG_R_SIGMA"));
-    if (forced_sigma > 0) sigma = forced_sigma;
     sell_layout(m, C, sigma, sh, false);
     // few distinct values (stencil matrices, their prolongators): value-indexed storage, 5 instead of 12 bytes per entry; up to
     // VI_WIDE_MAX - 1 distinct values (Galerkin matrix of the first coarse level): two index bytes, 6 instead of 12 (128-row layout only)
     bool vi_ok = false, vi_wide = false;
     {
       const char* e = getenv("PAMG_VALUE_INDEX");
-      const char* vv = getenv("PAMG_VI_VARIANT");
       const bool on = rpt == 2 && !(e && atoi(e) == 0);
       vi_ok = on && value_dictionary(m, sh.dict, 255);
-      if (on && !vi_ok && (vv ? atoi(vv) : VI_DEFAULT_VARIANT) == 3 && !(e && atoi(e) == 1) && o.sell_sigma <= 1 && forced_sigma <= 0)
+      if (on && !vi_ok && !(e && atoi(e) == 1) && o.sell_sigma <= 1)
         vi_wide = value_dictionary(m, sh.dict, VI_WIDE_MAX - 1);  // PAMG_VALUE_INDEX=1: one-byte indices only
     }
     // auto sigma: sort inside windows only when the unsorted padding is large (the permutation costs more than
     // ~20 % padding does: P at 256^3 runs 0.228 ms unsorted with 1.16x fill, 0.240 ms sorted with 1.01x).  A value-indexed
     // block pads with 5-byte entries and pays the same for the permutation: 0.202 ms unsorted (1.41x) vs 0.229 ms sorted
-    const double sort_fill = getenv("PAMG_SELL_SORT_FILL") ? atof(getenv("PAMG_SELL_SORT_FILL")) : ((vi_ok || vi_wide) ? 2.0 : 1.25);
-    if (o.sell_sigma <= 0 && forced_sigma <= 0 && sh.fill > sort_fill) {
+    const double sort_fill = (vi_ok || vi_wide) ? 2.0 : 1.25;
+    if (o.sell_sigma <= 0 && sh.fill > sort_fill) {
       SellHost s2;
       sell_layout(m, C, 64 * C, s2, false);
       if (s2.fill < sh.fill - 0.02) sigma = 64 * C;
@@ -328,8 +309,8 @@ void build_csr(const LocalCsr& m, bool compress, DevCsr& d, int lanes_override, 
       if (vi_ok || vi_wide) {
         d.ndict = (int)sh.dict.size();
         d.sl_dict.upload(sh.dict);
-        const char* vv = getenv("PAMG_VI_VARIANT");
-        if ((vv ? atoi(vv) : VI_DEFAULT_VARIANT) == 3 && !sh.permuted) {  // four interleaved rows per lane: a second, 128-row slicing
+        // four interleaved rows per lane (k_spmv_sell_vi4): a second, 128-row slicing.  Sorted rows keep the two-rows-per-lane kernel.
+        if (!sh.permuted) {
           SellHost s4;
           s4.dict = sh.dict;
           sell_layout(m, 128, 1, s4, true, 4);
@@ -487,20 +468,8 @@ struct Engine::Impl {
   std::vector<void*> ipc_opened;
   std::map<int, cudaStream_t> stream_of_device;
   bool connected = false;
-  int bnd_first = -1;       // block ids of a fused launch: 1 [pack | boundary | main], 0 [pack | main | boundary], -1 by size
-  bool persistent = true;   // SELL / CSR-stream main roles run as one resident wave (env PAMG_PERSISTENT=0: one CTA per work item)
   bool fused_halo = false;  // every local part has a GPU of its own: halo roles run inside the consuming kernel
   bool fold_check = false;  // the convergence check runs inside k_update_xr / k_pcg_init (every local part alone on its GPU)
-  bool stream_long = true;  // CSR-stream blocks with long rows use 16 lanes per row in phase B (env PAMG_STREAM_LONG=0: one thread per row)
-  int sell_pf = 0;          // persistent SELL launches with an L2 prefetch two slices ahead: bit mask 1 P, 2 long-row A, 4 R (env PAMG_SELL_PF)
-  int vi_occ = 2;           // one-byte value-indexed kernel, persistent launches (short rows): 2 = U = 2 at 64 registers / 4 CTAs per SM (shipped:
-                            // 256^3 solve 33.7 -> 31.4 ms, SpMV 0.163 -> 0.144 ms), 0 = U = 4 at 80 registers / 3 CTAs, 1 = U = 4 squeezed into 64
-                            // registers (spills: 40.3 ms); env PAMG_VI_OCC
-  bool vi_persist_long = false;  // long-row value-indexed blocks (level-1 A) as one resident wave too, so that the look-ahead applies (env PAMG_VI_PERSIST_LONG)
-  bool vi_ahead = true;     // 128-row value-indexed kernel, persistent launches: next slice's extents one iteration early + L2 prefetch
-                            // (env PAMG_VI_AHEAD=0 turns it off; 256^3: solve 34.03 -> 33.58 ms, Jacobi sweep 0.221 -> 0.209 ms, plain SpMV 0.159 -> 0.162)
-  int vi_variant = VI_DEFAULT_VARIANT;  // value-indexed SELL kernel (3 = four interleaved rows per lane): 0 = <U 4, 3 CTAs/SM>, 1 = <U 8, 2 CTAs/SM>, 2 = software-pipelined (env PAMG_VI_VARIANT)
-  int p_kernel = 0;         // SELL instantiation of the prolongators (launch_sell short_variant; env PAMG_P_KERNEL; measured: no gain)
   int64_t launches = 0;
   bool counting = true;
   // exchange needed per level/operator (decided on global metadata so every part agrees)
@@ -592,6 +561,21 @@ struct LaunchArgs {  // what every SpMV-family launch shares
   int publish, slot;   // fused dot: publish = 1 total goes to every part, 0 a boundary launch completes it
 };
 
+// The kernel an operation runs, decided once from its block (and long_rows, see launch_stream); the launch and the trace name both follow
+// from it.
+enum class SpmvKernel { SellDiag, SellVi, SellVi16, SellVi2, Sell, Stream, StreamLong, Csr };
+// sell-vi = four rows per lane (one-byte indices), sell-vi16 = the same with two-byte indices, sell-vi2 = two rows per lane (sorted rows)
+const char* const SPMV_KERNEL_NAMES[] = {"sell-diag", "sell-vi", "sell-vi16", "sell-vi2", "sell", "stream", "stream-long", "csr"};
+
+SpmvKernel spmv_kernel(const DevCsr& m, bool long_rows) {
+  if (m.sell_diag) return SpmvKernel::SellDiag;
+  if (m.sell_vi4) return m.vi4_ib == 2 ? SpmvKernel::SellVi16 : SpmvKernel::SellVi;
+  if (m.sell_vi) return SpmvKernel::SellVi2;
+  if (m.sell_rpt) return SpmvKernel::Sell;
+  if (m.stream) return long_rows ? SpmvKernel::StreamLong : SpmvKernel::Stream;
+  return SpmvKernel::Csr;
+}
+
 int main_grid(const LaunchArgs& L, const void* kernel, size_t dyn_smem = 0) {
   int n_main = L.grid;
   if (L.bounded) n_main = std::min(n_main, std::min(resident_ctas(kernel, dyn_smem), RED_GRID));
@@ -664,38 +648,38 @@ void launch_stream(int mode, bool dot, bool long_rows, StreamView A, const Launc
   });
 }
 
-// short_variant (operators whose rows have at most 8 entries, i.e. the prolongators; M_ADD only): 0 = the A kernel,
-// 1 = <RPT 2, U 2, 5 CTAs/SM>, 2 = <RPT 1, U 4, 6 CTAs/SM> (needs the C = 32 layout).
-void launch_sell(int mode, bool dot, int rpt, int short_variant, bool prefetch, SellView A, const LaunchArgs& L,
-                 const SellViView* vi = nullptr, int vi_variant = 0, int vi_occ = 0) {
+void launch_sell(int mode, bool dot, int rpt, SellView A, const LaunchArgs& L) {
   dispatch_mode(mode, dot, [&](auto md, auto dt) {
     constexpr int MD = decltype(md)::value;
     constexpr bool DT = decltype(dt)::value;
-    if (vi && rpt == 2) {  // value-indexed operator: its own kernel (the experimental variants below do not apply)
-      using KernVi = void (*)(SellViView, const double*, EpiArgs, DevState*, FusedHalo, double*, RedCtx, int, int);
-      KernVi kv = vi_variant == 5 && vi_occ == 1 ? (KernVi)k_spmv_sell_vi4<MD, DT, 1, 4, 4, 1>   // 64 registers (spills), 4 CTAs/SM
-                  : vi_variant == 5 && vi_occ == 2 ? (KernVi)k_spmv_sell_vi4<MD, DT, 1, 2, 4, 1> // U = 2, 64 registers, 4 CTAs/SM
-                  : vi_variant == 6 ? (KernVi)k_spmv_sell_vi4<MD, DT, 2, 4, 3, 1>
-                  : vi_variant == 5 ? (KernVi)k_spmv_sell_vi4<MD, DT, 1, 4, 3, 1>
-                  : vi_variant == 4 ? (KernVi)k_spmv_sell_vi4<MD, DT, 2>
-                  : vi_variant == 3 ? (KernVi)k_spmv_sell_vi4<MD, DT, 1>
-                  : vi_variant == 2 ? (KernVi)k_spmv_sell_vi_pipe<MD, DT>
-                  : vi_variant == 1 ? (KernVi)k_spmv_sell_vi<MD, DT, 8, 2>
-                                    : (KernVi)k_spmv_sell_vi<MD, DT, 4, 3>;
-      const size_t dyn = vi_variant >= 3 ? (size_t)vi->ndict * sizeof(double) : 0;  // the 128-row kernel keeps its dictionary in dynamic shared memory
-      kv<<<main_grid(L, (const void*)kv, dyn), BLOCK, dyn, L.s>>>(*vi, L.x, L.a, L.st, L.fh, L.partials, L.rc, L.publish, L.slot);
-      return;
-    }
     using Kern = void (*)(SellView, const double*, EpiArgs, DevState*, FusedHalo, double*, RedCtx, int, int);
     Kern k = rpt == 2 ? (Kern)k_spmv_sell<2, MD, DT> : (Kern)k_spmv_sell<1, MD, DT>;
-    if constexpr (MD == M_ADD && !DT) {
-      if (short_variant == 1 && rpt == 2) k = (Kern)k_spmv_sell<2, M_ADD, false, 2, 5>;
-      if (short_variant == 2 && rpt == 1) k = (Kern)k_spmv_sell<1, M_ADD, false, 4, 6>;
-    }
-    if constexpr (!DT) {  // L2 prefetch of the slice two iterations ahead (persistent launches of the latency-bound operators)
-      if (prefetch && rpt == 2 && short_variant == 0) k = (Kern)k_spmv_sell<2, MD, false, 4, 3, 2>;
-    }
     k<<<main_grid(L, (const void*)k), BLOCK, 0, L.s>>>(A, L.x, L.a, L.st, L.fh, L.partials, L.rc, L.publish, L.slot);
+  });
+}
+
+// value-indexed, two rows per lane (blocks with sorted rows)
+void launch_sell_vi(int mode, bool dot, const SellViView& A, const LaunchArgs& L) {
+  dispatch_mode(mode, dot, [&](auto md, auto dt) {
+    constexpr int MD = decltype(md)::value;
+    constexpr bool DT = decltype(dt)::value;
+    auto k = k_spmv_sell_vi<MD, DT>;
+    k<<<main_grid(L, (const void*)k), BLOCK, 0, L.s>>>(A, L.x, L.a, L.st, L.fh, L.partials, L.rc, L.publish, L.slot);
+  });
+}
+
+// value-indexed, four rows per lane with ib index bytes per entry.  A launch bounded to one resident wave takes the look-ahead, and in the
+// one-byte form U = 2 at 4 CTAs/SM (kernels.cuh k_spmv_sell_vi4).
+void launch_sell_vi4(int mode, bool dot, int ib, const SellViView& A, const LaunchArgs& L) {
+  dispatch_mode(mode, dot, [&](auto md, auto dt) {
+    constexpr int MD = decltype(md)::value;
+    constexpr bool DT = decltype(dt)::value;
+    using Kern = void (*)(SellViView, const double*, EpiArgs, DevState*, FusedHalo, double*, RedCtx, int, int);
+    const Kern by_ib_bounded[2][2] = {{k_spmv_sell_vi4<MD, DT, 1>, k_spmv_sell_vi4<MD, DT, 1, 2, 4, 1>},
+                                      {k_spmv_sell_vi4<MD, DT, 2>, k_spmv_sell_vi4<MD, DT, 2, 4, 3, 1>}};
+    const Kern k = by_ib_bounded[ib == 2][L.bounded];
+    const size_t dyn = (size_t)A.ndict * sizeof(double);  // the dictionary lives in dynamic shared memory
+    k<<<main_grid(L, (const void*)k, dyn), BLOCK, dyn, L.s>>>(A, L.x, L.a, L.st, L.fh, L.partials, L.rc, L.publish, L.slot);
   });
 }
 
@@ -750,8 +734,8 @@ void Engine::enqueue_op(const OpSpec& op, const std::vector<const double*>& xin,
     fh.fixed_parity = op.coarse_ghosts_local ? 0 : -1;
     fh.fused = fused ? 1 : 0;
     // boundary CTAs ahead of a SMALL main role (their latency is all there is), behind a large one (ahead of it
-    // they would hold resident-CTA slots while they spin: 256^3 on 4 GPUs 17.1 -> 15.9 ms); env PAMG_BND_FIRST forces
-    fh.bnd_first = I.bnd_first >= 0 ? I.bnd_first : (ld.blk[op.which].nnz < 4000000 ? 1 : 0);
+    // they would hold resident-CTA slots while they spin: 256^3 on 4 GPUs 17.1 -> 15.9 ms)
+    fh.bnd_first = ld.blk[op.which].nnz < 4000000 ? 1 : 0;
     fh.skip = need ? ld.bnd[wsel].skip.p : nullptr;
     if (ld.bnd[wsel].n == 0) fh.skip = nullptr;
     if (with_pack) {
@@ -777,15 +761,14 @@ void Engine::enqueue_op(const OpSpec& op, const std::vector<const double*>& xin,
     // B200 (256^3): SELL Jacobi sweep 0.316 ms persistent vs 0.344 ms with one CTA per 8 slices.
     // Long rows (level >= 1, 30+ entries per row) lose 10 % that way: they keep one CTA per 8 slices.
     const double mean_nnz = m.nrows ? (double)m.nnz / m.nrows : 0.0;
-    // PAMG_SELL_PF bit mask: 1 = P, 2 = A with long rows, 4 = R (these then run persistent, which the prefetch needs)
-    const int pf_bit = op.which == PAMG_P_OO ? 1 : op.which == PAMG_R_OO ? 4 : (mean_nnz > 12.0 ? 2 : 0);
-    const bool prefetch = I.persistent && m.sell_rpt == 2 && (I.sell_pf & pf_bit) && !op.dot;
-    const bool use_vi4 = m.sell_vi4 && I.vi_variant == 3;
-    const bool bounded = I.persistent && m.sell_rpt && (mean_nnz <= 12.0 || prefetch || (use_vi4 && I.vi_persist_long));
+    const bool bounded = m.sell_rpt && mean_nnz <= 12.0;
+    const SpmvKernel kern = spmv_kernel(m, mean_nnz >= 48.0 && !op.dot);
     LaunchArgs L{0, bounded || op.dot, pd.stream, xin[i], epi[i], pd.st.p, fh, pd.partials.p, pd.rc, publish, op.slot};
     L.fh.v = xin[i];
     int n_main;
-    if (m.sell_rpt) {
+    if (m.sell_diag || m.sell_vi4) {
+      n_main = (m.nslices4 + BLOCK / 32 - 1) / (BLOCK / 32);
+    } else if (m.sell_rpt) {
       n_main = (m.nslices + BLOCK / 32 - 1) / (BLOCK / 32);
     } else if (m.stream) {
       n_main = m.nblocks;
@@ -793,29 +776,21 @@ void Engine::enqueue_op(const OpSpec& op, const std::vector<const double*>& xin,
       n_main = I.grid_for(m.nrows, (BLOCK / m.lanes) * 4);
     }
     L.grid = std::max(n_main, 1);
-    SellViView viv{};
-    if (m.sell_vi || use_vi4) viv = use_vi4 ? m.vi4view() : m.viview();
-    if (use_vi4 || m.sell_diag) L.grid = std::max((m.nslices4 + BLOCK / 32 - 1) / (BLOCK / 32), 1);
-    const bool long_rows = I.stream_long && mean_nnz >= 48.0 && !op.dot;  // CSR-stream phase B with 16 lanes per row (no DOT form)
-    if (m.sell_diag)
-      launch_sell_diag(op.mode, op.dot, m.diagview(), L);
-    else if (m.sell_rpt)
-      launch_sell(op.mode, op.dot, m.sell_rpt, (op.which == PAMG_P_OO && m.short_rows) ? I.p_kernel : 0, prefetch, m.slview(), L,
-                  (m.sell_vi || use_vi4) ? &viv : nullptr,
-                  use_vi4 ? (m.vi4_ib == 2 ? 4 : 3) + (I.vi_ahead && L.bounded ? 2 : 0) : (I.vi_variant == 3 ? 0 : I.vi_variant), I.vi_occ);  // blocks without the 128-row layout (sorted rows): two rows per lane
-    else if (m.stream)
-      launch_stream(op.mode, op.dot, long_rows, m.sview(), L);
-    else
-      launch_csr(op.mode, op.dot, m.lanes, m.view(), L);
+    switch (kern) {
+      case SpmvKernel::SellDiag: launch_sell_diag(op.mode, op.dot, m.diagview(), L); break;
+      case SpmvKernel::SellVi:
+      case SpmvKernel::SellVi16: launch_sell_vi4(op.mode, op.dot, m.vi4_ib, m.vi4view(), L); break;
+      case SpmvKernel::SellVi2: launch_sell_vi(op.mode, op.dot, m.viview(), L); break;
+      case SpmvKernel::Sell: launch_sell(op.mode, op.dot, m.sell_rpt, m.slview(), L); break;
+      case SpmvKernel::Stream:
+      case SpmvKernel::StreamLong: launch_stream(op.mode, op.dot, kern == SpmvKernel::StreamLong, m.sview(), L); break;
+      case SpmvKernel::Csr: launch_csr(op.mode, op.dot, m.lanes, m.view(), L); break;
+    }
     if (I.naming) {
       static const char* MODES[] = {"mul", "resid", "jacobi", "add", "restrict", "cheb"};
       static const char* OPS[] = {"A", "P", "R"};
-      // the name says which kernel ran: sell-vi = four rows per lane (one-byte indices), sell-vi16 = the same with two-byte
-      // indices, sell-vi2 = two rows per lane (sorted rows), stream-long = CSR-stream with 16 lanes per row in phase B
-      const char* vi_name = use_vi4 ? (m.vi4_ib == 2 ? "sell-vi16 " : "sell-vi ") : "sell-vi2 ";
-      I.names.push_back(std::string(m.sell_diag ? "sell-diag " : m.sell_rpt ? ((m.sell_vi || use_vi4) ? vi_name : "sell ") : m.stream ? (long_rows ? "stream-long " : "stream ") : "csr ") + MODES[op.mode] + (op.dot ? "+dot " : " ") +
-                        OPS[wsel] + std::to_string(l) + (I.tail_mode ? " tail" : "") + (fh.n_pack ? " +pack" : "") +
-                        (fh.n_bnd ? " +bnd" : ""));
+      I.names.push_back(std::string(SPMV_KERNEL_NAMES[(int)kern]) + " " + MODES[op.mode] + (op.dot ? "+dot " : " ") + OPS[wsel] +
+                        std::to_string(l) + (I.tail_mode ? " tail" : "") + (fh.n_pack ? " +pack" : "") + (fh.n_bnd ? " +bnd" : ""));
       I.naming = false;
       I.note_launch();
       I.naming = true;
@@ -889,11 +864,6 @@ Engine::Engine(Hierarchy* h, int nlocal, const int32_t* local_parts, const int32
   I.ipc.resize(I.nparts);
   I.have_ipc.assign(I.nparts, 0);
   const pamg_options& o = h->opts;
-  if (const char* pk = getenv("PAMG_P_KERNEL")) I.p_kernel = std::max(0, std::min(2, atoi(pk)));
-  if (const char* va = getenv("PAMG_VI_AHEAD")) I.vi_ahead = atoi(va) != 0;
-  if (const char* vp = getenv("PAMG_VI_PERSIST_LONG")) I.vi_persist_long = atoi(vp) != 0;
-  if (const char* vo = getenv("PAMG_VI_OCC")) I.vi_occ = std::max(0, std::min(2, atoi(vo)));
-  if (const char* vv = getenv("PAMG_VI_VARIANT")) I.vi_variant = std::max(0, std::min(3, atoi(vv)));
 
   // global decisions (identical in every process because the metadata is replicated)
   I.need_halo_A.assign(I.L, 0);
@@ -980,7 +950,7 @@ Engine::Engine(Hierarchy* h, int nlocal, const int32_t* local_parts, const int32
       for (int b = 0; b < 6; b += 2) {
         int lanes = 0;
         if (b == PAMG_A_OO && o.lanes_per_row > 0) lanes = o.lanes_per_row;
-        build_csr(pl.blk[b], false, ld.blk[b], lanes, o.spmv_format, o, b, b == PAMG_P_OO && I.p_kernel == 2 ? 1 : 0);
+        build_csr(pl.blk[b], false, ld.blk[b], lanes, o.spmv_format, o, b);
         build_bnd(pl.blk[b], pl.blk[b + 1], ld.bnd[b / 2]);
         max_blocks = std::max(max_blocks, ld.blk[b].nblocks);
         max_blocks = std::max(max_blocks, (std::max(ld.blk[b].nslices, ld.blk[b].nslices4) + BLOCK / 32 - 1) / (BLOCK / 32));
@@ -1108,14 +1078,10 @@ Engine::Engine(Hierarchy* h, int nlocal, const int32_t* local_parts, const int32
     if (!symmetric && !one_stream)
       throw CommError("halo plan: a part's send-neighbour set differs from its receive-neighbour set (structurally non-symmetric "
                       "operator); the peer-memory exchange protocol needs symmetric neighbour sets on multi-GPU layouts");
-    if (const char* pe = getenv("PAMG_PERSISTENT")) I.persistent = atoi(pe) != 0;
-    if (const char* le = getenv("PAMG_STREAM_LONG")) I.stream_long = atoi(le) != 0;
-    if (const char* pe2 = getenv("PAMG_SELL_PF")) I.sell_pf = atoi(pe2);
     {
       const char* fe = getenv("PAMG_FOLD_CHECK");
       I.fold_check = alone && (!fe || atoi(fe) != 0);
     }
-    if (const char* be = getenv("PAMG_BND_FIRST")) I.bnd_first = atoi(be) != 0 ? 1 : 0;
     const char* env = getenv("PAMG_FUSE_HALO");
     const bool want = env ? atoi(env) != 0 : o.fuse_halo != 0;
     I.fused_halo = want && alone && symmetric;

@@ -739,15 +739,9 @@ __device__ __forceinline__ double sv_get(const double2& v, int k) { return k ? v
 __device__ __forceinline__ int sv_get(const int32_t& v, int) { return v; }
 __device__ __forceinline__ int sv_get(const int2& v, int k) { return k ? v.y : v.x; }
 
-// U: entries of a row in flight per step; MINB: resident CTAs per SM the register budget must allow.  The defaults are the
-// production kernels (RPT = 2: 4 x 128-bit value loads + 4 x 64-bit column loads per thread and step, 3 CTAs/SM).  The
-// short-row instantiations <2, M_ADD, false, 2, 5> and <1, M_ADD, false, 4, 6> (48 / 40 registers) were built for the
-// prolongators (rows of 1-8 entries) and measured in round 2: no gain (profiles/r02_kernel_sweep.md), kept for the record.
-// PF > 0 (persistent launches only): while a warp works on slice i it requests the entries of the slice it will reach PF
-// iterations later into L2 (prefetch.global.L2, no register, no scoreboard), so that the dependent chain of a slice
-// -- extents -> columns/values -> gathers -> epilogue -- starts from L2 instead of HBM latency.  For the latency-bound
-// operators (prolongators: 1-8 entries per row, 37 % warps active, 56 % DRAM throughput in ncu).
-template <int RPT, int MODE, bool DOT, int U = (RPT == 1 ? 8 : 4), int MINB = (RPT == 1 ? 4 : 3), int PF = 0>
+// U: entries of a row in flight per step; MINB: resident CTAs per SM the register budget must allow (RPT = 2: 4 x 128-bit value
+// loads + 4 x 64-bit column loads per thread and step, 3 CTAs/SM).
+template <int RPT, int MODE, bool DOT, int U = (RPT == 1 ? 8 : 4), int MINB = (RPT == 1 ? 4 : 3)>
 __global__ void __launch_bounds__(BLOCK, MINB) k_spmv_sell(SellView A, const double* __restrict__ x, EpiArgs a, DevState* st,
                                                       FusedHalo fh, double* partials, RedCtx rc, int publish, int red_slot) {
   if (st->done) return;
@@ -773,14 +767,6 @@ __global__ void __launch_bounds__(BLOCK, MINB) k_spmv_sell(SellView A, const dou
   for (int sl = bid * wpb + (threadIdx.x >> 5); sl < A.nslices; sl += n_main * wpb) {
     const int o0 = A.slice_off[sl], w = A.slice_off[sl + 1] - o0;
     const int slot0 = sl * (32 * RPT) + lane * RPT;
-    int pf0 = 0, pfw = 0;  // extents of the slice to prefetch (requested here, used behind the entry loop)
-    if (PF > 0) {
-      const int sp = sl + PF * n_main * wpb;
-      if (sp < A.nslices) {
-        pf0 = A.slice_off[sp];
-        pfw = A.slice_off[sp + 1] - pf0;
-      }
-    }
     // Nothing but the row sums stays in registers across the entry loop: the epilogue operands, the skip
     // flags and (with a permutation) the row ids are prefetched into L1 here and loaded after the loop.
 #pragma unroll
@@ -824,14 +810,6 @@ __global__ void __launch_bounds__(BLOCK, MINB) k_spmv_sell(SellView A, const dou
           for (int k = 0; k < RPT; ++k) s[k] = __dadd_rn(s[k], __dmul_rn(sv_get(v[u], k), xv[u][k]));
         }
     }
-    if (PF > 0) {
-      const char* pv = reinterpret_cast<const char*>(reinterpret_cast<const V*>(A.val) + (size_t)pf0 * 32 + lane);
-      const char* pc = reinterpret_cast<const char*>(reinterpret_cast<const I*>(A.col) + (size_t)pf0 * 32 + lane);
-      for (int j = 0; j < pfw; ++j) {
-        asm volatile("prefetch.global.L2 [%0];" ::"l"(pv + (size_t)j * 32 * sizeof(V)));
-        asm volatile("prefetch.global.L2 [%0];" ::"l"(pc + (size_t)j * 32 * sizeof(I)));
-      }
-    }
     double contrib = 0.0;
 #pragma unroll
     for (int k = 0; k < RPT; ++k) {
@@ -855,7 +833,8 @@ __global__ void __launch_bounds__(BLOCK, MINB) k_spmv_sell(SellView A, const dou
 // dictionary (<= 2 KB) sits in shared memory; every product is __dmul_rn(dict[i], x[c]) with the ORIGINAL double, summed in
 // the same order, so results are bit-identical to the fp64-valued kernel.  Layout of the indices = layout of the columns
 // (entry j of slot q at (slice_off[sl] + j) * 64 + q): a lane reads its two rows' indices with one 16-bit load.
-// A kernel of its own so that the fp64-valued production instantiations keep their registers and load schedule.
+// A kernel of its own so that the fp64-valued production instantiations keep their registers and load schedule.  Blocks whose
+// rows were sorted (permuted) run this two-rows-per-lane kernel; unsorted ones run k_spmv_sell_vi4 below.
 // ---------------------------------------------------------------------------------------------
 struct SellViView {
   const int32_t* slice_off;
@@ -869,9 +848,11 @@ struct SellViView {
 };
 constexpr int VI_WIDE_MAX = 4096;  // 32 KB of shared memory per CTA
 
-template <int MODE, bool DOT, int U = 4, int MINB = 3>
-__global__ void __launch_bounds__(BLOCK, MINB) k_spmv_sell_vi(SellViView A, const double* __restrict__ x, EpiArgs a, DevState* st, FusedHalo fh,
+// 4 entries of a row in flight per step, 3 CTAs/SM
+template <int MODE, bool DOT>
+__global__ void __launch_bounds__(BLOCK, 3) k_spmv_sell_vi(SellViView A, const double* __restrict__ x, EpiArgs a, DevState* st, FusedHalo fh,
                                                          double* partials, RedCtx rc, int publish, int red_slot) {
+  constexpr int U = 4;
   if (st->done) return;
   trace_mark(st);
   const int n_main = (int)gridDim.x - fh.n_pack - fh.n_bnd;
@@ -951,143 +932,6 @@ __global__ void __launch_bounds__(BLOCK, MINB) k_spmv_sell_vi(SellViView A, cons
   if (DOT) dot_finish(s_acc[threadIdx.x], partials, st, &st->ticket[0], rc, publish, 0, red_slot);
 }
 
-// Software-pipelined form of the value-indexed kernel.  The plain form above is LATENCY bound once the bytes are halved
-// (256^3: 0.221 ms for 0.86 GB, 3.9 TB/s): per slice a warp walks three dependent memory latencies -- extents -> columns /
-// indices -> x gathers -- and 24 resident warps per SM cannot cover them.  Here a warp keeps the NEXT slice's columns and
-// indices in flight (registers) while it gathers, multiplies and stores the CURRENT one, and the extents are loaded two
-// slices ahead: one latency (the gathers) stays on the chain.  The first U = 8 entries of a row are pipelined (all of a
-// 7-point row, all of a prolongator row); longer slices finish in a plain tail loop.  Same products, same order, same bits.
-template <int MODE, bool DOT>
-__global__ void __launch_bounds__(BLOCK, 2) k_spmv_sell_vi_pipe(SellViView A, const double* __restrict__ x, EpiArgs a, DevState* st, FusedHalo fh,
-                                                              double* partials, RedCtx rc, int publish, int red_slot) {
-  constexpr int U = 8;
-  if (st->done) return;
-  trace_mark(st);
-  const int n_main = (int)gridDim.x - fh.n_pack - fh.n_bnd;
-  const int bid = (int)blockIdx.x - fh.n_pack - (fh.bnd_first ? fh.n_bnd : 0);
-  const int b0 = fh.n_pack + (fh.bnd_first ? 0 : n_main);  // first boundary CTA
-  if ((int)blockIdx.x < fh.n_pack || ((int)blockIdx.x >= b0 && (int)blockIdx.x < b0 + fh.n_bnd)) {  // halo roles
-    double racc = 0.0;
-    if ((int)blockIdx.x < fh.n_pack)
-      pack_role(fh, st, blockIdx.x);
-    else
-      racc = boundary_role<MODE, DOT>(fh, x, a, st, (int)blockIdx.x - b0);
-    if (DOT) dot_finish(racc, partials, st, &st->ticket[0], rc, publish, 0, red_slot);
-    return;
-  }
-  __shared__ double s_dict[256];
-  __shared__ double s_acc[DOT ? BLOCK : 1];
-  s_dict[threadIdx.x] = A.dict[threadIdx.x];  // BLOCK == 256
-  if (DOT) s_acc[threadIdx.x] = 0.0;
-  __syncthreads();
-  const int lane = threadIdx.x & 31;
-  const int wpb = BLOCK / 32;
-  const int stride = n_main * wpb;
-  const int2* __restrict__ colb = reinterpret_cast<const int2*>(A.col) + lane;
-  const unsigned short* __restrict__ idxb = reinterpret_cast<const unsigned short*>(A.vidx) + lane;
-  int sl = bid * wpb + (threadIdx.x >> 5);
-  // extents of the current slice and of the next one; columns / indices of the current slice
-  int o0 = 0, w = 0, o0n = 0, wn = 0;
-  if (sl < A.nslices) {
-    o0 = A.slice_off[sl];
-    w = A.slice_off[sl + 1] - o0;
-  }
-  if (sl + stride < A.nslices) {
-    o0n = A.slice_off[sl + stride];
-    wn = A.slice_off[sl + stride + 1] - o0n;
-  }
-  int2 c[U];
-  unsigned short iv[U];
-#pragma unroll
-  for (int u = 0; u < U; ++u) {
-    c[u] = make_int2(0, 0);
-    iv[u] = 0;
-    if (u < w) {
-      c[u] = __ldcs(colb + (size_t)(o0 + u) * 32);
-      iv[u] = __ldcs(idxb + (size_t)(o0 + u) * 32);
-    }
-  }
-  for (; sl < A.nslices; sl += stride) {
-    // ---- stage A: extents two slices ahead, columns / indices and epilogue prefetches of the next slice
-    int o0nn = 0, wnn = 0;
-    if (sl + 2 * stride < A.nslices) {
-      o0nn = A.slice_off[sl + 2 * stride];
-      wnn = A.slice_off[sl + 2 * stride + 1] - o0nn;
-    }
-    int2 cn[U];
-    unsigned short ivn[U];
-#pragma unroll
-    for (int u = 0; u < U; ++u) {
-      cn[u] = make_int2(0, 0);
-      ivn[u] = 0;
-      if (u < wn) {
-        cn[u] = __ldcs(colb + (size_t)(o0n + u) * 32);
-        ivn[u] = __ldcs(idxb + (size_t)(o0n + u) * 32);
-      }
-    }
-    const int slot0 = sl * 64 + lane * 2;
-    int r0 = slot0, r1 = slot0 + 1;
-    if (A.perm) {
-      if (r0 < A.nrows) r0 = A.perm[r0];
-      if (slot0 + 1 < A.nrows) r1 = A.perm[slot0 + 1];
-    }
-#pragma unroll
-    for (int k = 0; k < 2; ++k) {
-      const int r = k ? r1 : r0;
-      if (slot0 + k < A.nrows) {
-        if (fh.skip) asm volatile("prefetch.global.L1 [%0];" ::"l"(fh.skip + r));
-        if (MODE == M_RESID || MODE == M_JACOBI || MODE == M_ADD || MODE == M_CHEB) prefetch_l1(a.in0 + r);
-        if (MODE == M_JACOBI || MODE == M_CHEB || (MODE == M_RESTRICT && a.out2)) prefetch_l1(a.w + r);
-        if (MODE == M_CHEB && a.aux) prefetch_l1(a.aux + r);
-        if (DOT && a.dotv != a.in0) prefetch_l1(a.dotv + r);
-      }
-    }
-    // ---- stage B: the current slice
-    double xv[U][2];
-#pragma unroll
-    for (int u = 0; u < U; ++u)
-      if (u < w) {
-        xv[u][0] = x[c[u].x];
-        xv[u][1] = x[c[u].y];
-      }
-    double s0 = 0.0, s1 = 0.0;
-#pragma unroll
-    for (int u = 0; u < U; ++u)
-      if (u < w) {
-        s0 = __dadd_rn(s0, __dmul_rn(s_dict[iv[u] & 0xffu], xv[u][0]));
-        s1 = __dadd_rn(s1, __dmul_rn(s_dict[iv[u] >> 8], xv[u][1]));
-      }
-    for (int j = U; j < w; ++j) {  // rows longer than the pipelined part
-      const int2 cc = __ldcs(colb + (size_t)(o0 + j) * 32);
-      const unsigned short ii = __ldcs(idxb + (size_t)(o0 + j) * 32);
-      s0 = __dadd_rn(s0, __dmul_rn(s_dict[ii & 0xffu], x[cc.x]));
-      s1 = __dadd_rn(s1, __dmul_rn(s_dict[ii >> 8], x[cc.y]));
-    }
-    double contrib = 0.0;
-#pragma unroll
-    for (int k = 0; k < 2; ++k) {
-      const int r = k ? r1 : r0;
-      if (slot0 + k < A.nrows) {
-        if (fh.skip && fh.skip[r]) continue;
-        const double res = apply_epilogue<MODE, false>(a, r, k ? s1 : s0);
-        if (DOT) contrib += a.dotv[r] * res;
-      }
-    }
-    if (DOT) s_acc[threadIdx.x] += contrib;
-    // ---- rotate
-#pragma unroll
-    for (int u = 0; u < U; ++u) {
-      c[u] = cn[u];
-      iv[u] = ivn[u];
-    }
-    o0 = o0n;
-    w = wn;
-    o0n = o0nn;
-    wn = wnn;
-  }
-  if (DOT) dot_finish(s_acc[threadIdx.x], partials, st, &st->ticket[0], rc, publish, 0, red_slot);
-}
-
 // Value-indexed SELL with FOUR rows per lane, interleaved (formats.hpp sell_layout interleave = 4): slices of 128 rows; lane l owns
 // rows l, l + 32, l + 64, l + 96 of its slice.  ncu on the two-row form (256^3 SpMV, 0.21 ms for 0.83 GB): DRAM 48 %, L1 49 %,
 // 6 warps per scheduler of which 0.37 eligible, 14.7 long-scoreboard stalls per issue -- latency bound with too little in
@@ -1158,7 +1002,8 @@ __device__ __forceinline__ double rows4_epilogue(const EpiArgs& a, const FusedHa
 
 // AHEAD = 1: the extents of a warp's NEXT slice are loaded one iteration early and that slice's columns / indices are requested into L2
 // (prefetch.global.L2: no register, no scoreboard), which takes the extents latency off the per-slice chain and turns the column latency
-// from HBM into L2.
+// from HBM into L2.  The engine launches four instantiations, IB x bounded: a launch capped at one resident wave of persistent CTAs runs
+// AHEAD = 1, and its one-byte form U = 2 at 4 CTAs/SM (64 registers, no spill); the others run U = 4 at 3 CTAs/SM.
 template <int MODE, bool DOT, int IB = 1, int U = 4, int MINB = 3, int AHEAD = 0>
 __global__ void __launch_bounds__(BLOCK, MINB) k_spmv_sell_vi4(SellViView A, const double* __restrict__ x, EpiArgs a, DevState* st, FusedHalo fh,
                                                             double* partials, RedCtx rc, int publish, int red_slot) {

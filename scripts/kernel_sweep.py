@@ -41,35 +41,8 @@ CONFIGS = {
 }
 # A/B switches of the engine (read at device_init): name -> environment
 ENVS = {
-    "auto-r1": dict(PAMG_P_KERNEL="0", PAMG_STREAM_LONG="0"),       # round-1 behaviour
-    "auto-p0": dict(PAMG_P_KERNEL="0"),
-    "auto-p2": dict(PAMG_P_KERNEL="2"),
-    "auto-nosort": dict(PAMG_SELL_SORT_FILL="9"),
-    "auto-p2-nosort": dict(PAMG_P_KERNEL="2", PAMG_SELL_SORT_FILL="9"),
-    "auto-p1": dict(PAMG_P_KERNEL="1"),
-    "auto-nolong": dict(PAMG_STREAM_LONG="0"),
-    "auto-psig256": dict(PAMG_P_SIGMA="256"),
-    "auto-psig512": dict(PAMG_P_SIGMA="512"),
-    "auto-psig1024": dict(PAMG_P_SIGMA="1024"),
-    "auto-rsig4096": dict(PAMG_R_SIGMA="4096"),
-    "auto-sort1.1": dict(PAMG_SELL_SORT_FILL="1.1"),
     "auto-novi": dict(PAMG_VALUE_INDEX="0"),       # fp64 values everywhere (round-2 kernels)
-    "auto-vi1": dict(PAMG_VI_VARIANT="1"),         # value-indexed kernel <U 8, 2 CTAs/SM>
-    "auto-vi2": dict(PAMG_VI_VARIANT="2"),         # software-pipelined value-indexed kernel
-    "auto-vi3": dict(PAMG_VI_VARIANT="3"),         # four interleaved rows per lane
-    "auto-ahead": dict(PAMG_VI_AHEAD="1"),
-    "auto-noahead": dict(PAMG_VI_AHEAD="0"),
-    "auto-occ1": dict(PAMG_VI_OCC="1"),            # one-byte value-indexed kernel at 64 registers / 4 CTAs per SM (U = 4, spills)
-    "auto-occ2": dict(PAMG_VI_OCC="2"),            # ... U = 2, no spills
-    "auto-plong": dict(PAMG_VI_PERSIST_LONG="1"),  # level-1 A (value-indexed, 31 entries per row) as one resident wave + look-ahead
     "auto-vi8only": dict(PAMG_VALUE_INDEX="1"),    # one-byte indices only (no wide dictionaries on the coarse levels)
-    "auto-vi0": dict(PAMG_VI_VARIANT="0"),         # two rows per lane
-    "auto-vi-sorted": dict(PAMG_SELL_SORT_FILL="1.25"),
-    "auto-vi2-sorted": dict(PAMG_VI_VARIANT="2", PAMG_SELL_SORT_FILL="1.25"),
-    "auto-pf1": dict(PAMG_SELL_PF="1"),
-    "auto-pf3": dict(PAMG_SELL_PF="3"),
-    "auto-pf5": dict(PAMG_SELL_PF="5"),
-    "auto-pf7": dict(PAMG_SELL_PF="7"),
 }
 for k in ENVS:
     CONFIGS[k] = dict(spmv_format=L.FORMAT_AUTO)
@@ -79,8 +52,7 @@ else:
     CONFIGS = {k: v for k, v in CONFIGS.items() if k not in ENVS}
 res = {}
 for name, kw in CONFIGS.items():
-    for k in ("PAMG_VI_OCC", "PAMG_VI_PERSIST_LONG", "PAMG_VI_AHEAD", "PAMG_VALUE_INDEX", "PAMG_VI_VARIANT", "PAMG_P_KERNEL", "PAMG_SELL_SORT_FILL", "PAMG_STREAM_LONG", "PAMG_P_SIGMA", "PAMG_R_SIGMA", "PAMG_SELL_PF"):
-        os.environ.pop(k, None)
+    os.environ.pop("PAMG_VALUE_INDEX", None)
     os.environ.update(ENVS.get(name, {}))
     c.set_kernel_options(**kw)
     c.device_init()
