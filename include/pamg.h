@@ -286,6 +286,27 @@ int pamg_fcg(pamg_ctx* c, const double* const* b, double* const* x, double rtol,
 int pamg_fgmres(pamg_ctx* c, const double* const* b, double* const* x, double rtol, int32_t maxiter, int32_t restart,
                 int32_t precond, int32_t* iters, double* resid_hist);
 
+/* ---- several right-hand sides with one matrix (k solve! calls sharing one setup) ----------
+ * The multi calls run k independent single-vector computations, sharing one launch per operation where the block's kernel has a
+ * k-wide form (value-indexed and implied-column SELL).  Column j of every result is bit-identical to the single-vector call on
+ * column j run with fuse_halo = 0 (which is what one GPU runs anyway).  Vectors: k * nparts pointers, column j of part p at
+ * [j * nparts + p] (NULL for parts that are not local).  Multi calls always exchange halos with separate launches. */
+#define PAMG_MAX_RHS 8
+/* columns of device state the next pamg_device_init allocates (1..PAMG_MAX_RHS, default 1); every process of a job must set the
+ * same value (pamg_comm_connect refuses a mismatch) */
+int pamg_set_rhs_capacity(pamg_ctx* c, int32_t kmax);
+int pamg_spmv_multi(pamg_ctx* c, int32_t level, int32_t k, const double* const* x, double* const* y);
+int pamg_vcycle_multi(pamg_ctx* c, int32_t k, const double* const* b, double* const* x);
+/* mode 0 CG, 1 AMG-PCG, 2 flexible AMG-PCG; each column has its own scalars, history, count and convergence decision, and a
+ * converged column stays frozen while the others continue.  iters[k], converged[k] (may be NULL); resid_hist k x (maxiter + 1),
+ * row j = column j, may be NULL.  PAMG_OK when every column converged, else PAMG_ERR_NOTCONV.  pamg_stats: iters = max over
+ * columns, r0_norm / r_norm of column 0. */
+int pamg_pcg_multi(pamg_ctx* c, int32_t k, const double* const* b, double* const* x, double rtol, int32_t maxiter,
+                   int32_t mode, int32_t* iters, int32_t* converged, double* resid_hist);
+/* pamg_time_kernel over k columns (kinds 0, 1, 2, 3, 6, 7): the time of the launches that serve all k columns at once, for a
+ * comparison of a k-wide launch with k single ones */
+int pamg_time_kernel_multi(pamg_ctx* c, int32_t k, int32_t kind, int32_t level, int32_t reps, int32_t flush_l2, float* ms_out);
+
 /* ---- device-resident benchmarking hooks (inputs already in HBM) ------------------------
  * pamg_load_rhs copies b to the device once; pamg_pcg_resident re-solves from x=0 with the
  * resident b and leaves x on the device (pamg_read_solution fetches it). */

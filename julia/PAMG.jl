@@ -96,7 +96,8 @@ end
 # nullspace: optional n x k matrix (global row order) of near-nullspace vectors, e.g. the 6 rigid-body modes from
 # `nullspace_linear_elasticity`; block_size: DOFs per node (3 for 3-D elasticity).
 # devices: GPU id per LOCAL part (debug backend default 0:np-1; MPI backend default [local rank of this process]).
-function setup(A::PSparseMatrix; devices = nothing, opts::Options = default_options(), nullspace = nothing, block_size = 1)
+function setup(A::PSparseMatrix; devices = nothing, opts::Options = default_options(), nullspace = nothing, block_size = 1,
+               rhs_capacity = 1)
     rows, cols = partition(axes(A, 1)), partition(axes(A, 2))
     np = length(rows)
     ranks = linear_indices(rows)
@@ -126,6 +127,7 @@ function setup(A::PSparseMatrix; devices = nothing, opts::Options = default_opti
                              ctx, block_size, size(nullspace, 2), B))
         end
         check(ctx, ccall((:pamg_setup, lib), Cint, (Ptr{Cvoid}, Ref{Options}), ctx, Ref(opts)))
+        check(ctx, ccall((:pamg_set_rhs_capacity, lib), Cint, (Ptr{Cvoid}, Int32), ctx, rhs_capacity))
         locals = mpi ? [rank] : collect(1:np)
         devs = devices === nothing ? (mpi ? Int32[parse(Int, get(ENV, "LOCAL_RANK", "0"))] : Int32.(0:np-1)) : Int32.(devices)
         check(ctx, ccall((:pamg_device_init, lib), Cint, (Ptr{Cvoid}, Int32, Ptr{Int32}, Ptr{Int32}),
@@ -205,6 +207,23 @@ function solve_gmres!(x::PVector, S::Setup, b::PVector; rtol = 1e-8, maxiter = 2
     st == -5 || check(S.ctx, st)
     wait(consistent!(x))
     (iterations = Int(iters[]), converged = st == 0, residuals = hist[1:iters[]+1])   # residuals: the Arnoldi estimates
+end
+
+# k solve! calls sharing one setup (pamg_pcg_multi; setup(...; rhs_capacity >= k)): xs[j] and the j-th result tuple are
+# bit-identical to solve!(xs[j], S, bs[j]); mode 0 CG, 1 AMG-PCG, 2 flexible AMG-PCG
+function solve_multi!(xs::Vector{<:PVector}, S::Setup, bs::Vector{<:PVector}; rtol = 1e-8, maxiter = 200, mode = 1)
+    k = length(bs)
+    iters = zeros(Int32, k)
+    conv = zeros(Int32, k)
+    hist = zeros(Float64, maxiter + 1, k)          # column j = row j of the C k x (maxiter + 1) array
+    bp = reduce(vcat, [own_ptrs(b, S) for b in bs])
+    xp = reduce(vcat, [own_ptrs(x, S) for x in xs])
+    st = GC.@preserve bs xs ccall((:pamg_pcg_multi, lib), Cint,
+        (Ptr{Cvoid}, Int32, Ptr{Ptr{Float64}}, Ptr{Ptr{Float64}}, Float64, Int32, Int32, Ptr{Int32}, Ptr{Int32}, Ptr{Float64}),
+        S.ctx, k, bp, xp, rtol, maxiter, mode, iters, conv, hist)
+    st == -5 || check(S.ctx, st)
+    foreach(x -> wait(consistent!(x)), xs)
+    [(iterations = Int(iters[j]), converged = conv[j] == 1, residuals = hist[1:iters[j]+1, j]) for j in 1:k]
 end
 
 function vcycle!(z::PVector, S::Setup, r::PVector)

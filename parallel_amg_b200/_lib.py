@@ -122,6 +122,11 @@ PROTOTYPES = {
     "pamg_trace_enable": [_ctx, C.c_int32],
     "pamg_trace_read": [_ctx, C.c_int32, _P(C.c_uint64), C.c_int32, _i32p],
     "pamg_trace_names": [_ctx, C.c_char_p, C.c_int32],
+    "pamg_set_rhs_capacity": [_ctx, C.c_int32],
+    "pamg_spmv_multi": [_ctx, C.c_int32, C.c_int32, _vecs, _vecs],
+    "pamg_vcycle_multi": [_ctx, C.c_int32, _vecs, _vecs],
+    "pamg_time_kernel_multi": [_ctx, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P(C.c_float)],
+    "pamg_pcg_multi": [_ctx, C.c_int32, _vecs, _vecs, C.c_double, C.c_int32, C.c_int32, _i32p, _i32p, _f64p],
 }
 _RESTYPE = {"pamg_set_num_threads": None, "pamg_default_options": None, "pamg_destroy": None, "pamg_last_error": C.c_char_p,
             "pamg_comm_handle_bytes": C.c_int32}
@@ -460,6 +465,17 @@ class Context:
             out[p] = _ptr(a, C.c_double)
         return out, keep
 
+    def _vecs_multi(self, cols, writable=False):
+        """k columns, each a per-part list as pcg() takes -> double*[k * nparts], column j of part p at [j * nparts + p]"""
+        out = (_f64p * (len(cols) * self.nparts))()
+        keep = []
+        for j, col in enumerate(cols):
+            ptrs, k = self._vecs(col, writable=writable)
+            keep.append((ptrs, k))
+            for p in range(self.nparts):
+                out[j * self.nparts + p] = ptrs[p]
+        return out, keep
+
     def _new_own(self, level):
         return [np.zeros(self.level_info(level, p).n_own) if p in self.local_parts else None
                 for p in range(self.nparts)]
@@ -551,6 +567,47 @@ class Context:
         st = self._ck(self.lib.pamg_fgmres(self._h, bp, xp, float(rtol), int(maxiter), int(restart), int(bool(precond)),
                                            C.byref(it), _ptr(hist, C.c_double)), allow=(ERR_NOTCONV,))
         return x, it.value, hist[:it.value + 1].copy(), st == OK
+
+    # ---- several right-hand sides (k solve! calls sharing one setup) ----
+    def set_rhs_capacity(self, kmax):
+        """columns of device state the next device_init allocates (1..8)"""
+        self._ck(self.lib.pamg_set_rhs_capacity(self._h, int(kmax)))
+
+    def spmv_multi(self, level, X):
+        """X: list of k columns, each a per-part list as spmv() takes; returns the k results (column j == spmv(level, X[j]))"""
+        Y = [self._new_own(level) for _ in X]
+        xp, k1 = self._vecs_multi(X)
+        yp, k2 = self._vecs_multi(Y, writable=True)
+        self._ck(self.lib.pamg_spmv_multi(self._h, int(level), len(X), xp, yp))
+        return Y
+
+    def vcycle_multi(self, B):
+        """one cycle from x = 0 per column; column j == vcycle(B[j])"""
+        X = [self._new_own(0) for _ in B]
+        bp, k1 = self._vecs_multi(B)
+        xp, k2 = self._vecs_multi(X, writable=True)
+        self._ck(self.lib.pamg_vcycle_multi(self._h, len(B), bp, xp))
+        return X
+
+    def pcg_multi(self, B, rtol=1e-8, maxiter=200, mode=1):
+        """k independent solves (mode 0 CG, 1 AMG-PCG, 2 flexible); per column the results tuple of pcg():
+        list of (x, iters, hist, converged), column j == pcg(B[j]) (mode 0/1) or fcg(B[j]) (mode 2)"""
+        k = len(B)
+        X = [self._new_own(0) for _ in B]
+        bp, k1 = self._vecs_multi(B)
+        xp, k2 = self._vecs_multi(X, writable=True)
+        it = np.zeros(k, np.int32)
+        conv = np.zeros(k, np.int32)
+        hist = np.zeros((k, maxiter + 1))
+        self._ck(self.lib.pamg_pcg_multi(self._h, k, bp, xp, float(rtol), int(maxiter), int(mode), _ptr(it, C.c_int32),
+                                         _ptr(conv, C.c_int32), _ptr(hist, C.c_double)), allow=(ERR_NOTCONV,))
+        return [(X[j], int(it[j]), hist[j, :it[j] + 1].copy(), bool(conv[j])) for j in range(k)]
+
+    def time_kernel_multi(self, k, kind, level, reps=10, flush_l2=True):
+        """time_kernel over k columns: one k-wide launch where the block has one, else k single launches"""
+        ms = np.zeros(reps, np.float32)
+        self._ck(self.lib.pamg_time_kernel_multi(self._h, int(k), kind, level, reps, int(flush_l2), _ptr(ms, C.c_float)))
+        return ms
 
     def load_rhs(self, b):
         bp, k1 = self._vecs(b)

@@ -32,6 +32,7 @@ struct pamg_ctx {
   Hierarchy h;
   int32_t ext_levels = 0;
   std::unique_ptr<Engine> eng;
+  int32_t rhs_capacity = 1;  // for the next pamg_device_init
   std::string err;
 };
 
@@ -78,6 +79,15 @@ const PartLevel& part_level(pamg_ctx* c, int32_t level, int32_t part) {
 Engine& engine(pamg_ctx* c) {
   if (!c->eng) throw std::runtime_error("device not initialised: call pamg_device_init");
   return *c->eng;
+}
+
+// the device state of a multi-column call: initialised with the capacity now set
+Engine& engine_multi(pamg_ctx* c, int32_t k) {
+  need(k >= 1 && k <= c->rhs_capacity, "k must be in 1..capacity (pamg_set_rhs_capacity)");
+  Engine& e = engine(c);
+  need(e.rhs_capacity() == c->rhs_capacity,
+       "the right-hand-side capacity changed after pamg_device_init: call pamg_device_init again before a multi call");
+  return e;
 }
 
 void merge_staged(pamg_ctx* c) {
@@ -695,7 +705,15 @@ int pamg_device_init(pamg_ctx* c, int32_t nlocal, const int32_t* local_parts, co
     need(c->h.ready, "hierarchy not set up");
     need(nlocal >= 1 && nlocal <= c->nparts && local_parts, "bad local part list");
     c->eng.reset();
-    c->eng.reset(new Engine(&c->h, nlocal, local_parts, device_ids));
+    c->eng.reset(new Engine(&c->h, nlocal, local_parts, device_ids, c->rhs_capacity));
+    return PAMG_OK;
+  });
+}
+
+int pamg_set_rhs_capacity(pamg_ctx* c, int32_t kmax) {
+  return guard(c, [&] {
+    need(kmax >= 1 && kmax <= PAMG_MAX_RHS, "right-hand-side capacity must be in 1..PAMG_MAX_RHS (8)");
+    c->rhs_capacity = kmax;
     return PAMG_OK;
   });
 }
@@ -807,6 +825,34 @@ int pamg_fcg(pamg_ctx* c, const double* const* b, double* const* x, double rtol,
   return guard(c, [&] {
     need(b && x && rtol >= 0.0 && maxiter >= 0, "bad arguments");
     return engine(c).pcg(b, x, rtol, maxiter, 2, iters, resid_hist);
+  });
+}
+int pamg_spmv_multi(pamg_ctx* c, int32_t level, int32_t k, const double* const* x, double* const* y) {
+  return guard(c, [&] {
+    need(x && y, "null vectors");
+    engine_multi(c, k).spmv_multi(level, k, x, y);
+    return PAMG_OK;
+  });
+}
+int pamg_vcycle_multi(pamg_ctx* c, int32_t k, const double* const* b, double* const* x) {
+  return guard(c, [&] {
+    need(b && x, "null vectors");
+    engine_multi(c, k).vcycle_multi(k, b, x);
+    return PAMG_OK;
+  });
+}
+int pamg_pcg_multi(pamg_ctx* c, int32_t k, const double* const* b, double* const* x, double rtol, int32_t maxiter, int32_t mode,
+                   int32_t* iters, int32_t* converged, double* resid_hist) {
+  return guard(c, [&] {
+    need(b && x && rtol >= 0.0 && maxiter >= 0 && mode >= 0 && mode <= 2, "bad arguments");
+    return engine_multi(c, k).pcg_multi(k, b, x, rtol, maxiter, mode, iters, converged, resid_hist);
+  });
+}
+int pamg_time_kernel_multi(pamg_ctx* c, int32_t k, int32_t kind, int32_t level, int32_t reps, int32_t flush_l2, float* ms_out) {
+  return guard(c, [&] {
+    need(reps >= 1 && ms_out, "bad arguments");
+    engine_multi(c, k).time_kernel_multi(k, kind, level, reps, flush_l2 != 0, ms_out);
+    return PAMG_OK;
   });
 }
 int pamg_fgmres(pamg_ctx* c, const double* const* b, double* const* x, double rtol, int32_t maxiter, int32_t restart,

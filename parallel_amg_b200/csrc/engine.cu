@@ -63,6 +63,18 @@ struct DBuf {
   void upload(const std::vector<T>& v) { upload(v.data(), v.size()); }
 };
 
+// the buffer of the column a multi-column call is working on (Engine::Impl::bind); column 0 outside such calls
+template <class T>
+struct DView {
+  T* p = nullptr;
+  size_t n = 0;
+  DView& operator=(const DBuf<T>& b) {
+    p = b.p;
+    n = b.n;
+    return *this;
+  }
+};
+
 size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 struct DevCsr {
@@ -363,6 +375,9 @@ void build_csr(const LocalCsr& m, bool compress, DevCsr& d, int lanes_override, 
 struct ArenaLayout {
   std::vector<size_t> ghost, flags, asm_stage, asm_flags;
   size_t coarse = 0, coarse_flags = 0, red = 0, red_flags = 0, total = 0;
+  // a part's arena holds kmax copies of this layout, column j at j * col_stride; the word at `capacity` (behind column 0's
+  // layout) is the kmax its owner allocated, checked by every process at connect
+  size_t capacity = 0, col_stride = 0;
 };
 
 // First level of the replicated coarse tail: levels [tail, L) are merged over all parts and run by every
@@ -398,6 +413,8 @@ ArenaLayout arena_layout(const Hierarchy& h, int part) {
   a.red = take(2 * (size_t)h.nparts * RED_W * sizeof(double));
   a.red_flags = take((size_t)h.nparts * sizeof(uint32_t));
   a.total = off;
+  a.capacity = take(sizeof(int32_t));
+  a.col_stride = off;
   return a;
 }
 
@@ -407,9 +424,19 @@ struct LevelDev {
   DevBnd bnd[3];      // boundary rows of A, P, R
   DBuf<double> w;     // smoother weight: w/a_ii (Jacobi), 1/l1-diag (l1), 1/(theta a_ii) (Chebyshev zero-guess step)
   DBuf<double> dinv;  // 1/a_ii (Chebyshev)
-  DBuf<double> x, x2, b, t, d, d2;
+  // per right-hand side: work vectors and the halo staging of that column's arena copy
+  struct Col {
+    DBuf<double> x, x2, b, t, d, d2;
+    double* xstart = nullptr;
+    HaloRecv hr{};
+    DBuf<SendNbr> send_nbrs;
+  };
+  std::unique_ptr<Col[]> cols;
+  // Views of the BOUND column's buffers (Engine::Impl::bind).  Read them only after selecting the column: Impl::S(slot) (or LV(slot,
+  // l)) binds the slot's column; Impl::P(i) does not, so after P(i) these still show whichever column was bound last.
+  DView<double> x, x2, b, t, d, d2;
   DBuf<int32_t> send_idx;
-  DBuf<SendNbr> send_nbrs;
+  DView<SendNbr> send_nbrs;
   int n_send = 0, n_send_nbrs = 0, n_recv_nbrs = 0;
   HaloRecv hr{};
   // assemble! plan
@@ -434,22 +461,32 @@ struct PartDev {
   std::vector<std::unique_ptr<LevelDev>> tlev;  // merged (replicated) levels [tail_level, L), null below
   ArenaLayout lay;
   char* arena = nullptr;
-  DBuf<DevState> st;
-  DBuf<double> partials;
-  int partials_cap = 0;
-  DBuf<RedPub> red_pubs;
+  // per right-hand side: solve state, Krylov vectors and the all-reduce / coarse-gather wiring of that column's arena copy
+  struct Col {
+    DBuf<DevState> st;
+    DBuf<double> partials, xsol, p, q, bsave, hist, rprev;  // rprev: r_k of flexible CG (allocated on first use)
+    int hist_cap = 0;
+    DBuf<RedPub> red_pubs;
+    RedCtx rc{};
+    DBuf<CoarsePub> coarse_pubs;
+  };
+  std::unique_ptr<Col[]> cols;
+  // views of the BOUND column's state: valid for a slot only after Impl::S(slot) (see LevelDev)
+  char* carena = nullptr;
+  DView<DevState> st;
+  DView<double> partials, xsol, p, q, bsave, hist, rprev;
   RedCtx rc{};
-  DBuf<CoarsePub> coarse_pubs;
+  DView<CoarsePub> coarse_pubs;
+  int partials_cap = 0;
   DBuf<double> inv;
   DBuf<int64_t> own_gid_T, ghost_gid_T;
-  DBuf<double> xsol, p, q, bsave, hist, scratch4, rprev;  // rprev: r_k of flexible CG (allocated on first use)
+  DBuf<double> scratch4;
   DBuf<double> io_local;  // own+ghost staging for consistent!/assemble!
   DBuf<double> gm_basis;  // FGMRES: V_0..V_m then Z_0..Z_{m-1}, own length each (allocated on first use)
   DBuf<double> gm_h;      // FGMRES: one Hessenberg column (m + 2 doubles), written by k_gs_sub / k_gs_norm
   int gm_restart = 0;
   bool gm_precond = false;
   DBuf<unsigned long long> trace;
-  int hist_cap = 0;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
 };
 
@@ -459,7 +496,7 @@ struct Engine::Impl {
   int tail_level = 0;      // levels >= tail_level run replicated (merged over all parts) on every GPU
   bool tail_mode = false;  // enqueue_* address the merged levels
   LevelDev& LV(PartDev& pd, int l) { return tail_mode ? *pd.tlev[l] : *pd.lev[l]; }
-  LevelDev& LV(size_t i, int l) { return LV(*parts[i], l); }
+  LevelDev& LV(size_t s, int l) { return LV(S(s), l); }  // slot s (binds its column)
   std::vector<std::unique_ptr<PartDev>> parts;         // local parts
   std::vector<int> local_index;                        // part -> index in parts or -1
   std::vector<char*> arena_of;                         // part -> arena base as seen from this process
@@ -475,15 +512,66 @@ struct Engine::Impl {
   // exchange needed per level/operator (decided on global metadata so every part agrees)
   std::vector<char> need_halo_A, need_halo_R, need_halo_P;
   // graphs (one per distinct stream)
-  std::vector<cudaGraphExec_t> g_iter, g_vcycle;
+  std::vector<cudaGraphExec_t> g_iter, g_vcycle, g_vcycle_multi;
   std::vector<cudaStream_t> g_streams;
-  int64_t g_iter_nodes = 0, g_vcycle_nodes = 0;
+  int64_t g_iter_nodes = 0, g_vcycle_nodes = 0, g_vcycle_multi_nodes = 0;
   int g_iter_mode = -1;  // mode the iteration graph was captured for: 0 plain CG, 1 PCG, 2 flexible PCG
+  int g_iter_k = 0;      // columns it was captured for (0: the single-column solve), likewise for g_vcycle_multi
+  int g_vcycle_multi_k = 0;
   double* flush_buf = nullptr;
   size_t flush_n = 0;
   pamg_stats stats{};
-  HostStat* hstat = nullptr;  // pinned, device-mapped ring written by k_check of the first local part
+  HostStat* hstat_base = nullptr;  // pinned, device-mapped rings (HS_RING per column) written by k_check of the first local part
+  HostStat* hstat = nullptr;       // the bound column's ring
   bool rhs_loaded = false;
+  // right-hand sides: kmax columns of per-solve state exist; `cols` are the ones the enqueue_* functions run over (slot s = column
+  // cols[s / nparts_local], part s % nparts_local), {0} outside multi-column calls, which also set `multi` (split halo launches)
+  int kmax = 1;
+  std::vector<int> cols{0};
+  bool multi = false;
+  int bound = -1;
+  size_t nslots() const { return cols.size() * parts.size(); }
+  int col_of(size_t s) const { return cols[s / parts.size()]; }
+  PartDev& S(size_t s) {
+    bind(col_of(s));
+    return *parts[s % parts.size()];
+  }
+  // point the views of every part and level at column c's buffers
+  void bind(int c, bool force = false) {
+    if (c == bound && !force) return;
+    bound = c;
+    auto bind_level = [c](LevelDev& ld) {
+      LevelDev::Col& lc = ld.cols[c];
+      ld.x = lc.x;
+      ld.x2 = lc.x2;
+      ld.b = lc.b;
+      ld.t = lc.t;
+      ld.d = lc.d;
+      ld.d2 = lc.d2;
+      ld.xstart = lc.xstart;
+      ld.hr = lc.hr;
+      ld.send_nbrs = lc.send_nbrs;
+    };
+    for (auto& up : parts) {
+      PartDev& pd = *up;
+      PartDev::Col& pc = pd.cols[c];
+      pd.carena = pd.arena + (size_t)c * pd.lay.col_stride;
+      pd.st = pc.st;
+      pd.partials = pc.partials;
+      pd.xsol = pc.xsol;
+      pd.p = pc.p;
+      pd.q = pc.q;
+      pd.bsave = pc.bsave;
+      pd.hist = pc.hist;
+      pd.rprev = pc.rprev;
+      pd.rc = pc.rc;
+      pd.coarse_pubs = pc.coarse_pubs;
+      for (auto& ld : pd.lev) bind_level(*ld);
+      for (auto& ld : pd.tlev)
+        if (ld) bind_level(*ld);
+    }
+    hstat = hstat_base + (size_t)c * HS_RING;
+  }
 
   ~Impl();
   PartDev& P(int i) { return *parts[i]; }
@@ -510,7 +598,8 @@ struct Engine::Impl {
 Engine::Impl::~Impl() {
   for (auto g : g_iter) cudaGraphExecDestroy(g);
   for (auto g : g_vcycle) cudaGraphExecDestroy(g);
-  if (hstat) cudaFreeHost(hstat);
+  for (auto g : g_vcycle_multi) cudaGraphExecDestroy(g);
+  if (hstat_base) cudaFreeHost(hstat_base);
   for (auto& up : parts) {
     cudaSetDevice(up->device);
     if (up->ev0) cudaEventDestroy(up->ev0);
@@ -693,6 +782,46 @@ void launch_sell_diag(int mode, bool dot, const SellDiagView& A, const LaunchArg
   });
 }
 
+// k-wide form of the block's kernel for K columns (multi-column calls, main role only).  The grid is the one the single kernel would
+// get for this launch, so every column sees the same slices per CTA and the same fused-dot partials as on its own.
+//
+// Width of the launch for the next g (>= 1) columns of one block: 2 or 4 (one k-wide launch; g = 3 runs K = 4 with one column absent)
+// or 1 (the single kernel for one column).  Chosen per block class from the B200 measurements of DESIGN §4.9
+// (profiles/r05_multi_rhs.json; L2 flushed, k-wide launch against k single launches): the k-wide forms hold 2 CTAs per SM against the
+// single kernels' 3-4, and where that loses the class keeps its single launches:
+//   implied-column A (k_spmv_sell_diag): K = 2 loses in every mode (1.17x the time of two single launches for the Jacobi sweep); K = 4
+//     wins for the Jacobi sweep (0.93x), the residual and the SpMV + p.q (0.83x) but loses for the Jacobi sweep + r.z (1.07x);
+//   value-indexed P (prolongation, 1-8 entries per row): 1.04-1.24x at K = 2 and 4 on the Poisson and jump-coefficient hierarchies;
+//   value-indexed A and R (elasticity A0, level-1 A, restriction): 0.61-0.97x at K = 2 and 4 in every mode measured.
+int multi_width(SpmvKernel k, int which, int mode, bool dot, int g) {
+  if (g < 2) return 1;
+  if (k == SpmvKernel::SellDiag) return (g >= 3 && !(mode == M_JACOBI && dot)) ? 4 : 1;
+  if ((k == SpmvKernel::SellVi || k == SpmvKernel::SellVi16) && which != PAMG_P_OO) return g == 2 ? 2 : 4;
+  return 1;
+}
+
+template <int K>
+void launch_multi(SpmvKernel kern, const DevCsr& m, int mode, bool dot, const LaunchArgs& L, const MultiCols<K>& mc) {
+  dispatch_mode(mode, dot, [&](auto md, auto dt) {
+    constexpr int MD = decltype(md)::value;
+    constexpr bool DT = decltype(dt)::value;
+    if (kern == SpmvKernel::SellDiag) {
+      const int grid = main_grid(L, (const void*)k_spmv_sell_diag<MD, DT>);
+      k_spmv_sell_diag_multi<MD, DT, K><<<grid, BLOCK, 0, L.s>>>(m.diagview(), mc, L.fh, L.publish, L.slot);
+      return;
+    }
+    using Kern = void (*)(SellViView, const double*, EpiArgs, DevState*, FusedHalo, double*, RedCtx, int, int);
+    const Kern by_ib_bounded[2][2] = {{k_spmv_sell_vi4<MD, DT, 1>, k_spmv_sell_vi4<MD, DT, 1, 2, 4, 1>},
+                                      {k_spmv_sell_vi4<MD, DT, 2>, k_spmv_sell_vi4<MD, DT, 2, 4, 3, 1>}};
+    const size_t dyn = (size_t)m.ndict * sizeof(double);
+    const int grid = main_grid(L, (const void*)by_ib_bounded[m.vi4_ib == 2][L.bounded], dyn);
+    if (m.vi4_ib == 2)
+      k_spmv_sell_vi4_multi<MD, DT, 2, K><<<grid, BLOCK, dyn, L.s>>>(m.vi4view(), mc, L.fh, L.publish, L.slot);
+    else
+      k_spmv_sell_vi4_multi<MD, DT, 1, K><<<grid, BLOCK, dyn, L.s>>>(m.vi4view(), mc, L.fh, L.publish, L.slot);
+  });
+}
+
 void launch_boundary(int mode, bool dot, const LaunchArgs& L) {
   dispatch_mode(mode, dot, [&](auto md, auto dt) {
     k_boundary<decltype(md)::value, decltype(dt)::value><<<L.grid, BLOCK, 0, L.s>>>(L.x, L.a, L.st, L.fh, L.partials, L.rc, L.slot);
@@ -723,8 +852,9 @@ void Engine::enqueue_op(const OpSpec& op, const std::vector<const double*>& xin,
     need = I.need_halo_P[l];
   if (I.tail_mode) need = false;  // merged levels: every column is an own column
   const bool exchange = need && !op.coarse_ghosts_local;
-  const bool fused = I.fused_halo;
+  const bool fused = I.fused_halo && !I.multi;  // multi-column calls: split launches on every layout
   const int wsel = op.which / 2;  // 0 A, 1 P, 2 R
+  const size_t np = I.parts.size(), ns = I.nslots();
 
   auto halo_args = [&](PartDev& pd, bool with_pack, bool with_bnd) {
     LevelDev& ld = I.LV(pd, l);
@@ -754,7 +884,18 @@ void Engine::enqueue_op(const OpSpec& op, const std::vector<const double*>& xin,
     }
     return fh;
   };
-  auto launch_main = [&](PartDev& pd, size_t i, const FusedHalo& fh, int publish) {
+  auto launch_name = [&](SpmvKernel kern, int width, const FusedHalo& fh) {
+    static const char* MODES[] = {"mul", "resid", "jacobi", "add", "restrict", "cheb"};
+    static const char* OPS[] = {"A", "P", "R"};
+    I.names.push_back(std::string(SPMV_KERNEL_NAMES[(int)kern]) + (width > 1 ? " x" + std::to_string(width) : "") + " " + MODES[op.mode] +
+                      (op.dot ? "+dot " : " ") + OPS[wsel] + std::to_string(l) + (I.tail_mode ? " tail" : "") + (fh.n_pack ? " +pack" : "") +
+                      (fh.n_bnd ? " +bnd" : ""));
+    I.naming = false;
+    I.note_launch();
+    I.naming = true;
+  };
+  // the launch arguments of slot s (its column must be bound)
+  auto main_args = [&](PartDev& pd, size_t s, const FusedHalo& fh, int publish, SpmvKernel* kern) {
     LevelDev& ld = I.LV(pd, l);
     const DevCsr& m = ld.blk[op.which];
     // persistent main role: one resident wave of CTAs striding over the slices / row blocks.  Measured on
@@ -762,9 +903,9 @@ void Engine::enqueue_op(const OpSpec& op, const std::vector<const double*>& xin,
     // Long rows (level >= 1, 30+ entries per row) lose 10 % that way: they keep one CTA per 8 slices.
     const double mean_nnz = m.nrows ? (double)m.nnz / m.nrows : 0.0;
     const bool bounded = m.sell_rpt && mean_nnz <= 12.0;
-    const SpmvKernel kern = spmv_kernel(m, mean_nnz >= 48.0 && !op.dot);
-    LaunchArgs L{0, bounded || op.dot, pd.stream, xin[i], epi[i], pd.st.p, fh, pd.partials.p, pd.rc, publish, op.slot};
-    L.fh.v = xin[i];
+    *kern = spmv_kernel(m, mean_nnz >= 48.0 && !op.dot);
+    LaunchArgs L{0, bounded || op.dot, pd.stream, xin[s], epi[s], pd.st.p, fh, pd.partials.p, pd.rc, publish, op.slot};
+    L.fh.v = xin[s];
     int n_main;
     if (m.sell_diag || m.sell_vi4) {
       n_main = (m.nslices4 + BLOCK / 32 - 1) / (BLOCK / 32);
@@ -776,6 +917,13 @@ void Engine::enqueue_op(const OpSpec& op, const std::vector<const double*>& xin,
       n_main = I.grid_for(m.nrows, (BLOCK / m.lanes) * 4);
     }
     L.grid = std::max(n_main, 1);
+    return L;
+  };
+  auto launch_main = [&](PartDev& pd, size_t s, const FusedHalo& fh, int publish) {
+    LevelDev& ld = I.LV(pd, l);
+    const DevCsr& m = ld.blk[op.which];
+    SpmvKernel kern;
+    const LaunchArgs L = main_args(pd, s, fh, publish, &kern);
     switch (kern) {
       case SpmvKernel::SellDiag: launch_sell_diag(op.mode, op.dot, m.diagview(), L); break;
       case SpmvKernel::SellVi:
@@ -786,21 +934,36 @@ void Engine::enqueue_op(const OpSpec& op, const std::vector<const double*>& xin,
       case SpmvKernel::StreamLong: launch_stream(op.mode, op.dot, kern == SpmvKernel::StreamLong, m.sview(), L); break;
       case SpmvKernel::Csr: launch_csr(op.mode, op.dot, m.lanes, m.view(), L); break;
     }
-    if (I.naming) {
-      static const char* MODES[] = {"mul", "resid", "jacobi", "add", "restrict", "cheb"};
-      static const char* OPS[] = {"A", "P", "R"};
-      I.names.push_back(std::string(SPMV_KERNEL_NAMES[(int)kern]) + " " + MODES[op.mode] + (op.dot ? "+dot " : " ") + OPS[wsel] +
-                        std::to_string(l) + (I.tail_mode ? " tail" : "") + (fh.n_pack ? " +pack" : "") + (fh.n_bnd ? " +bnd" : ""));
-      I.naming = false;
+    if (I.naming)
+      launch_name(kern, 1, fh);
+    else
       I.note_launch();
-      I.naming = true;
-    } else {
-      I.note_launch();
+  };
+  // K columns of part i in one k-wide launch: slots ss[0..n), n <= K (the rest absent)
+  auto launch_group = [&](auto kc, size_t i, const size_t* ss, int n, const FusedHalo& fh, int publish) {
+    constexpr int K = decltype(kc)::value;
+    MultiCols<K> mc{};
+    LaunchArgs L{};
+    SpmvKernel kern = SpmvKernel::Csr;
+    for (int c = 0; c < n; ++c) {
+      PartDev& pd = I.S(ss[c]);
+      const LaunchArgs Lc = main_args(pd, ss[c], fh, publish, &kern);
+      if (c == 0) L = Lc;
+      mc.x[c] = Lc.x;
+      mc.a[c] = Lc.a;
+      mc.st[c] = Lc.st;
+      mc.partials[c] = Lc.partials;
+      mc.rc[c] = Lc.rc;
     }
+    launch_multi<K>(kern, I.LV(I.P(i), l).blk[op.which], op.mode, op.dot, L, mc);
+    if (I.naming)
+      launch_name(kern, n, fh);
+    else
+      I.note_launch();
   };
 
   if (fused) {  // one launch per part: pack + main + boundary roles
-    for (size_t i = 0; i < I.parts.size(); ++i) {
+    for (size_t i = 0; i < np; ++i) {
       PartDev& pd = I.P(i);
       LevelDev& hl = I.LV(pd, op.halo_level);
       const bool nbrs = hl.n_recv_nbrs > 0 || hl.n_send_nbrs > 0;
@@ -814,33 +977,51 @@ void Engine::enqueue_op(const OpSpec& op, const std::vector<const double*>& xin,
   // split: three phases over all parts so that no kernel waits for a later kernel of its own stream
   // phase 1: producers (never wait)
   if (exchange)
-    for (size_t i = 0; i < I.parts.size(); ++i) {
-      PartDev& pd = I.P(i);
+    for (size_t s = 0; s < ns; ++s) {
+      PartDev& pd = I.S(s);
       LevelDev& hl = I.LV(pd, op.halo_level);
       if (hl.n_send_nbrs == 0 && hl.n_recv_nbrs == 0) continue;
       I.set_dev(pd);
-      k_halo_pack<<<I.grid_for(hl.n_send, BLOCK * 4), BLOCK, 0, pd.stream>>>(xin[i], hl.send_idx.p, hl.n_send, hl.send_nbrs.p,
+      k_halo_pack<<<I.grid_for(hl.n_send, BLOCK * 4), BLOCK, 0, pd.stream>>>(xin[s], hl.send_idx.p, hl.n_send, hl.send_nbrs.p,
                                                                              hl.n_send_nbrs, pd.st.p, op.halo_level);
       I.note_launch("k_halo_pack");
     }
-  // phase 2: all rows of the own-own block (boundary rows are computed but not stored)
-  for (size_t i = 0; i < I.parts.size(); ++i) {
+  // phase 2: all rows of the own-own block (boundary rows are computed but not stored).  Several columns of a block whose class
+  // takes a k-wide launch (multi_width) share launches of up to four columns; the others run the single kernel per column.
+  // fh, bnd_follows and the kernel depend on the part only (matrices, boundary-row marks, halo plan), not on the bound column:
+  // every per-column argument is taken after I.S(slot) in main_args.
+  const size_t nc = I.cols.size();
+  for (size_t i = 0; i < np; ++i) {
     PartDev& pd = I.P(i);
     LevelDev& hl = I.LV(pd, op.halo_level);
     const bool bnd_follows = need && hl.n_recv_nbrs > 0;
     I.set_dev(pd);
     const FusedHalo fh = halo_args(pd, false, false);
-    launch_main(pd, i, fh, bnd_follows ? 0 : 1);
+    const SpmvKernel kern = spmv_kernel(I.LV(pd, l).blk[op.which], false);
+    for (size_t c0 = 0; c0 < nc;) {
+      const int K = multi_width(kern, op.which, op.mode, op.dot, (int)std::min<size_t>(4, nc - c0));
+      const int g = std::min<int>(K, (int)(nc - c0));
+      size_t ss[4];
+      for (int c = 0; c < g; ++c) ss[c] = (c0 + c) * np + i;
+      if (K == 1) {
+        launch_main(I.S(ss[0]), ss[0], fh, bnd_follows ? 0 : 1);
+      } else if (K == 2) {
+        launch_group(std::integral_constant<int, 2>{}, i, ss, g, fh, bnd_follows ? 0 : 1);
+      } else {
+        launch_group(std::integral_constant<int, 4>{}, i, ss, g, fh, bnd_follows ? 0 : 1);
+      }
+      c0 += g;
+    }
   }
   // phase 3: boundary rows (consumers: wait for the neighbours' flags)
   if (need)
-    for (size_t i = 0; i < I.parts.size(); ++i) {
-      PartDev& pd = I.P(i);
+    for (size_t s = 0; s < ns; ++s) {
+      PartDev& pd = I.S(s);
       LevelDev& hl = I.LV(pd, op.halo_level);
       if (hl.n_recv_nbrs == 0) continue;
       I.set_dev(pd);
       const FusedHalo fh = halo_args(pd, false, true);
-      LaunchArgs L{fh.n_bnd, false, pd.stream, xin[i], epi[i], pd.st.p, fh, pd.partials.p, pd.rc, 1, op.slot};
+      LaunchArgs L{fh.n_bnd, false, pd.stream, xin[s], epi[s], pd.st.p, fh, pd.partials.p, pd.rc, 1, op.slot};
       launch_boundary(op.mode, op.dot, L);
       I.note_launch("k_boundary");
     }
@@ -850,8 +1031,10 @@ void Engine::enqueue_op(const OpSpec& op, const std::vector<const double*>& xin,
 // ---------------------------------------------------------------------------------------------
 // construction
 // ---------------------------------------------------------------------------------------------
-Engine::Engine(Hierarchy* h, int nlocal, const int32_t* local_parts, const int32_t* device_ids) : impl(new Impl) {
+Engine::Engine(Hierarchy* h, int nlocal, const int32_t* local_parts, const int32_t* device_ids, int kmax) : impl(new Impl) {
   Impl& I = *impl;
+  if (kmax < 1 || kmax > PAMG_MAX_RHS) throw std::runtime_error("right-hand-side capacity must be in 1..PAMG_MAX_RHS");
+  I.kmax = kmax;
   I.h = h;
   I.nparts = h->nparts;
   I.L = (int)h->levels.size();
@@ -929,14 +1112,20 @@ Engine::Engine(Hierarchy* h, int nlocal, const int32_t* local_parts, const int32
     CK(cudaEventCreate(&pd.ev0));
     CK(cudaEventCreate(&pd.ev1));
     pd.lay = arena_layout(*h, part);
-    CK(cudaMalloc(&pd.arena, pd.lay.total));
-    CK(cudaMemset(pd.arena, 0, pd.lay.total));
-    I.arena_of[part] = pd.arena;
-    pd.st.alloc(1);
+    CK(cudaMalloc(&pd.arena, pd.lay.col_stride * kmax));
+    CK(cudaMemset(pd.arena, 0, pd.lay.col_stride * kmax));
     {
+      const int32_t cap = kmax;
+      CK(cudaMemcpy(pd.arena + pd.lay.capacity, &cap, sizeof(cap), cudaMemcpyHostToDevice));
+    }
+    I.arena_of[part] = pd.arena;
+    pd.cols.reset(new PartDev::Col[kmax]);
+    for (int c = 0; c < kmax; ++c) {
+      DBuf<DevState>& st = pd.cols[c].st;
+      st.alloc(1);
       unsigned long long tmo = SPIN_TIMEOUT_NS;
       if (const char* te = getenv("PAMG_SPIN_TIMEOUT_MS")) tmo = std::max(1ll, atoll(te)) * 1000000ull;
-      CK(cudaMemcpy(&pd.st.p->spin_timeout_ns, &tmo, sizeof(tmo), cudaMemcpyHostToDevice));
+      CK(cudaMemcpy(&st.p->spin_timeout_ns, &tmo, sizeof(tmo), cudaMemcpyHostToDevice));
     }
     pd.scratch4.alloc(RED_W);
     int max_blocks = Impl::MAX_GRID;
@@ -971,22 +1160,27 @@ Engine::Engine(Hierarchy* h, int nlocal, const int32_t* local_parts, const int32
       }
       ld.w.upload(w);
       ld.dinv.upload(dinv);
-      ld.x.alloc(pl.n_own);
-      ld.x2.alloc(pl.n_own);
-      ld.b.alloc(pl.n_own);
-      ld.t.alloc(pl.n_own);
-      if (o.smoother == PAMG_SMOOTHER_CHEBYSHEV) {
-        ld.d.alloc(pl.n_own);
-        ld.d2.alloc(pl.n_own);
-      }
       ld.send_idx.upload(pl.send_idx);
       ld.n_send = (int)pl.send_idx.size();
       ld.n_send_nbrs = (int)pl.send.size();
       ld.n_recv_nbrs = (int)pl.recv.size();
-      ld.hr.ghost[0] = (const double*)(pd.arena + pd.lay.ghost[l]);
-      ld.hr.ghost[1] = ld.hr.ghost[0] + pl.n_ghost;
-      ld.hr.flags = (const uint32_t*)(pd.arena + pd.lay.flags[l]);
-      ld.hr.n_nbrs = ld.n_recv_nbrs;
+      ld.cols.reset(new LevelDev::Col[kmax]);
+      for (int c = 0; c < kmax; ++c) {
+        LevelDev::Col& lc = ld.cols[c];
+        lc.x.alloc(pl.n_own);
+        lc.x2.alloc(pl.n_own);
+        lc.b.alloc(pl.n_own);
+        lc.t.alloc(pl.n_own);
+        if (o.smoother == PAMG_SMOOTHER_CHEBYSHEV) {
+          lc.d.alloc(pl.n_own);
+          lc.d2.alloc(pl.n_own);
+        }
+        const char* ca = pd.arena + (size_t)c * pd.lay.col_stride;
+        lc.hr.ghost[0] = (const double*)(ca + pd.lay.ghost[l]);
+        lc.hr.ghost[1] = lc.hr.ghost[0] + pl.n_ghost;
+        lc.hr.flags = (const uint32_t*)(ca + pd.lay.flags[l]);
+        lc.hr.n_nbrs = ld.n_recv_nbrs;
+      }
       // assemble! gather plan: for every own row that some neighbour holds as a ghost, the staging
       // positions that contribute to it (ascending neighbour part, ascending slot).  It works on the caller's
       // local vector (io_local).
@@ -1009,7 +1203,7 @@ Engine::Engine(Hierarchy* h, int nlocal, const int32_t* local_parts, const int32
       }
     }
     pd.partials_cap = max_blocks + 8 * 148;  // one partial per CTA of a fused-reduction kernel (+ halo roles)
-    pd.partials.alloc((size_t)pd.partials_cap);
+    for (int c = 0; c < kmax; ++c) pd.cols[c].partials.alloc((size_t)pd.partials_cap);
     // replicated tail: merged levels + the maps of the level it is entered through
     pd.tlev.resize(I.L);
     if (I.tail_level < I.L - 1)
@@ -1026,16 +1220,20 @@ Engine::Engine(Hierarchy* h, int nlocal, const int32_t* local_parts, const int32
         for (int b = 0; b < 3; ++b) build_bnd(empty, empty, tl.bnd[b]);
         tl.w.upload(tw[l]);
         tl.dinv.upload(tdinv[l]);
-        tl.x.alloc(n);
-        tl.x2.alloc(n);
-        tl.b.alloc(n);
-        tl.t.alloc(n);
-        if (o.smoother == PAMG_SMOOTHER_CHEBYSHEV) {
-          tl.d.alloc(n);
-          tl.d2.alloc(n);
+        tl.cols.reset(new LevelDev::Col[kmax]);
+        for (int c = 0; c < kmax; ++c) {
+          LevelDev::Col& lc = tl.cols[c];
+          lc.x.alloc(n);
+          lc.x2.alloc(n);
+          lc.b.alloc(n);
+          lc.t.alloc(n);
+          if (o.smoother == PAMG_SMOOTHER_CHEBYSHEV) {
+            lc.d.alloc(n);
+            lc.d2.alloc(n);
+          }
+          lc.send_nbrs.alloc(0);
         }
         tl.send_idx.alloc(0);
-        tl.send_nbrs.alloc(0);
       }
     const PartLevel& pc = h->levels[I.tail_level].parts[part];
     pd.inv.upload(h->coarse_inv);
@@ -1043,16 +1241,19 @@ Engine::Engine(Hierarchy* h, int nlocal, const int32_t* local_parts, const int32
     pd.ghost_gid_T.upload(pc.ghost_to_global);
     // PCG vectors on level 0
     const int64_t n0 = h->levels[0].parts[part].n_own;
-    pd.xsol.alloc(n0);
-    pd.p.alloc(n0);
-    pd.q.alloc(n0);
-    pd.bsave.alloc(n0);
+    for (int c = 0; c < kmax; ++c) {
+      PartDev::Col& pc = pd.cols[c];
+      pc.xsol.alloc(n0);
+      pc.p.alloc(n0);
+      pc.q.alloc(n0);
+      pc.bsave.alloc(n0);
+    }
     int64_t maxloc = 0;
     for (int l = 0; l < I.L; ++l) maxloc = std::max(maxloc, h->levels[l].parts[part].n_own + h->levels[l].parts[part].n_ghost);
     pd.io_local.alloc(maxloc);
   }
-  CK(cudaHostAlloc(&I.hstat, sizeof(HostStat) * HS_RING, cudaHostAllocMapped | cudaHostAllocPortable));
-  std::memset(I.hstat, 0, sizeof(HostStat) * HS_RING);
+  CK(cudaHostAlloc(&I.hstat_base, sizeof(HostStat) * HS_RING * kmax, cudaHostAllocMapped | cudaHostAllocPortable));
+  std::memset(I.hstat_base, 0, sizeof(HostStat) * HS_RING * kmax);
   plan_buffers();
   {  // fused halo roles need every local part alone on its device (a kernel may then wait for its peers)
     std::map<int, int> per_dev;
@@ -1100,17 +1301,23 @@ void Engine::plan_buffers() {
   int flips = 1;  // prolongation writes out of place
   if (o.nu_pre > 0) flips += o.nu_pre * steps - 1;  // the zero-guess first step is written by the producer of b
   flips += o.nu_post * steps;
+  auto plan = [&](LevelDev& ld) {
+    for (int c = 0; c < I.kmax; ++c) ld.cols[c].xstart = (flips % 2 == 0) ? ld.cols[c].x.p : ld.cols[c].x2.p;
+  };
   for (auto& up : I.parts) {
-    for (auto& ld : up->lev) ld->xstart = (flips % 2 == 0) ? ld->x.p : ld->x2.p;
+    for (auto& ld : up->lev) plan(*ld);
     for (auto& ld : up->tlev)
-      if (ld) ld->xstart = (flips % 2 == 0) ? ld->x.p : ld->x2.p;
+      if (ld) plan(*ld);
   }
+  I.bind(0, true);
 }
 
 // ---------------------------------------------------------------------------------------------
 // peer wiring
 // ---------------------------------------------------------------------------------------------
 int32_t Engine::handle_bytes() { return (int32_t)sizeof(cudaIpcMemHandle_t); }
+
+int Engine::rhs_capacity() const { return impl->kmax; }
 
 void Engine::export_handle(int part, void* blob) {
   Impl& I = *impl;
@@ -1159,11 +1366,23 @@ void Engine::connect() {
   }
   std::vector<ArenaLayout> lay(I.nparts);
   for (int p = 0; p < I.nparts; ++p) lay[p] = arena_layout(h, p);
+  // every process must have allocated the same number of column copies: the wiring below addresses column c of a peer's arena
+  for (int p = 0; p < I.nparts; ++p) {
+    if (I.local_index[p] >= 0) continue;
+    int32_t cap = 0;
+    I.set_dev(I.P(0));
+    CK(cudaMemcpy(&cap, I.arena_of[p] + lay[p].capacity, sizeof(cap), cudaMemcpyDeviceToHost));
+    if (cap != I.kmax)
+      throw CommError("connect: part " + std::to_string(p) + " was initialised with right-hand-side capacity " + std::to_string(cap) +
+                      ", this process with " + std::to_string(I.kmax) + " (pamg_set_rhs_capacity must agree in every process)");
+  }
 
-  for (auto& up : I.parts) {
+  for (auto& up : I.parts)
+    for (int c = 0; c < I.kmax; ++c) {
     PartDev& pd = *up;
     I.set_dev(pd);
     const int me = pd.part;
+    auto arena_c = [&](int q) { return I.arena_of[q] + (size_t)c * lay[q].col_stride; };
     for (int l = 0; l < I.L; ++l) {
       const PartLevel& pl = h.levels[l].parts[me];
       LevelDev& ld = *pd.lev[l];
@@ -1175,7 +1394,7 @@ void Engine::connect() {
         for (size_t k = 0; k < ql.recv.size(); ++k)
           if (ql.recv[k].part == me) idx = (int)k;
         if (idx < 0) throw std::runtime_error("halo plan asymmetry");
-        char* qa = I.arena_of[nb.part];
+        char* qa = arena_c(nb.part);
         SendNbr s;
         double* g0 = (double*)(qa + lay[nb.part].ghost[l]);
         s.ghost[0] = g0 + nb.slot0;
@@ -1185,7 +1404,8 @@ void Engine::connect() {
         s.count = nb.count;
         sn.push_back(s);
       }
-      ld.send_nbrs.upload(sn);
+      ld.cols[c].send_nbrs.upload(sn);
+      if (c > 0) continue;  // assemble! is a single-column operation
       // assemble!: my ghosts owned by q go to q's staging at the offset of q's send segment for me
       for (const Neighbor& rb : pl.recv) {
         const PartLevel& ql = h.levels[l].parts[rb.part];
@@ -1207,7 +1427,7 @@ void Engine::connect() {
     std::vector<RedPub> rp(I.nparts);
     std::vector<CoarsePub> cp(I.nparts);
     for (int d = 0; d < I.nparts; ++d) {
-      char* qa = I.arena_of[d];
+      char* qa = arena_c(d);
       double* r0 = (double*)(qa + lay[d].red);
       rp[d].slot[0] = r0 + (size_t)me * RED_W;
       rp[d].slot[1] = r0 + (size_t)I.nparts * RED_W + (size_t)me * RED_W;
@@ -1217,13 +1437,15 @@ void Engine::connect() {
       cp[d].buf[1] = c0 + h.levels[I.tail_level].n_global;
       cp[d].flag = (uint32_t*)(qa + lay[d].coarse_flags) + me;
     }
-    pd.red_pubs.upload(rp);
-    pd.coarse_pubs.upload(cp);
-    pd.rc.pubs = pd.red_pubs.p;
-    pd.rc.local = (const double*)(pd.arena + pd.lay.red);
-    pd.rc.flags = (const uint32_t*)(pd.arena + pd.lay.red_flags);
-    pd.rc.nparts = I.nparts;
+    PartDev::Col& pc = pd.cols[c];
+    pc.red_pubs.upload(rp);
+    pc.coarse_pubs.upload(cp);
+    pc.rc.pubs = pc.red_pubs.p;
+    pc.rc.local = (const double*)(arena_c(me) + pd.lay.red);
+    pc.rc.flags = (const uint32_t*)(arena_c(me) + pd.lay.red_flags);
+    pc.rc.nparts = I.nparts;
   }
+  I.bind(0, true);
   I.connected = true;
 }
 
@@ -1242,14 +1464,15 @@ void Engine::sync_all() {
   }
 }
 
+// host vectors: one pointer per part, column j of a multi-column call at [j * nparts + part]
 void Engine::upload_vec(int level, const double* const* host, int which_buf) {
   Impl& I = *impl;
-  for (auto& up : I.parts) {
-    PartDev& pd = *up;
+  for (size_t s = 0; s < I.nslots(); ++s) {
+    PartDev& pd = I.S(s);
+    const double* hv = host[(size_t)I.col_of(s) * I.nparts + pd.part];
     I.set_dev(pd);
-    if (!host[pd.part]) throw std::runtime_error("null vector pointer for a local part");
-    CK(cudaMemcpyAsync(vec(pd, level, which_buf), host[pd.part], pd.lev[level]->n_own * sizeof(double), cudaMemcpyHostToDevice,
-                       pd.stream));
+    if (!hv) throw std::runtime_error("null vector pointer for a local part");
+    CK(cudaMemcpyAsync(vec(pd, level, which_buf), hv, pd.lev[level]->n_own * sizeof(double), cudaMemcpyHostToDevice, pd.stream));
   }
 }
 
@@ -1261,11 +1484,12 @@ void Engine::download_own(PartDev& pd, int level, const double* src, double* hos
 
 void Engine::download_vec(int level, double* const* host, int which_buf) {
   Impl& I = *impl;
-  for (auto& up : I.parts) {
-    PartDev& pd = *up;
+  for (size_t s = 0; s < I.nslots(); ++s) {
+    PartDev& pd = I.S(s);
+    double* hv = host[(size_t)I.col_of(s) * I.nparts + pd.part];
     I.set_dev(pd);
-    if (!host[pd.part]) throw std::runtime_error("null vector pointer for a local part");
-    download_own(pd, level, vec(pd, level, which_buf), host[pd.part]);
+    if (!hv) throw std::runtime_error("null vector pointer for a local part");
+    download_own(pd, level, vec(pd, level, which_buf), hv);
   }
   sync_all();
 }
@@ -1288,22 +1512,24 @@ double* Engine::vec(PartDev& pd, int level, int which) {
 
 void Engine::check_device_error() {
   Impl& I = *impl;
-  for (auto& up : I.parts) {
-    I.set_dev(*up);
-    DevState s;
-    CK(cudaMemcpy(&s, up->st.p, sizeof(s), cudaMemcpyDeviceToHost));
-    if (s.error) {
-      CK(cudaMemset(&up->st.p->error, 0, sizeof(int32_t)));
-      throw CommError("halo/all-reduce wait timed out on part " + std::to_string(up->part));
+  for (size_t s = 0; s < I.nslots(); ++s) {
+    PartDev& pd = I.S(s);
+    I.set_dev(pd);
+    DevState ds;
+    CK(cudaMemcpy(&ds, pd.st.p, sizeof(ds), cudaMemcpyDeviceToHost));
+    if (ds.error) {
+      CK(cudaMemset(&pd.st.p->error, 0, sizeof(int32_t)));
+      throw CommError("halo/all-reduce wait timed out on part " + std::to_string(pd.part));
     }
   }
 }
 
 void Engine::clear_done() {
   Impl& I = *impl;
-  for (auto& up : I.parts) {
-    I.set_dev(*up);
-    CK(cudaMemsetAsync(&up->st.p->done, 0, sizeof(int32_t), up->stream));
+  for (size_t s = 0; s < I.nslots(); ++s) {
+    PartDev& pd = I.S(s);
+    I.set_dev(pd);
+    CK(cudaMemsetAsync(&pd.st.p->done, 0, sizeof(int32_t), pd.stream));
   }
 }
 
@@ -1312,7 +1538,7 @@ void Engine::clear_done() {
 // ---------------------------------------------------------------------------------------------
 std::vector<const double*> Engine::ptrs(int level, int which) {
   std::vector<const double*> v;
-  for (auto& up : impl->parts) v.push_back(vec(*up, level, which));
+  for (size_t s = 0; s < impl->nslots(); ++s) v.push_back(vec(impl->S(s), level, which));
   return v;
 }
 
@@ -1321,7 +1547,7 @@ std::vector<const double*> Engine::ptrs(int level, int which) {
 void Engine::enqueue_smooth(int l, int nu, std::vector<double*>& cur, bool zero_guess_done, bool dot_last) {
   Impl& I = *impl;
   const pamg_options& o = I.h->opts;
-  const size_t np = I.parts.size();
+  const size_t np = I.nslots();
   auto other = [&](size_t i) {
     LevelDev& ld = I.LV(i, l);
     return cur[i] == ld.x.p ? ld.x2.p : ld.x.p;
@@ -1403,8 +1629,8 @@ void Engine::enqueue_tail(bool zero_guess) {
       throw;
     }
     I.tail_mode = false;
-    for (auto& up : I.parts) {
-      PartDev& pd = *up;
+    for (size_t s = 0; s < I.nslots(); ++s) {
+      PartDev& pd = I.S(s);
       LevelDev& ld = *pd.lev[l];
       LevelDev& tl = *pd.tlev[l];
       I.set_dev(pd);
@@ -1415,8 +1641,8 @@ void Engine::enqueue_tail(bool zero_guess) {
     CK(cudaGetLastError());
     return;
   }
-  for (auto& up : I.parts) {
-    PartDev& pd = *up;
+  for (size_t s = 0; s < I.nslots(); ++s) {
+    PartDev& pd = I.S(s);
     LevelDev& ld = *pd.lev[l];
     I.set_dev(pd);
     k_coarse_gather<<<I.grid_for(ld.n_own, BLOCK), BLOCK, 0, pd.stream>>>(ld.b.p, pd.own_gid_T.p, (int)ld.n_own, pd.coarse_pubs.p,
@@ -1424,26 +1650,26 @@ void Engine::enqueue_tail(bool zero_guess) {
     I.note_launch("k_coarse_gather");
   }
   if (l == I.L - 1) {
-    for (auto& up : I.parts) {
-      PartDev& pd = *up;
+    for (size_t s = 0; s < I.nslots(); ++s) {
+      PartDev& pd = I.S(s);
       LevelDev& ld = *pd.lev[l];
       I.set_dev(pd);
       const int rows = (int)(ld.n_own + ld.n_ghost);
-      const double* c0 = (const double*)(pd.arena + pd.lay.coarse);
+      const double* c0 = (const double*)(pd.carena + pd.lay.coarse);
       k_coarse_solve<<<I.grid_for(std::max(rows, 1), BLOCK / 32), BLOCK, 0, pd.stream>>>(
-          pd.inv.p, n, c0, c0 + n, (const uint32_t*)(pd.arena + pd.lay.coarse_flags), I.nparts, pd.own_gid_T.p, (int)ld.n_own,
+          pd.inv.p, n, c0, c0 + n, (const uint32_t*)(pd.carena + pd.lay.coarse_flags), I.nparts, pd.own_gid_T.p, (int)ld.n_own,
           pd.ghost_gid_T.p, (int)ld.n_ghost, ld.x.p, (double*)ld.hr.ghost[0], pd.st.p);
       I.note_launch("k_coarse_solve");
     }
     CK(cudaGetLastError());
     return;
   }
-  for (auto& up : I.parts) {
-    PartDev& pd = *up;
+  for (size_t s = 0; s < I.nslots(); ++s) {
+    PartDev& pd = I.S(s);
     LevelDev& tl = *pd.tlev[l];
     I.set_dev(pd);
-    const double* c0 = (const double*)(pd.arena + pd.lay.coarse);
-    k_tail_in<<<I.grid_for(n, BLOCK), BLOCK, 0, pd.stream>>>(c0, c0 + n, (const uint32_t*)(pd.arena + pd.lay.coarse_flags), I.nparts,
+    const double* c0 = (const double*)(pd.carena + pd.lay.coarse);
+    k_tail_in<<<I.grid_for(n, BLOCK), BLOCK, 0, pd.stream>>>(c0, c0 + n, (const uint32_t*)(pd.carena + pd.lay.coarse_flags), I.nparts,
                                                              tl.b.p, tl.xstart, o.nu_pre > 0 ? tl.w.p : nullptr, n, pd.st.p);
     I.note_launch("k_tail_in");
   }
@@ -1456,8 +1682,8 @@ void Engine::enqueue_tail(bool zero_guess) {
     throw;
   }
   I.tail_mode = false;
-  for (auto& up : I.parts) {
-    PartDev& pd = *up;
+  for (size_t s = 0; s < I.nslots(); ++s) {
+    PartDev& pd = I.S(s);
     LevelDev& ld = *pd.lev[l];
     LevelDev& tl = *pd.tlev[l];
     I.set_dev(pd);
@@ -1474,14 +1700,14 @@ void Engine::enqueue_tail(bool zero_guess) {
 void Engine::enqueue_vcycle(int l, bool dot_rz, bool zero_guess) {
   Impl& I = *impl;
   const pamg_options& o = I.h->opts;
-  const size_t np = I.parts.size();
+  const size_t np = I.nslots();
   if (!I.tail_mode && l == I.tail_level) {
     enqueue_tail(zero_guess);
     return;
   }
   if (I.tail_mode && l == I.L - 1) {  // coarsest level of the replicated tail: x = A_L^-1 b, whole vector
-    for (auto& up : I.parts) {
-      PartDev& pd = *up;
+    for (size_t s = 0; s < I.nslots(); ++s) {
+      PartDev& pd = I.S(s);
       LevelDev& ld = I.LV(pd, l);
       I.set_dev(pd);
       k_dense<<<I.grid_for(std::max<int64_t>(ld.n_own, 1), BLOCK / 32), BLOCK, 0, pd.stream>>>(pd.inv.p, (int)ld.n_own, ld.b.p, ld.x.p,
@@ -1526,7 +1752,7 @@ void Engine::enqueue_vcycle(int l, bool dot_rz, bool zero_guess) {
     enqueue_op(op, xin, epi);
     if (!coarse_is_last && o.nu_pre == 0)
       for (size_t i = 0; i < np; ++i) {
-        PartDev& pd = I.P(i);
+        PartDev& pd = I.S(i);
         LevelDev& lc = I.LV(pd, l + 1);
         I.set_dev(pd);
         k_scale<<<I.grid_for(lc.n_own, BLOCK * 4), BLOCK, 0, pd.stream>>>(lc.b.p, nullptr, lc.xstart, (int)lc.n_own, pd.st.p);
@@ -1558,7 +1784,7 @@ void Engine::enqueue_vcycle(int l, bool dot_rz, bool zero_guess) {
     if (cur[i] == ld.x.p) continue;
     if (zero_guess) throw std::runtime_error("internal: V-cycle buffer plan mismatch");
     // a visit that started from x has one buffer flip more than the plan of the zero-guess visit: copy back
-    PartDev& pd = I.P(i);
+    PartDev& pd = I.S(i);
     I.set_dev(pd);
     k_copy<<<I.grid_for(ld.n_own, BLOCK * 4), BLOCK, 0, pd.stream>>>(cur[i], ld.x.p, (int)ld.n_own, pd.st.p);
     I.note_launch("k_copy");
@@ -1568,8 +1794,8 @@ void Engine::enqueue_vcycle(int l, bool dot_rz, bool zero_guess) {
 // r.z when the V-cycle could not fuse it (nu_post == 0, Chebyshev, or a single-level hierarchy)
 void Engine::enqueue_dot_rz() {
   Impl& I = *impl;
-  for (auto& up : I.parts) {
-    PartDev& pd = *up;
+  for (size_t s = 0; s < I.nslots(); ++s) {
+    PartDev& pd = I.S(s);
     LevelDev& l0 = *pd.lev[0];
     I.set_dev(pd);
     k_dot<<<I.grid_red(l0.n_own), BLOCK, 0, pd.stream>>>(l0.b.p, l0.x.p, (int)l0.n_own, pd.st.p, pd.partials.p, pd.rc,
@@ -1589,12 +1815,12 @@ bool Engine::vcycle_fuses_rz() const {
 //   alpha = rz/pq ; x += alpha p ; r -= alpha q ; z0 = w .* r ; rr ; check
 void Engine::enqueue_pcg_iteration(int mode) {
   Impl& I = *impl;
-  const size_t np = I.parts.size();
+  const size_t np = I.nslots();
   const bool precond = mode != 0, flexible = mode == 2;
   if (flexible) {  // z = M^-1 r, then r.z and r_prev.z in one pass (one all-reduce)
     enqueue_vcycle(0, false, true);
-    for (auto& up : I.parts) {
-      PartDev& pd = *up;
+    for (size_t s = 0; s < I.nslots(); ++s) {
+      PartDev& pd = I.S(s);
       LevelDev& l0 = *pd.lev[0];
       I.set_dev(pd);
       k_dot2<<<I.grid_red(l0.n_own), BLOCK, 0, pd.stream>>>(l0.b.p, l0.x.p, pd.rprev.p, (int)l0.n_own, pd.st.p, pd.partials.p, pd.rc);
@@ -1604,8 +1830,8 @@ void Engine::enqueue_pcg_iteration(int mode) {
     enqueue_vcycle(0, vcycle_fuses_rz(), true);
     if (!vcycle_fuses_rz()) enqueue_dot_rz();
   } else {
-    for (auto& up : I.parts) {
-      PartDev& pd = *up;
+    for (size_t s = 0; s < I.nslots(); ++s) {
+      PartDev& pd = I.S(s);
       LevelDev& l0 = *pd.lev[0];
       I.set_dev(pd);
       k_copy_dot<<<I.grid_red(l0.n_own), BLOCK, 0, pd.stream>>>(l0.b.p, l0.x.p, (int)l0.n_own, pd.st.p, pd.partials.p,
@@ -1613,8 +1839,8 @@ void Engine::enqueue_pcg_iteration(int mode) {
       I.note_launch("k_copy_dot");
     }
   }
-  for (auto& up : I.parts) {
-    PartDev& pd = *up;
+  for (size_t s = 0; s < I.nslots(); ++s) {
+    PartDev& pd = I.S(s);
     LevelDev& l0 = *pd.lev[0];
     I.set_dev(pd);
     k_update_p<<<I.grid_for(l0.n_own, BLOCK * 4), BLOCK, 0, pd.stream>>>(l0.x.p, pd.p.p, (int)l0.n_own, pd.st.p, pd.rc, flexible ? 1 : 0);
@@ -1624,7 +1850,7 @@ void Engine::enqueue_pcg_iteration(int mode) {
     std::vector<EpiArgs> epi(np);
     std::vector<const double*> xin(np);
     for (size_t i = 0; i < np; ++i) {
-      PartDev& pd = I.P(i);
+      PartDev& pd = I.S(i);
       xin[i] = pd.p.p;
       epi[i] = EpiArgs{pd.q.p, nullptr, nullptr, nullptr, nullptr, nullptr, pd.p.p, 0.0, 0.0};
     }
@@ -1632,22 +1858,22 @@ void Engine::enqueue_pcg_iteration(int mode) {
     enqueue_op(op, xin, epi);
   }
   const bool zero_guess = precond && I.L > 1 && I.h->opts.nu_pre > 0;
-  for (auto& up : I.parts) {
-    PartDev& pd = *up;
+  for (size_t s = 0; s < I.nslots(); ++s) {
+    PartDev& pd = I.S(s);
     LevelDev& l0 = *pd.lev[0];
     I.set_dev(pd);
     k_update_xr<<<I.grid_red(l0.n_own), BLOCK, 0, pd.stream>>>(pd.xsol.p, l0.b.p, pd.p.p, pd.q.p, l0.xstart,
                                                                          zero_guess ? l0.w.p : nullptr, (int)l0.n_own, pd.st.p,
                                                                          pd.partials.p, pd.rc, I.fold_check ? 1 : 0, pd.hist.p,
-                                                                         up.get() == I.parts[0].get() ? I.hstat : nullptr,
+                                                                         &pd == I.parts[0].get() ? I.hstat : nullptr,
                                                                          flexible ? pd.rprev.p : nullptr);
     I.note_launch(I.fold_check ? "k_update_xr+check" : "k_update_xr");
   }
   if (!I.fold_check)  // several parts on one GPU: a kernel must not wait for a later kernel of its own stream
-    for (auto& up : I.parts) {
-      PartDev& pd = *up;
+    for (size_t s = 0; s < I.nslots(); ++s) {
+      PartDev& pd = I.S(s);
       I.set_dev(pd);
-      k_check<<<1, 1, 0, pd.stream>>>(pd.st.p, pd.rc, pd.hist.p, up.get() == I.parts[0].get() ? I.hstat : nullptr);
+      k_check<<<1, 1, 0, pd.stream>>>(pd.st.p, pd.rc, pd.hist.p, &pd == I.parts[0].get() ? I.hstat : nullptr);
       I.note_launch("k_check");
     }
   CK(cudaGetLastError());
@@ -1717,10 +1943,10 @@ void Engine::spmv(int level, const double* const* x, double* const* y) {
   I.launches = 0;
   clear_done();
   upload_vec(level, x, V_X);
-  const size_t np = I.parts.size();
-  std::vector<EpiArgs> epi(np);
-  for (size_t i = 0; i < np; ++i)
-    epi[i] = EpiArgs{I.P(i).lev[level]->t.p, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0.0, 0.0};
+  const size_t ns = I.nslots();
+  std::vector<EpiArgs> epi(ns);
+  for (size_t s = 0; s < ns; ++s)
+    epi[s] = EpiArgs{I.S(s).lev[level]->t.p, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0.0, 0.0};
   OpSpec op{level, PAMG_A_OO, level, M_MUL, false, 0, false};
   enqueue_op(op, ptrs(level, V_X), epi);
   download_vec(level, y, V_T);
@@ -1892,8 +2118,8 @@ void Engine::enqueue_vcycle_entry() {
   Impl& I = *impl;
   const pamg_options& o = I.h->opts;
   if (I.L > 1)
-    for (auto& up : I.parts) {
-      PartDev& pd = *up;
+    for (size_t s = 0; s < I.nslots(); ++s) {
+      PartDev& pd = I.S(s);
       LevelDev& l0 = *pd.lev[0];
       I.set_dev(pd);
       k_scale<<<I.grid_for(l0.n_own, BLOCK * 4), BLOCK, 0, pd.stream>>>(l0.b.p, o.nu_pre > 0 ? l0.w.p : nullptr, l0.xstart,
@@ -1910,13 +2136,23 @@ void Engine::vcycle(const double* const* b, double* const* x) {
   clear_done();
   upload_vec(0, b, V_B);
   const bool use_graph = I.h->opts.use_graph != 0;
-  if (use_graph && I.g_vcycle.empty()) capture(I.g_vcycle, &I.g_vcycle_nodes, [&] { enqueue_vcycle_entry(); });
+  // multi-column cycles have a graph of their own, captured for the last column count
+  std::vector<cudaGraphExec_t>& graph = I.multi ? I.g_vcycle_multi : I.g_vcycle;
+  int64_t& nodes = I.multi ? I.g_vcycle_multi_nodes : I.g_vcycle_nodes;
+  if (I.multi && I.g_vcycle_multi_k != (int)I.cols.size()) {
+    for (auto g : graph) cudaGraphExecDestroy(g);
+    graph.clear();
+  }
+  if (use_graph && graph.empty()) {
+    capture(graph, &nodes, [&] { enqueue_vcycle_entry(); });
+    if (I.multi) I.g_vcycle_multi_k = (int)I.cols.size();
+  }
   for (auto& up : I.parts) {
     I.set_dev(*up);
     CK(cudaEventRecord(up->ev0, up->stream));
   }
   if (use_graph)
-    launch_graphs(I.g_vcycle, I.g_vcycle_nodes);
+    launch_graphs(graph, nodes);
   else
     enqueue_vcycle_entry();
   for (auto& up : I.parts) {
@@ -1950,35 +2186,42 @@ int Engine::pcg(const double* const* b, double* const* x, double rtol, int maxit
   return rc;
 }
 
-// mode: 0 plain CG, 1 AMG-preconditioned CG, 2 flexible AMG-preconditioned CG
 int Engine::pcg_resident(double rtol, int maxiter, int mode, int* iters, double* hist) {
   require_connected();
+  if (!impl->rhs_loaded) throw std::runtime_error("pamg_pcg_resident: call pamg_load_rhs first");
+  return run_pcg(rtol, maxiter, mode, iters, nullptr, hist);
+}
+
+// mode: 0 plain CG, 1 AMG-preconditioned CG, 2 flexible AMG-preconditioned CG.  Runs the columns I.cols (right-hand sides in
+// bsave), each with its own scalars, history and convergence decision; iters / converged / hist (rows of maxiter + 1) per column.
+int Engine::run_pcg(double rtol, int maxiter, int mode, int* iters, int* converged, double* hist) {
   Impl& I = *impl;
-  if (!I.rhs_loaded) throw std::runtime_error("pamg_pcg_resident: call pamg_load_rhs first");
   if (maxiter < 0) throw std::runtime_error("maxiter < 0");
   if (mode < 0 || mode > 2) throw std::runtime_error("bad Krylov mode");
   const bool precond = mode != 0;
-  if (mode == 2)
-    for (auto& up : I.parts)
-      if (up->rprev.n == 0) {
-        I.set_dev(*up);
-        up->rprev.alloc((size_t)up->lev[0]->n_own);
-        for (auto g : I.g_iter) cudaGraphExecDestroy(g);
-        I.g_iter.clear();
-      }
+  const int graph_k = I.multi ? (int)I.cols.size() : 0;
+  auto drop_graph = [&] {
+    for (auto g : I.g_iter) cudaGraphExecDestroy(g);
+    I.g_iter.clear();
+  };
+  for (size_t s = 0; s < I.nslots(); ++s) {
+    PartDev& pd = I.S(s);
+    PartDev::Col& pc = pd.cols[I.col_of(s)];
+    I.set_dev(pd);
+    if (mode == 2 && pc.rprev.n == 0) {
+      pc.rprev.alloc((size_t)pd.lev[0]->n_own);
+      drop_graph();
+    }
+    if (pc.hist_cap < maxiter + 2) {
+      pc.hist.alloc(maxiter + 2);
+      pc.hist_cap = maxiter + 2;
+      drop_graph();  // hist pointer is baked into the graph
+    }
+    I.bind(I.col_of(s), true);
+  }
   I.launches = 0;
   const bool use_graph = I.h->opts.use_graph != 0;
-  for (auto& up : I.parts) {
-    PartDev& pd = *up;
-    I.set_dev(pd);
-    if (pd.hist_cap < maxiter + 2) {
-      pd.hist.alloc(maxiter + 2);
-      pd.hist_cap = maxiter + 2;
-      for (auto g : I.g_iter) cudaGraphExecDestroy(g);  // hist pointer is baked into the graph
-      I.g_iter.clear();
-    }
-  }
-  if (use_graph && (I.g_iter.empty() || I.g_iter_mode != mode)) {
+  if (use_graph && (I.g_iter.empty() || I.g_iter_mode != mode || I.g_iter_k != graph_k)) {
     I.names.clear();
     I.naming = true;
     try {
@@ -1989,26 +2232,30 @@ int Engine::pcg_resident(double rtol, int maxiter, int mode, int* iters, double*
     }
     I.naming = false;
     I.g_iter_mode = mode;
+    I.g_iter_k = graph_k;
   }
   const bool zero_guess = precond && I.L > 1 && I.h->opts.nu_pre > 0;
   sync_all();
-  std::memset(I.hstat, 0, sizeof(HostStat) * HS_RING);
+  for (int c : I.cols) std::memset(I.hstat_base + (size_t)c * HS_RING, 0, sizeof(HostStat) * HS_RING);
   for (auto& up : I.parts) {
-    PartDev& pd = *up;
+    I.set_dev(*up);
+    CK(cudaEventRecord(up->ev0, up->stream));
+  }
+  for (size_t s = 0; s < I.nslots(); ++s) {
+    PartDev& pd = I.S(s);
     LevelDev& l0 = *pd.lev[0];
     I.set_dev(pd);
-    CK(cudaEventRecord(pd.ev0, pd.stream));
     k_pcg_init<<<I.grid_red(l0.n_own), BLOCK, 0, pd.stream>>>(pd.bsave.p, pd.xsol.p, l0.b.p, pd.p.p, l0.xstart,
                                                                         zero_guess ? l0.w.p : nullptr, (int)l0.n_own, pd.st.p,
                                                                         pd.partials.p, pd.rc, rtol, maxiter, I.fold_check ? 1 : 0,
-                                                                        pd.hist.p, up.get() == I.parts[0].get() ? I.hstat : nullptr);
+                                                                        pd.hist.p, &pd == I.parts[0].get() ? I.hstat : nullptr);
     I.note_launch("k_pcg_init");
   }
   if (!I.fold_check)
-    for (auto& up : I.parts) {
-      PartDev& pd = *up;
+    for (size_t s = 0; s < I.nslots(); ++s) {
+      PartDev& pd = I.S(s);
       I.set_dev(pd);
-      k_check<<<1, 1, 0, pd.stream>>>(pd.st.p, pd.rc, pd.hist.p, up.get() == I.parts[0].get() ? I.hstat : nullptr);
+      k_check<<<1, 1, 0, pd.stream>>>(pd.st.p, pd.rc, pd.hist.p, &pd == I.parts[0].get() ? I.hstat : nullptr);
       I.note_launch("k_check");
     }
   CK(cudaGetLastError());
@@ -2017,6 +2264,8 @@ int Engine::pcg_resident(double rtol, int maxiter, int mode, int* iters, double*
   PartDev& p0 = I.P(0);
   const int LOOKAHEAD = 1;
   if (maxiter + 2 >= (1 << 30)) throw std::runtime_error("maxiter too large");
+  const size_t nc = I.cols.size();
+  std::vector<char> col_done(nc, 0);  // a column that reported done or error is frozen: its ring is not waited for again
   bool finished = false;
   int launched = 0;
   while (!finished) {
@@ -2036,13 +2285,19 @@ int Engine::pcg_resident(double rtol, int maxiter, int mode, int* iters, double*
     if (launched > LOOKAHEAD) {  // status written by k_check number (launched - LOOKAHEAD + 1), straight into pinned memory
       // k_check number 1 is the one of r0, number k + 1 the one of iteration k; none exists beyond maxiter + 1
       const uint32_t want = (uint32_t)std::min(launched - LOOKAHEAD + 1, maxiter + 1);
-      volatile HostStat* hsl = I.hstat + (want % HS_RING);
-      const auto t0 = std::chrono::steady_clock::now();
-      while (hsl->seq != want) {
-        if (std::chrono::steady_clock::now() - t0 > std::chrono::seconds(30))
-          throw CommError("timed out waiting for the device status of a PCG iteration");
+      bool all = true;
+      for (size_t c = 0; c < nc; ++c) {
+        if (col_done[c]) continue;
+        volatile HostStat* hsl = I.hstat_base + (size_t)I.cols[c] * HS_RING + (want % HS_RING);
+        const auto t0 = std::chrono::steady_clock::now();
+        while (hsl->seq != want) {
+          if (std::chrono::steady_clock::now() - t0 > std::chrono::seconds(30))
+            throw CommError("timed out waiting for the device status of a PCG iteration");
+        }
+        if (hsl->done || hsl->error) col_done[c] = 1;
+        all = all && col_done[c];
       }
-      if (hsl->done || hsl->error) finished = true;
+      if (all) finished = true;
     }
     if (launched > maxiter + LOOKAHEAD + 1) finished = true;
   }
@@ -2051,9 +2306,6 @@ int Engine::pcg_resident(double rtol, int maxiter, int mode, int* iters, double*
     CK(cudaEventRecord(up->ev1, up->stream));
   }
   sync_all();
-  DevState fin;
-  I.set_dev(p0);
-  CK(cudaMemcpy(&fin, p0.st.p, sizeof(fin), cudaMemcpyDeviceToHost));
   float ms = 0, mx = 0;
   for (auto& up : I.parts) {
     I.set_dev(*up);
@@ -2061,17 +2313,101 @@ int Engine::pcg_resident(double rtol, int maxiter, int mode, int* iters, double*
     mx = std::max(mx, ms);
   }
   check_device_error();
-  const double r0 = std::sqrt(fin.sc[SC_RR0]), rn = std::sqrt(fin.sc[SC_RR]);
-  const bool conv = rn <= rtol * r0;
-  if (iters) *iters = fin.iters;
-  if (hist && fin.iters >= 0) CK(cudaMemcpy(hist, p0.hist.p, (fin.iters + 1) * sizeof(double), cudaMemcpyDeviceToHost));
-  I.stats.iters = fin.iters;
-  I.stats.converged = conv;
-  I.stats.r0_norm = r0;
-  I.stats.r_norm = rn;
+  bool all_conv = true;
+  int max_iters = 0;
+  for (size_t c = 0; c < nc; ++c) {
+    DevState fin;
+    I.bind(I.cols[c]);
+    I.set_dev(p0);
+    CK(cudaMemcpy(&fin, p0.st.p, sizeof(fin), cudaMemcpyDeviceToHost));
+    const double r0 = std::sqrt(fin.sc[SC_RR0]), rn = std::sqrt(fin.sc[SC_RR]);
+    const bool conv = rn <= rtol * r0;
+    if (iters) iters[c] = fin.iters;
+    if (converged) converged[c] = conv ? 1 : 0;
+    if (hist && fin.iters >= 0)
+      CK(cudaMemcpy(hist + c * (size_t)(maxiter + 1), p0.hist.p, (fin.iters + 1) * sizeof(double), cudaMemcpyDeviceToHost));
+    all_conv = all_conv && conv;
+    max_iters = std::max(max_iters, (int)fin.iters);
+    if (c == 0) {
+      I.stats.r0_norm = r0;
+      I.stats.r_norm = rn;
+    }
+  }
+  I.stats.iters = max_iters;
+  I.stats.converged = all_conv;
   I.stats.solve_ms = mx;
   I.stats.kernel_launches = I.launches;
-  return conv ? PAMG_OK : PAMG_ERR_NOTCONV;
+  return all_conv ? PAMG_OK : PAMG_ERR_NOTCONV;
+}
+
+// ---------------------------------------------------------------------------------------------
+// several right-hand sides (columns 0..k-1 of the per-solve state): the enqueue_* functions run over all of them, with k-wide
+// launches where the block's kernel has one (enqueue_op) and the single-column kernels per column elsewhere
+// ---------------------------------------------------------------------------------------------
+void Engine::begin_multi(int k) {
+  Impl& I = *impl;
+  if (k < 1 || k > I.kmax)
+    throw std::runtime_error("k = " + std::to_string(k) + " right-hand sides exceed the capacity " + std::to_string(I.kmax) +
+                             " this device state was initialised with (pamg_set_rhs_capacity before pamg_device_init)");
+  require_connected();
+  I.cols.resize(k);
+  for (int c = 0; c < k; ++c) I.cols[c] = c;
+  I.multi = true;
+}
+
+void Engine::end_multi() {
+  Impl& I = *impl;
+  I.cols.assign(1, 0);
+  I.multi = false;
+  I.bind(0);
+}
+
+template <class F>
+auto Engine::in_multi(int k, F&& body) -> decltype(body()) {
+  begin_multi(k);
+  try {
+    auto r = body();
+    end_multi();
+    return r;
+  } catch (...) {
+    end_multi();
+    throw;
+  }
+}
+
+// kernel timing of k columns (kinds whose operations run through enqueue_op: 0, 1, 2, 3, 6, 7), so a k-wide launch can be
+// compared with k single launches of the same block (scripts/multi_rhs_sweep.py)
+void Engine::time_kernel_multi(int k, int kind, int level, int reps, bool flush_l2, float* ms_out) {
+  if (kind != 0 && kind != 1 && kind != 2 && kind != 3 && kind != 6 && kind != 7)
+    throw std::runtime_error("multi-column timing covers kinds 0, 1, 2, 3, 6 and 7");
+  in_multi(k, [&] {
+    time_kernel(kind, level, reps, flush_l2, ms_out);
+    return 0;
+  });
+}
+
+void Engine::spmv_multi(int level, int k, const double* const* x, double* const* y) {
+  in_multi(k, [&] {
+    spmv(level, x, y);
+    return 0;
+  });
+}
+
+void Engine::vcycle_multi(int k, const double* const* b, double* const* x) {
+  in_multi(k, [&] {
+    vcycle(b, x);
+    return 0;
+  });
+}
+
+int Engine::pcg_multi(int k, const double* const* b, double* const* x, double rtol, int maxiter, int mode, int* iters, int* converged,
+                      double* hist) {
+  return in_multi(k, [&] {
+    load_rhs(b);
+    const int rc = run_pcg(rtol, maxiter, mode, iters, converged, hist);
+    read_solution(x);
+    return rc;
+  });
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -2304,7 +2640,7 @@ void Engine::time_kernel(int kind, int level, int reps, bool flush_l2, float* ms
     CK(cudaMalloc(&I.flush_buf, I.flush_n * sizeof(double)));
     CK(cudaMemset(I.flush_buf, 0, I.flush_n * sizeof(double)));
   }
-  const size_t np = I.parts.size();
+  const size_t np = I.nslots();
   clear_done();
   cudaEvent_t e0, e1;
   CK(cudaEventCreate(&e0));
@@ -2319,26 +2655,26 @@ void Engine::time_kernel(int kind, int level, int reps, bool flush_l2, float* ms
     std::vector<EpiArgs> epi(np);
     if (kind == 0) {
       for (size_t i = 0; i < np; ++i)
-        epi[i] = EpiArgs{I.P(i).lev[level]->t.p, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0.0, 0.0};
+        epi[i] = EpiArgs{I.S(i).lev[level]->t.p, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0.0, 0.0};
       enqueue_op(OpSpec{level, PAMG_A_OO, level, M_MUL, false, 0, false}, ptrs(level, V_X), epi);
     } else if (kind == 1) {
       std::vector<double*> cur;
-      for (auto& up : I.parts) cur.push_back(up->lev[level]->x.p);
+      for (size_t s = 0; s < np; ++s) cur.push_back(I.S(s).lev[level]->x.p);
       enqueue_smooth(level, 1, cur, false, false);
     } else if (kind == 2) {
       for (size_t i = 0; i < np; ++i) {
-        LevelDev& ld = *I.P(i).lev[level];
+        LevelDev& ld = *I.S(i).lev[level];
         epi[i] = EpiArgs{ld.t.p, ld.b.p, nullptr, nullptr, nullptr, nullptr, nullptr, 0.0, 0.0};
       }
       enqueue_op(OpSpec{level, PAMG_A_OO, level, M_RESID, false, 0, false}, ptrs(level, V_X), epi);
       for (size_t i = 0; i < np; ++i) {
-        LevelDev& lc = *I.P(i).lev[level + 1];
+        LevelDev& lc = *I.S(i).lev[level + 1];
         epi[i] = EpiArgs{lc.b.p, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0.0, 0.0};
       }
       enqueue_op(OpSpec{level, PAMG_R_OO, level, M_RESTRICT, false, 0, false}, ptrs(level, V_T), epi);
     } else if (kind == 3) {
       for (size_t i = 0; i < np; ++i) {
-        LevelDev& ld = *I.P(i).lev[level];
+        LevelDev& ld = *I.S(i).lev[level];
         epi[i] = EpiArgs{ld.x2.p, ld.x.p, nullptr, nullptr, nullptr, nullptr, nullptr, 0.0, 0.0};
       }
       enqueue_op(OpSpec{level, PAMG_P_OO, level + 1, M_ADD, false, 0, false}, ptrs(level + 1, V_X), epi);
@@ -2354,14 +2690,14 @@ void Engine::time_kernel(int kind, int level, int reps, bool flush_l2, float* ms
       k_flush<<<148 * 8, 256, 0, p0.stream>>>(I.flush_buf, I.flush_n);
     } else if (kind == 6) {  // SpMV with the fused p.q dot (as in the PCG iteration) + its reduce launch
       for (size_t i = 0; i < np; ++i) {
-        LevelDev& ld = *I.P(i).lev[level];
+        LevelDev& ld = *I.S(i).lev[level];
         epi[i] = EpiArgs{ld.t.p, nullptr, nullptr, nullptr, nullptr, nullptr, ld.x.p, 0.0, 0.0};
       }
       enqueue_op(OpSpec{level, PAMG_A_OO, level, M_MUL, true, 3, false}, ptrs(level, V_X), epi);
     } else if (kind == 7) {  // Jacobi sweep with the fused r.z dot
       if (I.h->opts.smoother == PAMG_SMOOTHER_CHEBYSHEV) throw std::runtime_error("kind 7 needs a Jacobi smoother");
       std::vector<double*> cur;
-      for (auto& up : I.parts) cur.push_back(up->lev[level]->x.p);
+      for (size_t s = 0; s < np; ++s) cur.push_back(I.S(s).lev[level]->x.p);
       enqueue_smooth(level, 1, cur, false, true);
     } else if (kind == 5) {
       const bool use_graph = I.h->opts.use_graph != 0;

@@ -29,12 +29,14 @@ enum VecId { V_X = 0, V_X2, V_B, V_T, V_XSTART, V_XSOL, V_P, V_Q, V_BSAVE };
 
 class Engine {
  public:
-  Engine(Hierarchy* h, int nlocal, const int32_t* local_parts, const int32_t* device_ids);
+  // kmax: columns of per-solve device state (right-hand sides a multi-column call may use), 1..PAMG_MAX_RHS
+  Engine(Hierarchy* h, int nlocal, const int32_t* local_parts, const int32_t* device_ids, int kmax = 1);
   ~Engine();
   Engine(const Engine&) = delete;
   Engine& operator=(const Engine&) = delete;
 
   static int32_t handle_bytes();
+  int rhs_capacity() const;
   void export_handle(int part, void* blob);
   void import_handle(int part, const void* blob);
   void connect();
@@ -48,6 +50,12 @@ class Engine {
   double dot(int level, const double* const* u, const double* const* v);
   void vcycle(const double* const* b, double* const* x);
   int pcg(const double* const* b, double* const* x, double rtol, int maxiter, int mode, int* iters, double* hist);
+  // k right-hand sides: vectors at [j * nparts + part]; column j bit-identical to the single-column call on it
+  void spmv_multi(int level, int k, const double* const* x, double* const* y);
+  void vcycle_multi(int k, const double* const* b, double* const* x);
+  void time_kernel_multi(int k, int kind, int level, int reps, bool flush_l2, float* ms_out);
+  int pcg_multi(int k, const double* const* b, double* const* x, double rtol, int maxiter, int mode, int* iters, int* converged,
+                double* hist);
   int fgmres(const double* const* b, double* const* x, double rtol, int maxiter, int restart, int precond, int* iters,
              double* hist);
   void load_rhs(const double* const* b);
@@ -81,6 +89,11 @@ class Engine {
   void enqueue_dot_rz();
   bool vcycle_fuses_rz() const;
   void enqueue_pcg_iteration(int mode);
+  int run_pcg(double rtol, int maxiter, int mode, int* iters, int* converged, double* hist);
+  void begin_multi(int k);
+  void end_multi();
+  template <class F>
+  auto in_multi(int k, F&& body) -> decltype(body());
   template <class F>
   void capture(std::vector<cudaGraphExec_t>& out, int64_t* nodes, F&& body);
   void launch_graphs(const std::vector<cudaGraphExec_t>& gs, int64_t nodes);

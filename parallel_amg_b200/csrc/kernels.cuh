@@ -1193,6 +1193,203 @@ __global__ void __launch_bounds__(BLOCK, MINB) k_spmv_sell_diag(SellDiagView A, 
 }
 
 // ---------------------------------------------------------------------------------------------
+// k-wide forms of k_spmv_sell_diag and k_spmv_sell_vi4: K right-hand sides per launch (pamg_*_multi)
+// ---------------------------------------------------------------------------------------------
+// Per step a lane loads the index word (and for vi4 the column word) once, then gathers and accumulates for every live column.  Per
+// column everything is the single kernel's: the slice -> warp -> lane map and slice stride (the engine launches the same grid), the
+// per-row __dmul_rn / __dadd_rn order, rows4_prefetch / rows4_epilogue, one s_acc slot per thread, and dot_finish on the column's own
+// partials, ticket and RedCtx.  So column c of a k-wide launch is bit-identical to the single kernel on column c alone.  Main role only:
+// multi-column calls run their halo exchange as separate k_halo_pack / k_boundary launches per column.  A column is live when its
+// pointer is set and its DevState is not `done` (a converged column is frozen as in the single-column solve).
+template <int K>
+struct MultiCols {
+  const double* x[K];
+  EpiArgs a[K];
+  DevState* st[K];  // nullptr: absent column
+  double* partials[K];
+  RedCtx rc[K];
+};
+
+template <int K>
+__device__ __forceinline__ unsigned live_columns(const MultiCols<K>& m) {
+  unsigned live = 0;
+#pragma unroll
+  for (int c = 0; c < K; ++c)
+    if (m.st[c] && !m.st[c]->done) live |= 1u << c;
+  return live;
+}
+
+template <int MODE, bool DOT, int K>
+__device__ __forceinline__ void multi_finish(const MultiCols<K>& m, unsigned live, double (&s_acc)[K][BLOCK], int publish, int red_slot) {
+#pragma unroll
+  for (int c = 0; c < K; ++c)
+    if (live >> c & 1u) dot_finish(s_acc[c][threadIdx.x], m.partials[c], m.st[c], &m.st[c]->ticket[0], m.rc[c], publish, 0, red_slot);
+}
+
+// U = 1 diagonal per step at K = 4, 2 at K = 2 (scripts/ptxas_table.py: no spills)
+template <int MODE, bool DOT, int K, int U = (K >= 4 ? 1 : 2), int MINB = 2>
+__global__ void __launch_bounds__(BLOCK, MINB) k_spmv_sell_diag_multi(SellDiagView A, MultiCols<K> m, FusedHalo fh, int publish, int red_slot) {
+  const unsigned live = live_columns(m);
+  if (!live) return;
+#pragma unroll
+  for (int c = 0; c < K; ++c)
+    if (live >> c & 1u) trace_mark(m.st[c]);
+  const int n_main = (int)gridDim.x;
+  __shared__ double s_dict[256];
+  __shared__ int s_off[SELL_DIAG_MAX];
+  __shared__ double s_acc[K][DOT ? BLOCK : 1];
+  s_dict[threadIdx.x] = A.dict[threadIdx.x];  // BLOCK == 256
+  if (threadIdx.x < A.ndiag) s_off[threadIdx.x] = A.off[threadIdx.x];
+  if (DOT)
+#pragma unroll
+    for (int c = 0; c < K; ++c) s_acc[c][threadIdx.x] = 0.0;
+  __syncthreads();
+  const int lane = threadIdx.x & 31;
+  const int wpb = BLOCK / 32;
+  const int last = A.nrows - 1;
+  for (int sl = blockIdx.x * wpb + (threadIdx.x >> 5); sl < A.nslices; sl += n_main * wpb) {
+    const int base = sl * 128;
+    const bool full = base + 128 <= A.nrows;
+    const int rstep = full ? 32 : 1;
+    const int r_first = full ? base + lane : base + lane * 4;
+#pragma unroll
+    for (int c = 0; c < K; ++c)
+      if (live >> c & 1u) rows4_prefetch<MODE, DOT>(m.a[c], fh, r_first, rstep, A.nrows);
+    double s[K][4];
+#pragma unroll
+    for (int c = 0; c < K; ++c)
+#pragma unroll
+      for (int k = 0; k < 4; ++k) s[c][k] = 0.0;
+    const uint32_t* __restrict__ ij = A.idx + (size_t)sl * A.ndiag * 32 + lane;
+#pragma unroll 1
+    for (int j0 = 0; j0 < A.ndiag; j0 += U) {
+      unsigned iv[U];
+      double xv[K][U][4];
+#pragma unroll
+      for (int u = 0; u < U; ++u)
+        if (j0 + u < A.ndiag) {
+          iv[u] = __ldcs(ij + (j0 + u) * 32);
+          const int o = s_off[j0 + u];
+#pragma unroll
+          for (int c = 0; c < K; ++c)
+            if (live >> c & 1u)
+#pragma unroll
+              for (int k = 0; k < 4; ++k) xv[c][u][k] = m.x[c][min(max(r_first + k * rstep + o, 0), last)];
+        }
+#pragma unroll
+      for (int u = 0; u < U; ++u)
+        if (j0 + u < A.ndiag) {
+#pragma unroll
+          for (int k = 0; k < 4; ++k) {
+            const unsigned v = vi_index(iv[u], k);
+            if (v != SELL_DIAG_ABSENT) {
+              const double d = s_dict[v];
+#pragma unroll
+              for (int c = 0; c < K; ++c)
+                if (live >> c & 1u) s[c][k] = __dadd_rn(s[c][k], __dmul_rn(d, xv[c][u][k]));
+            }
+          }
+        }
+    }
+#pragma unroll
+    for (int c = 0; c < K; ++c)
+      if (live >> c & 1u) {
+        const double contrib = rows4_epilogue<MODE, DOT>(m.a[c], fh, s[c], r_first, rstep, A.nrows);
+        if (DOT) s_acc[c][threadIdx.x] += contrib;
+      }
+  }
+  if constexpr (DOT) multi_finish<MODE, DOT, K>(m, live, s_acc, publish, red_slot);
+}
+
+// IB index bytes per entry as in k_spmv_sell_vi4; U = 1 entry per step at K = 4, 2 at K = 2
+template <int MODE, bool DOT, int IB, int K, int U = (K >= 4 ? 1 : 2), int MINB = 2>
+__global__ void __launch_bounds__(BLOCK, MINB) k_spmv_sell_vi4_multi(SellViView A, MultiCols<K> m, FusedHalo fh, int publish, int red_slot) {
+  const unsigned live = live_columns(m);
+  if (!live) return;
+#pragma unroll
+  for (int c = 0; c < K; ++c)
+    if (live >> c & 1u) trace_mark(m.st[c]);
+  const int n_main = (int)gridDim.x;
+  extern __shared__ double s_dict[];
+  __shared__ double s_acc[K][DOT ? BLOCK : 1];
+  for (int i = threadIdx.x; i < A.ndict; i += BLOCK) s_dict[i] = A.dict[i];
+  if (DOT)
+#pragma unroll
+    for (int c = 0; c < K; ++c) s_acc[c][threadIdx.x] = 0.0;
+  __syncthreads();
+  const int lane = threadIdx.x & 31;
+  const int wpb = BLOCK / 32;
+  for (int sl = blockIdx.x * wpb + (threadIdx.x >> 5); sl < A.nslices; sl += n_main * wpb) {
+    const int o0 = A.slice_off[sl];
+    const int w = A.slice_off[sl + 1] - o0;
+    const int base = sl * 128;
+    const bool full = base + 128 <= A.nrows;
+    const int rstep = full ? 32 : 1;
+    const int r_first = full ? base + lane : base + lane * 4;
+#pragma unroll
+    for (int c = 0; c < K; ++c)
+      if (live >> c & 1u) rows4_prefetch<MODE, DOT>(m.a[c], fh, r_first, rstep, A.nrows);
+    double s[K][4];
+#pragma unroll
+    for (int c = 0; c < K; ++c)
+#pragma unroll
+      for (int k = 0; k < 4; ++k) s[c][k] = 0.0;
+    const int4* __restrict__ cj = reinterpret_cast<const int4*>(A.col) + (size_t)o0 * 32 + lane;
+    using IV = typename std::conditional<IB == 1, unsigned, uint2>::type;
+    const IV* __restrict__ ij = reinterpret_cast<const IV*>(A.vidx) + (size_t)o0 * 32 + lane;
+#pragma unroll 1
+    for (int j0 = 0; j0 < w; j0 += U, cj += U * 32, ij += U * 32) {
+      int4 cv[U];
+      IV iv[U];
+#pragma unroll
+      for (int u = 0; u < U; ++u)
+        if (j0 + u < w) {
+          cv[u] = __ldcs(cj + u * 32);
+          iv[u] = __ldcs(ij + u * 32);
+        }
+      // the data dependence of k_spmv_sell_vi4: every gather of the step goes out after all of its column and index loads
+      int allc = 0;
+#pragma unroll
+      for (int u = 0; u < U; ++u)
+        if (j0 + u < w) allc |= cv[u].x | cv[u].y | cv[u].z | cv[u].w | (int)(vi_bits(iv[u]) >> 1);
+      const int z = allc >> 31;
+      double xv[K][U][4];
+#pragma unroll
+      for (int u = 0; u < U; ++u)
+        if (j0 + u < w) {
+#pragma unroll
+          for (int c = 0; c < K; ++c)
+            if (live >> c & 1u) {
+              xv[c][u][0] = m.x[c][cv[u].x + z];
+              xv[c][u][1] = m.x[c][cv[u].y + z];
+              xv[c][u][2] = m.x[c][cv[u].z + z];
+              xv[c][u][3] = m.x[c][cv[u].w + z];
+            }
+        }
+      asm volatile("" ::: "memory");
+#pragma unroll
+      for (int u = 0; u < U; ++u)
+        if (j0 + u < w) {
+#pragma unroll
+          for (int k = 0; k < 4; ++k) {
+            const double d = s_dict[vi_index(iv[u], k)];
+#pragma unroll
+            for (int c = 0; c < K; ++c)
+              if (live >> c & 1u) s[c][k] = __dadd_rn(s[c][k], __dmul_rn(d, xv[c][u][k]));
+          }
+        }
+    }
+#pragma unroll
+    for (int c = 0; c < K; ++c)
+      if (live >> c & 1u) {
+        const double contrib = rows4_epilogue<MODE, DOT>(m.a[c], fh, s[c], r_first, rstep, A.nrows);
+        if (DOT) s_acc[c][threadIdx.x] += contrib;
+      }
+  }
+  if constexpr (DOT) multi_finish<MODE, DOT, K>(m, live, s_acc, publish, red_slot);
+}
+
+// ---------------------------------------------------------------------------------------------
 // halo pack: owner -> ghost (consistent!).  Stores into the neighbours' staging, then flags.
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(BLOCK) k_halo_pack(const double* __restrict__ v, const int32_t* __restrict__ send_idx,
